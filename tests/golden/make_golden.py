@@ -4,7 +4,8 @@ Run in the build container only (needs /root/reference):  python tests/golden/ma
 Reference version: _version.py -> 0.1.dev68+g9b77c89e2.d20250827; numpy 2.3.5 (NEP 50), fp32 actions,
 fp32-representable noise (SURVEY.md section 8c "canonical for parity").
 
-Fixtures (all small, committed):
+Fixtures (all small, committed; a set larger than 1 MB is stored as parts <name>.1.npz, <name>.2.npz, ... that
+tests/util.py:load_golden merges):
   <env>_forced.npz : M independent (state, ep_step, action, noise) -> env.step() tuples, sampled to hit every
                      branch of the dynamics / reward / constraint / termination logic.
   <env>_trace.npz  : BASELINE config #1 -- one env, 1000 steps, random fp32 actions, reset on done; everything
@@ -27,7 +28,9 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
+sys.path.insert(0, os.path.dirname(HERE))
 import ref_loader  # noqa: E402
+from util import save_golden  # noqa: E402
 
 ENV_CLASS = {"reactor": "ChemicalReactorEnv", "grid": "PowerGridEnv", "robot": "RobotAssemblyEnv"}
 NOISE_SHAPES = {"reactor": [None, None], "grid": [8, 8, 7], "robot": []}
@@ -174,14 +177,14 @@ def make_forced(envs, name, m, seed):
             for k, v in zip(("next_state", "reward", "terminated", "truncated", "n_viol", "n_crit", "crit", "viol_mask", "noise"),
                             (ns, r, te, tr, nv, nc, cs, vm, flat)):
                 out[k].append(v)
-    np.savez_compressed(os.path.join(HERE, f"{name}_forced.npz"),
-                        state=S, ep_step=steps, action=A,
-                        noise=np.array(out["noise"], np.float32).reshape(m, NZ[name]),
-                        next_state=np.array(out["next_state"], np.float32),
-                        reward=np.array(out["reward"], np.float64),
-                        terminated=np.array(out["terminated"], bool), truncated=np.array(out["truncated"], bool),
-                        n_viol=np.array(out["n_viol"], np.int32), n_crit=np.array(out["n_crit"], np.int32),
-                        crit=np.array(out["crit"], bool), viol_mask=np.array(out["viol_mask"], np.uint8))
+    save_golden(os.path.join(HERE, f"{name}_forced"),
+                state=S, ep_step=steps, action=A,
+                noise=np.array(out["noise"], np.float32).reshape(m, NZ[name]),
+                next_state=np.array(out["next_state"], np.float32),
+                reward=np.array(out["reward"], np.float64),
+                terminated=np.array(out["terminated"], bool), truncated=np.array(out["truncated"], bool),
+                n_viol=np.array(out["n_viol"], np.int32), n_crit=np.array(out["n_crit"], np.int32),
+                crit=np.array(out["crit"], bool), viol_mask=np.array(out["viol_mask"], np.uint8))
     te, tr, cr = np.array(out["terminated"]), np.array(out["truncated"]), np.array(out["crit"])
     print(f"{name}_forced: {m} tuples, terminated {te.sum()}, truncated {tr.sum()}, critical {cr.sum()}, "
           f"violations {np.sum(out['n_viol'])}")
@@ -361,7 +364,7 @@ def make_policy_forced(envs, seed, per_case=2000):
             print(f"policy_forced {key}: {len(rows)} transitions recorded, {len(pick)} kept, coin drawn in "
                   f"{np.isfinite(c).sum()}, normals in {(np.abs(out[key + '_z']).sum(1) > 0).sum()}, "
                   f"uniforms in {(np.abs(out[key + '_u']).sum(1) > 0).sum()}")
-    np.savez_compressed(os.path.join(HERE, "policy_forced.npz"), **out)
+    save_golden(os.path.join(HERE, "policy_forced"), **out)
 
 
 def make_baseline_goldens(seed):

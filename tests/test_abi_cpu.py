@@ -179,15 +179,15 @@ def test_bench_reference_arm_runs_without_a_gpu():
 
 
 def test_reference_copy_is_byte_identical_and_not_in_history():
-    """oracle/_ref holds the seven hot-path reference modules byte for byte (SHA-256 manifest; compared with the reference
-    tree too when that exists), and it is git-ignored: reference sources never enter this repo's history."""
+    """oracle/_ref, where oracle/make_ref.py made it, holds the seven hot-path reference modules byte for byte (SHA-256
+    manifest; compared with the reference tree too when that exists), and it is git-ignored: reference sources never
+    enter this repo's history."""
     import subprocess
     from oracle import make_ref
-    if not make_ref.available():
-        pytest.skip("oracle/_ref not built (no reference tree on this machine)")
-    assert make_ref.verify()
+    if make_ref.available():
+        assert make_ref.verify()
     r = subprocess.run(["git", "-C", ROOT, "check-ignore", "-q", "oracle/_ref/MANIFEST.json"])
-    if r.returncode in (0, 1):                                      # 128: not a git checkout (the GPU box snapshot)
+    if r.returncode in (0, 1):                                      # 128: not a git checkout (a copy of the tree)
         assert r.returncode == 0
     tracked = subprocess.run(["git", "-C", ROOT, "ls-files", "oracle/_ref"], capture_output=True, text=True)
     assert tracked.stdout.strip() == ""

@@ -13,7 +13,7 @@ import os
 import numpy as np
 import pytest
 
-from util import ENV_IDS, KINDS, assert_bits_equal, ulp_diff
+from util import ENV_IDS, KINDS, assert_bits_equal, load_golden, ulp_diff
 
 pytestmark = pytest.mark.gpu
 
@@ -63,7 +63,7 @@ def _noise(rng, O, kind, n):
 @pytest.mark.parametrize("name", ["reactor", "grid", "robot"])
 def test_step_vs_reference_goldens(mods, golden_dir, name):
     ni, N, O, torch = mods
-    g = np.load(os.path.join(golden_dir, f"{name}_forced.npz"))
+    g = load_golden(golden_dir, f"{name}_forced")
     kind, m = KINDS[name], len(g["reward"])
     env = _native_env(ni, kind, m, auto_reset=False)
     env.set_state_host(g["state"], g["ep_step"], np.zeros(m, np.int32), np.zeros(m, np.uint8))

@@ -15,7 +15,7 @@ import numpy as np
 import pytest
 
 from oracle import oracle as O
-from util import KINDS, assert_bits_equal, ulp_diff
+from util import KINDS, assert_bits_equal, load_golden, ulp_diff
 
 
 def _load(golden_dir, name):
@@ -46,7 +46,7 @@ def _check_step_outputs(kind_name, g, ns, r, fl, vm):
 @pytest.mark.parametrize("name", ["reactor", "grid", "robot"])
 def test_forced_tuples(golden_dir, name):
     """M independent (state, step counter, action, noise) -> env.step() tuples covering every branch."""
-    g = _load(golden_dir, f"{name}_forced.npz")
+    g = load_golden(golden_dir, f"{name}_forced")
     kind = KINDS[name]
     m = len(g["reward"])
     env = O.OracleEnv(kind, m, auto_reset=False)
@@ -90,7 +90,7 @@ def test_robot_spec_trig_vs_reference(golden_dir):
     the reference's outputs (numpy -> libm): flags / masks identical; positions, joints, forces and scores bit-identical
     (the two sin / cos differ by <= 2 ulp of fp64, which does not survive the rounding to fp32); end-effector
     velocities within 1e-12 absolute (a cancelling difference of positions); reward <= 1e-6 relative."""
-    g = _load(golden_dir, "robot_forced.npz")
+    g = load_golden(golden_dir, "robot_forced")
     m = len(g["reward"])
     env = O.OracleEnv(O.ROBOT, m, auto_reset=False, exp_mode=1)
     env.state[:] = g["state"]

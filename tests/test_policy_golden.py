@@ -1,6 +1,6 @@
 """get_dataset's policies and the benchmark baseline controllers, pinned to the UNMODIFIED reference.
 
-tests/golden/policy_forced.npz holds, per env x quality, transitions of the reference's own get_dataset run
+tests/golden/policy_forced.npz (stored in parts) holds, per env x quality, transitions of the reference's own get_dataset run
 (chemical_reactor.py:324-420, power_grid.py:194-249, robot_assembly.py:246-308): the observation the policy saw, every
 random value it drew (coin, normals / scale, uniforms / half-range -- recorded by interposing np.random.*) and the action
 the dataset stores. tests/golden/baseline_agents.npz holds action sequences of the reference's
@@ -23,14 +23,14 @@ import os
 import numpy as np
 import pytest
 
-from util import ENV_IDS, KINDS, assert_bits_equal, ulp_diff
+from util import ENV_IDS, KINDS, assert_bits_equal, load_golden, ulp_diff
 
 ENV_CLASS = {"reactor": "ChemicalReactorEnv", "grid": "PowerGridEnv", "robot": "RobotAssemblyEnv"}
 CASES = [(n, q) for n in ("reactor", "grid", "robot") for q in ("expert", "medium", "mixed", "random")]
 
 
 def _case(golden_dir, name, quality):
-    g = np.load(os.path.join(golden_dir, "policy_forced.npz"))
+    g = load_golden(golden_dir, "policy_forced")
     key = f"{name}_{quality}"
     coin = g[key + "_coin"]
     coin32 = np.where(np.isfinite(coin), coin, 0.5).astype(np.float32)
@@ -70,7 +70,7 @@ def test_oracle_policy_vs_reference_get_dataset(golden_dir, name, quality):
 
 
 def test_policy_golden_covers_every_branch(golden_dir):
-    g = np.load(os.path.join(golden_dir, "policy_forced.npz"))
+    g = load_golden(golden_dir, "policy_forced")
     for name, quality in CASES:
         key = f"{name}_{quality}"
         assert len(g[key + "_obs"]) >= 300, key

@@ -1,5 +1,51 @@
 """Shared helpers for the parity tests."""
+import glob
+import io
+import os
+
 import numpy as np
+
+GOLDEN_FILE_LIMIT = 1_000_000     # bytes per fixture file; a larger set is stored as parts <stem>.1.npz, <stem>.2.npz, ...
+
+
+def save_golden(path_stem, **arrays):
+    """np.savez_compressed to <path_stem>.npz, or, when that file would exceed GOLDEN_FILE_LIMIT, whole arrays spread in
+    order over the parts <path_stem>.<k>.npz. Replaces whatever <path_stem>.npz / parts an earlier run left."""
+    def packed(d):
+        buf = io.BytesIO()
+        np.savez_compressed(buf, **d)
+        return buf.getvalue()
+
+    parts = [packed(arrays)]
+    if len(parts[0]) > GOLDEN_FILE_LIMIT:
+        parts, cur = [], {}
+        for k, v in arrays.items():
+            if cur and len(packed({**cur, k: v})) > GOLDEN_FILE_LIMIT:
+                parts.append(packed(cur))
+                cur = {}
+            cur[k] = v
+        parts.append(packed(cur))
+    for old in glob.glob(path_stem + ".npz") + glob.glob(path_stem + ".[0-9]*.npz"):
+        os.remove(old)
+    names = [path_stem + ".npz"] if len(parts) == 1 else [f"{path_stem}.{k}.npz" for k in range(1, len(parts) + 1)]
+    for name, data in zip(names, parts):
+        assert len(data) <= GOLDEN_FILE_LIMIT, (name, len(data))
+        with open(name, "wb") as f:
+            f.write(data)
+
+
+def load_golden(golden_dir, stem):
+    """The arrays of <stem>.npz, or of all its parts <stem>.<k>.npz (save_golden), as one dict."""
+    base = os.path.join(golden_dir, stem)
+    paths = glob.glob(base + ".npz") + sorted(glob.glob(base + ".[0-9]*.npz"), key=lambda p: int(p.split(".")[-2]))
+    assert paths, f"no golden fixture {base}.npz"
+    out = {}
+    for p in paths:
+        with np.load(p) as z:
+            for k in z.files:
+                assert k not in out, (p, k)
+                out[k] = z[k]
+    return out
 
 
 def ulp_diff(a, b):
