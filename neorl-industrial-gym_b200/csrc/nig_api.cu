@@ -94,7 +94,7 @@ struct nig_env {
     bool dev_dirty;                // ... and whether a *_host call still has to wait for them
     // device staging of the *_host calls (lazily allocated)
     float *h_actions, *h_noise, *h_reset, *h_obs, *h_next_obs, *h_reward;
-    uint8_t *h_hostmask, *h_flags, *h_viol, *h_mask;
+    uint8_t *h_hostmask, *h_flags, *h_viol, *h_mask, *h_terminated, *h_truncated;
     int32_t *h_i32a, *h_i32b;
     unsigned long long* stats_shards;   // kStatsShards x NIG_STATS_SLOTS: where the PLAIN single-step kernel adds (folded into stats on read)
     bool shards_dirty;
@@ -220,20 +220,33 @@ int fold_stats(nig_env* e, cudaStream_t st)
     return NIG_OK;
 }
 
-int pick_vec(const nig_env* e, bool soa)
+// the VEC > 1 flavours move VEC envs per thread with one vector load / store per row: every caller array must be aligned
+// to it (a torch view at an odd element offset is not)
+bool vec_aligned(const StepArgs& a, int vec)
 {
-    if (e->step_vec) return e->step_vec;
-    if (!soa) return 1;
+    const uintptr_t f = (uintptr_t)(4 * vec) - 1, b = (uintptr_t)vec - 1;
+    return !((((uintptr_t)a.actions | (uintptr_t)a.noise | (uintptr_t)a.reset_states | (uintptr_t)a.obs | (uintptr_t)a.next_obs |
+               (uintptr_t)a.reward) & f) | (((uintptr_t)a.flags | (uintptr_t)a.viol_mask) & b));
+}
+
+int pick_vec(const nig_env* e, const StepArgs& a)
+{
+    // AoS calls always take VEC = 1: the wider flavours store reward / flags / masks for every env up to the pitch, which
+    // would write past the caller's exact-size [n] arrays (nig_step_host's zero-copy path hands those to the kernel)
+    if (a.action_aos || a.aux_aos) return 1;
+    int vec = 1;
+    if (e->step_vec) vec = e->step_vec;
     // reactor: two envs per thread (64-bit LDG/STG, 96 registers) once there are enough threads to fill the GPU
     // twice over; measured on B200 (tools/perf_sweep.py): VEC=2 beats VEC=1 and VEC=4 from 1M envs up.
-    const int64_t full = 148LL * 2048;
-    if (e->kind == NIG_ENV_CHEMICAL_REACTOR) return e->pitch >= 2 * full ? 2 : 1;
-    return 1;   // 32-/24-d states: two envs per thread would need > 190 registers
+    // (32-/24-d states: two envs per thread would need > 190 registers)
+    else if (e->kind == NIG_ENV_CHEMICAL_REACTOR && e->pitch >= 2 * 148LL * 2048) vec = 2;
+    while (vec > 1 && !vec_aligned(a, vec)) vec /= 2;
+    return vec;
 }
 
 int launch_step(nig_env* e, const StepArgs& a, cudaStream_t st)
 {
-    const int vec = pick_vec(e, a.action_aos == 0 && a.aux_aos == 0);
+    const int vec = pick_vec(e, a);
     e->launches++;
     note_device_work(e, st);
     // plain SoA step (no teacher forcing, no observation copies, no host-evaluated constraints): persistent TMA pipeline
@@ -732,6 +745,7 @@ int nig_destroy(nig_env_t* e)
     cudaFree(e->state); cudaFree(e->ep_word); cudaFree(e->ep_return); cudaFree(e->stats); cudaFree(e->stats_shards);
     cudaFree(e->h_actions); cudaFree(e->h_noise); cudaFree(e->h_reset); cudaFree(e->h_obs); cudaFree(e->h_next_obs);
     cudaFree(e->h_reward); cudaFree(e->h_hostmask); cudaFree(e->h_flags); cudaFree(e->h_viol); cudaFree(e->h_mask);
+    cudaFree(e->h_terminated); cudaFree(e->h_truncated);
     cudaFree(e->h_i32a); cudaFree(e->h_i32b); cudaFree(e->pid_state); cudaFree(e->tick_dev); cudaFree(e->cons_masks); cudaFree(e->extrema); cudaFree(e->d_len); cudaFree(e->d_off); cudaFree(e->d_total);
     for (int b = 0; b < 2; ++b) {
         cudaFree(e->r_act[b]); cudaFree(e->r_nz[b]);
@@ -907,12 +921,16 @@ int nig_step_host(nig_env_t* e, const nig_step_io_t* io)
     if (io->reward) { if ((rc = dev_alloc(&e->h_reward, cap)) != NIG_OK) return rc; d.reward = e->h_reward; }
     if (io->flags) { if ((rc = dev_alloc(&e->h_flags, cap)) != NIG_OK) return rc; d.flags = e->h_flags; }
     if (io->viol_mask) { if ((rc = dev_alloc(&e->h_viol, cap)) != NIG_OK) return rc; d.viol_mask = e->h_viol; }
+    if (io->terminated) { if ((rc = dev_alloc(&e->h_terminated, cap)) != NIG_OK) return rc; d.terminated = e->h_terminated; }
+    if (io->truncated) { if ((rc = dev_alloc(&e->h_truncated, cap)) != NIG_OK) return rc; d.truncated = e->h_truncated; }
     if ((rc = nig_step(e, &d, st)) != NIG_OK) return rc;
     if (io->obs) NIG_CUDA(cudaMemcpyAsync(io->obs, e->h_obs, n * e->S * sizeof(float), cudaMemcpyDeviceToHost, st));
     if (io->next_obs) NIG_CUDA(cudaMemcpyAsync(io->next_obs, e->h_next_obs, n * e->S * sizeof(float), cudaMemcpyDeviceToHost, st));
     if (io->reward) NIG_CUDA(cudaMemcpyAsync(io->reward, e->h_reward, n * sizeof(float), cudaMemcpyDeviceToHost, st));
     if (io->flags) NIG_CUDA(cudaMemcpyAsync(io->flags, e->h_flags, n, cudaMemcpyDeviceToHost, st));
     if (io->viol_mask) NIG_CUDA(cudaMemcpyAsync(io->viol_mask, e->h_viol, n, cudaMemcpyDeviceToHost, st));
+    if (io->terminated) NIG_CUDA(cudaMemcpyAsync(io->terminated, e->h_terminated, n, cudaMemcpyDeviceToHost, st));
+    if (io->truncated) NIG_CUDA(cudaMemcpyAsync(io->truncated, e->h_truncated, n, cudaMemcpyDeviceToHost, st));
     NIG_CUDA(cudaStreamSynchronize(st));
     return NIG_OK;
 }

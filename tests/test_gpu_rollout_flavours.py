@@ -8,7 +8,7 @@ target silently when a dispatch threshold moves."""
 import numpy as np
 import pytest
 
-from util import KINDS, assert_bits_equal
+from util import KINDS, Track, adversarial, assert_bits_equal, compare_state, compare_stats
 
 pytestmark = pytest.mark.gpu
 
@@ -24,146 +24,9 @@ def mods():
     return ni, N, O, torch
 
 
-def _popcount8(v):
-    return np.unpackbits(np.ascontiguousarray(v, np.uint8)[:, None], axis=1).sum(1, dtype=np.int64)
-
-
-class _Track:
-    """Steps the oracle one tick at a time and keeps what a fused launch reports: per-env reward sum (fp32, sequential
-    within the launch), violation and done counts; and, over a statistics window (up to clear()), successes, episode
-    length sum / square, the fp64 return sum / square, the fp64 reward sum and the return extrema. Returns accumulate in
-    the env's accumulator type (fp32 reactor, fp64 grid / robot); a NaN return is skipped by the extrema like the kernels'
-    compare-selects skip it."""
-
-    def __init__(self, orc, name):
-        self.orc, self.reactor = orc, name == "reactor"
-        self.acc_t = np.float32 if self.reactor else np.float64
-        self.ep_ret = np.zeros(orc.n, self.acc_t)
-        self.clear()
-
-    def clear(self):
-        self.orc.stats[:] = 0
-        self.succ = self.len_sum = self.len_sq = 0
-        self.ret_sum = self.ret_sq = self.rew_sum = 0.0
-        self.ret_abs = self.rew_abs = 0.0           # sums of magnitudes (tolerance scale of the fp64 sums)
-        self.lo, self.hi = np.inf, -np.inf
-
-    def launch(self, K, policy):
-        orc, n = self.orc, self.orc.n
-        rsum = np.zeros(n, np.float32)
-        vcnt = np.zeros(n, np.int64)
-        dcnt = np.zeros(n, np.int64)
-        for _ in range(K):
-            a = policy()
-            steps_before = orc.ep_step.copy()
-            _, r, fl, vm = orc.step(a, want_next_obs=False)
-            rsum = (rsum + r).astype(np.float32)
-            if not self.reactor:
-                self.rew_sum += float(r.astype(np.float64).sum())
-                self.rew_abs += float(np.nansum(np.abs(r.astype(np.float64))))
-            self.ep_ret = (self.ep_ret + r.astype(self.acc_t)).astype(self.acc_t)
-            vcnt += _popcount8(vm)
-            done = (fl & 3) > 0
-            dcnt += done
-            if done.any():
-                er = self.ep_ret[done].astype(np.float64)
-                ln = (steps_before[done] + 1).astype(np.int64)
-                self.ret_sum += float(er.sum()); self.ret_sq += float((er * er).sum())
-                self.ret_abs += float(np.nansum(np.abs(er)))
-                self.succ += int((er > 0).sum()); self.len_sum += int(ln.sum()); self.len_sq += int((ln * ln).sum())
-                fin = er[~np.isnan(er)]
-                if fin.size:
-                    self.lo, self.hi = min(self.lo, float(fin.min())), max(self.hi, float(fin.max()))
-                self.ep_ret[done] = 0
-        if self.reactor:            # the kernels add each env's fp32 launch sum to the fp64 reward-sum slot
-            self.rew_sum += float(rsum.astype(np.float64).sum())
-        return rsum, vcnt, dcnt
-
-
-def _close(got, want, rtol, atol, what):
-    if np.isnan(want):
-        assert np.isnan(got), (what, got, want)
-    else:
-        np.testing.assert_allclose(got, want, rtol=rtol, atol=atol, err_msg=what)
-
-
-def _compare_state(env, orc, what):
-    st, ep_step, ep_viol, done = env.get_state_host()
-    assert_bits_equal(st, orc.state, f"{what}: state")
-    assert_bits_equal(ep_step, orc.ep_step, f"{what}: episode step")
-    assert_bits_equal(ep_viol, orc.ep_viol, f"{what}: episode violations")
-    assert_bits_equal(done, orc.done_latch.astype(bool), f"{what}: done latch")
-
-
-def _compare_stats(N, counters, sums, tr, ncons, extrema, what, lohi=None):
-    """Counters [:6], per-constraint counters, episode statistics and fp64 sums of one window against the tracker."""
-    orc = tr.orc
-    assert counters[:6].tolist() == orc.stats[:6].tolist(), (what, counters[:8], orc.stats[:8])
-    assert counters[N.ST_CON0:N.ST_CON0 + ncons].tolist() == orc.stats[8:8 + ncons].tolist(), what
-    assert (int(counters[N.ST_SUCCESSES]), int(counters[N.ST_EP_LEN_SUM]), int(counters[N.ST_EP_LEN_SQ])) == \
-        (tr.succ, tr.len_sum, tr.len_sq), what
-    # grid / robot: the kernels sum unrounded fp64 rewards, the oracle hands them back rounded to fp32 (relative 6e-8
-    # each): bounded by the magnitude of what was summed, as sums of mixed signs may cancel
-    rtol, atol = (1e-9, 1e-6) if tr.reactor else (1e-6, 1e-3)
-    _close(sums[0], tr.ret_sum, rtol, atol + rtol * tr.ret_abs, f"{what}: return sum")
-    _close(sums[1], tr.ret_sq, rtol, atol, f"{what}: return square sum")
-    _close(sums[N.ST_F_REWARD_SUM - 24], tr.rew_sum, rtol, atol + rtol * tr.rew_abs, f"{what}: reward sum")
-    if lohi is not None:
-        lo, hi = lohi
-        if not extrema or tr.lo == np.inf:
-            assert lo is None and hi is None, what
-        else:
-            tol = 1e-15 if tr.reactor else 1e-6
-            np.testing.assert_allclose([lo, hi], [tr.lo, tr.hi], rtol=tol, atol=0 if tr.reactor else 1e-3, err_msg=what)
-
-
 def _compare_window(env, N, tr, ncons, extrema, what):
     counters, sums = env.read_stats()
-    _compare_stats(N, counters, sums, tr, ncons, extrema, what, env.read_extrema())
-
-
-def _adversarial(O, kind, rng, s0, n, max_steps, clean_from=None):
-    """Entry states that spoil whole warps of the loop invariants of the dedicated kernels (see test_gpu_round2.py),
-    episodes about to be truncated, NaN states (and grid states that overflow to NaN) that truncate on their first step,
-    so that a NaN return reaches the fp64 sums of the first launch only. Special envs are drawn from [0, clean_from)."""
-    st = s0.copy()
-    ep_step = np.zeros(n, np.int32)
-    m = n if clean_from is None else clean_from
-
-    def some(k):
-        return rng.choice(m, k, replace=False)
-    if kind == O.REACTOR:
-        st[some(40), 8] = 1.0                      # e-stop already tripped
-        st[some(40), 9] = 1.0                      # alarm latched (inside the invariant)
-        st[some(10), 8] = 0.3                      # fractional and negative-zero latches
-        st[some(10), 9] = 0.7
-        st[some(10), 8] = -0.0
-        st[some(10), 9] = -0.0
-        st[some(30), 0] = rng.uniform(350.0, 356.0, 30).astype(np.float32)     # over the temperature limit
-        st[some(30), 1] = rng.uniform(5.0e5, 5.2e5, 30).astype(np.float32)     # around the pressure limit
-        st[some(10), 0] = 150.0                    # outside the 200 .. 350 K entry range
-        st[some(10), 5] = rng.choice([0.0, 1e-35, 49.0, 50.0, 3e30], 10).astype(np.float32)
-        st[some(5), 4] = 0.0
-    elif kind == O.GRID:
-        st[some(40), 0] = rng.uniform(-1.2, 1.2, 40).astype(np.float32)
-        st[some(6), 0] = np.array([0.5, -0.5, 1.0, -1.0, -0.0, 0.49999997], np.float32)
-        i = some(40); st[i, 1 + rng.integers(0, 8, 40)] = rng.uniform(0.88, 1.12, 40).astype(np.float32)
-        i = some(30); st[i, 9 + rng.integers(0, 8, 30)] = rng.choice([0.0, -0.0, 100.0, 99.5, 0.4, 100.5, -3.0, 1e-30], 30).astype(np.float32)
-        i = some(20); st[i, 17 + rng.integers(0, 8, 20)] = rng.choice([0.0, -0.0, 1e-20, 0.3, 1e30, 3e38, -2.0], 20).astype(np.float32)
-        brink = i                                  # (huge generation overflows to inf / NaN: truncate these on the first step)
-        w = 32 * 7                                 # one warp with zero imbalance and zero frequency (division guard)
-        st[w:w + 32, 0] = 0.0; st[w:w + 32, 9:17] = 50.0; st[w:w + 32, 17:25] = 50.0
-    else:
-        i = some(40); st[i, :3] = rng.uniform(-0.9, 0.9, (40, 3)).astype(np.float32)        # end effector near / past the workspace
-        i = some(40); st[i, 7 + rng.integers(0, 7, 40)] = rng.uniform(-np.pi, np.pi, 40).astype(np.float32)
-        i = some(30); st[i, 18 + rng.integers(0, 3, 30)] = rng.choice([0.0, -0.0, 49.9, 50.0, 79.0, 81.0, -60.0], 30).astype(np.float32)
-    ep_step[some(200)] = rng.integers(max(0, max_steps - 60), max_steps, 200)
-    nan = some(3)
-    st[nan, 0] = np.nan
-    ep_step[nan] = max_steps - 1
-    if kind == O.GRID:
-        ep_step[brink] = max_steps - 1
-    return st, ep_step
+    compare_stats(N, counters, sums, tr, ncons, extrema, what, env.read_extrema())
 
 
 def _start(ni, N, O, kind, n, *, seed, env_id_offset=0, max_episode_steps=None, auto_reset=True, constraints=None,
@@ -203,7 +66,7 @@ def _run_launches(env, orc, tr, N, torch, chunks, policy_id, policy, ncons, extr
         assert_bits_equal(rsum[:n].cpu().numpy(), o_rs, f"{w}: per-env reward sum")
         assert_bits_equal(vcnt[:n].cpu().numpy().astype(np.int64), o_v, f"{w}: per-env violation count")
         assert_bits_equal(dcnt[:n].cpu().numpy().astype(np.int64), o_d, f"{w}: per-env done count")
-        _compare_state(env, orc, w)
+        compare_state(env, orc, w)
         _compare_window(env, N, tr, ncons, extrema, w)
         env.clear_stats()
         tr.clear()
@@ -213,7 +76,7 @@ def _pair_population(O, rng, s0, n, max_steps):
     """The adversarial population in the first 65,536 envs; behind it whole 64-env warps of the pair kernel (32 threads x 2
     envs) with exactly the pair-specific defects: only env 2j outside the invariant, only env 2j + 1, one warp entirely
     outside, and the warp of the unpartnered last env (n odd) spoiled by that env alone."""
-    st, ep_step = _adversarial(O, O.REACTOR, rng, s0, n, max_steps, clean_from=65_536)
+    st, ep_step = adversarial(O, O.REACTOR, rng, s0, n, max_steps, clean_from=65_536)
     w0 = 65_536 // 64 + 10
     for q in range(8):                          # eight warps, each with one defect: env 2j of pair j = 5 + q only ...
         st[64 * (w0 + q) + 2 * (5 + q), 8] = 1.0
@@ -245,7 +108,7 @@ def test_pair_kernel_default_dispatch_vs_oracle(mods, extrema, max_steps):
     st, ep_step = _pair_population(O, np.random.default_rng(12), orc.state.copy(), n, env.max_episode_steps)
     _set_population(env, orc, st, ep_step)
     env.track_extrema(extrema)
-    tr = _Track(orc, "reactor")
+    tr = Track(orc, "reactor")
     _run_launches(env, orc, tr, N, torch, (64, 17, 1, 70), N.POLICY_UNIFORM,
                   lambda: O.policy_actions(orc, O.POLICY_UNIFORM), 3, extrema, what="pair kernel")
     env.close()
@@ -264,12 +127,12 @@ def test_pair_kernel_forced_small_vs_oracle(mods, monkeypatch, block, extrema, a
     n = 4_096 + 37
     env, orc = _start(ni, N, O, O.REACTOR, n, seed=77, env_id_offset=333, max_episode_steps=60, auto_reset=auto_reset)
     rng = np.random.default_rng(block)
-    st, ep_step = _adversarial(O, O.REACTOR, rng, orc.state.copy(), n, 60)
+    st, ep_step = adversarial(O, O.REACTOR, rng, orc.state.copy(), n, 60)
     st[2 * 700, 8] = 1.0; st[2 * 900 + 1, 9] = 0.5; st[64 * 40:64 * 41, 8] = 1.0
     done = None if auto_reset else (rng.random(n) < 0.05).astype(np.uint8)
     _set_population(env, orc, st, ep_step, done)
     env.track_extrema(extrema)
-    tr = _Track(orc, "reactor")
+    tr = Track(orc, "reactor")
     _run_launches(env, orc, tr, N, torch, (64, 17, 1, 70), N.POLICY_UNIFORM,
                   lambda: O.policy_actions(orc, O.POLICY_UNIFORM), 3, extrema, what=f"pair kernel, {block} threads")
     env.close()
@@ -283,7 +146,7 @@ def test_pair_kernel_in_sliced_device_rollout_vs_oracle(mods):
     ni, N, O, torch = mods
     n, T, K = (1 << 20) - 1_000, 150, 64
     env, orc = _start(ni, N, O, O.REACTOR, n, seed=2027, env_id_offset=5, max_episode_steps=100, threads=O.max_threads())
-    tr = _Track(orc, "reactor")
+    tr = Track(orc, "reactor")
     policy = lambda: O.policy_actions(orc, O.POLICY_UNIFORM)
     rsum, vcnt, dcnt = env.empty(), env.empty(dtype=torch.int32), env.empty(dtype=torch.int32)
     for call in range(2):
@@ -297,7 +160,7 @@ def test_pair_kernel_in_sliced_device_rollout_vs_oracle(mods):
         w = f"sliced call {call}"
         assert_bits_equal(rsum[:n].cpu().numpy(), total, f"{w}: per-env reward sum")
         assert np.array_equal(vcnt[:n].cpu().numpy(), o_v) and np.array_equal(dcnt[:n].cpu().numpy(), o_d), w
-        _compare_state(env, orc, w)
+        compare_state(env, orc, w)
         _compare_window(env, N, tr, 3, False, w)
         env.clear_stats()
         tr.clear()
@@ -316,7 +179,7 @@ def test_pair_kernel_in_host_rollout_vs_oracle(mods, monkeypatch, direct):
     monkeypatch.setenv("NIG_HOST_DIRECT_MAX_MB", "1e9")
     n, T, K = (1 << 18) + 77, 150, 64
     env, orc = _start(ni, N, O, O.REACTOR, n, seed=88, env_id_offset=3, max_episode_steps=100, threads=O.max_threads())
-    tr = _Track(orc, "reactor")
+    tr = Track(orc, "reactor")
     policy = lambda: O.policy_actions(orc, O.POLICY_UNIFORM)
     for call in range(2):
         out = env.rollout_host(T, N.POLICY_UNIFORM, steps_per_launch=K)
@@ -329,9 +192,9 @@ def test_pair_kernel_in_host_rollout_vs_oracle(mods, monkeypatch, direct):
         assert_bits_equal(out["obs"], orc.state, f"{w}: final observations")
         assert_bits_equal(out["reward_sum"], total, f"{w}: per-env reward sum")
         assert np.array_equal(out["violations"], o_v) and np.array_equal(out["episodes"], o_d), w
-        _compare_state(env, orc, w)
+        compare_state(env, orc, w)
         # the counters / sums a host call returns are the handle's lifetime statistics: the tracker's window spans both calls
-        _compare_stats(N, out["counters"], out["sums"], tr, 3, False, w)
+        compare_stats(N, out["counters"], out["sums"], tr, 3, False, w)
     env.close()
 
 
@@ -392,7 +255,7 @@ def test_pair_kernel_graph_replay_vs_eager_and_oracle(mods, mode):
     assert_bits_equal(sg, se, "state after graph replays vs eager")
     assert np.array_equal(stg, ste) and np.array_equal(vg, ve)
     assert_bits_equal(bufs[0][0][:n].cpu().numpy(), bufs[1][0][:n].cpu().numpy(), "last reward")
-    _compare_state(eager_env, orc, "eager vs oracle")
+    compare_state(eager_env, orc, "eager vs oracle")
     assert_bits_equal(bufs[1][0][:n].cpu().numpy(), o_r, "last reward vs oracle")
     cg, _ = graph_env.read_stats()
     ce, _ = eager_env.read_stats()
@@ -468,7 +331,7 @@ def test_zero_policy_vs_oracle(mods, name, extrema, cons):
     cs = None if cons == "default" else _bound_cons(N, kind)
     env, orc = _start(ni, N, O, kind, n, seed=44, env_id_offset=17, max_episode_steps=50, constraints=cs)
     env.track_extrema(extrema)
-    tr = _Track(orc, name)
+    tr = Track(orc, name)
     _run_launches(env, orc, tr, N, torch, (70, 33), N.POLICY_ZERO, lambda: O.policy_actions(orc, O.POLICY_ZERO),
                   3 if cs is None else 4, extrema, what=f"zero policy, {cons}")
     env.close()
@@ -482,7 +345,7 @@ def test_industrial_env_zero_rollout_vs_oracle(mods):
     orc = O.OracleEnv(O.REACTOR, n, seed=9, env_id0=40, exp_mode=1, max_episode_steps=60)
     orc.reset()
     res = env.rollout(T, "zero", steps_per_launch=K, reset=True)
-    tr = _Track(orc, "reactor")
+    tr = Track(orc, "reactor")
     total, o_v, o_d = None, np.zeros(n, np.int64), np.zeros(n, np.int64)
     for c0 in range(0, T, K):
         part, v, d = tr.launch(min(K, T - c0), lambda: O.policy_actions(orc, O.POLICY_ZERO))
@@ -517,7 +380,7 @@ def test_random_baseline_vs_oracle(mods, name, extrema):
         u = O.policy_actions(orc, O.POLICY_UNIFORM)
         return (mid + (half * u).astype(np.float32)).astype(np.float32)
     env.track_extrema(extrema)
-    tr = _Track(orc, name)
+    tr = Track(orc, name)
     _run_launches(env, orc, tr, N, torch, (70, 33), pid, policy, 3, extrema, params=pp, what="random baseline")
     env.close()
 
@@ -539,7 +402,7 @@ def test_pid_mpc_baselines_with_extrema_and_bound_vs_host_agents(mods, name, kin
     pid, pp = Factory.create(kind, env.S, env.A, **kw).device_policy()
     agents = [Factory.create(kind, env.S, env.A, **kw) for _ in range(n)]
     env.track_extrema(True)
-    tr = _Track(orc, name)
+    tr = Track(orc, name)
     policy = lambda: np.stack([ag.act(o) for ag, o in zip(agents, orc.state)]).astype(np.float32)
     _run_launches(env, orc, tr, N, torch, (45, 32), pid, policy, 4, True, params=pp, what=f"{kind} baseline")
     env.close()
@@ -560,10 +423,10 @@ def test_opt_in_shapes_vs_oracle(mods, monkeypatch, case, extrema):
         monkeypatch.setenv(k, v)
     kind, n = KINDS[name], 4_096 + 37
     env, orc = _start(ni, N, O, kind, n, seed=21, env_id_offset=96, max_episode_steps=60 if name == "reactor" else None)
-    st, ep_step = _adversarial(O, kind, np.random.default_rng(kind + 3), orc.state.copy(), n, env.max_episode_steps)
+    st, ep_step = adversarial(O, kind, np.random.default_rng(kind + 3), orc.state.copy(), n, env.max_episode_steps)
     _set_population(env, orc, st, ep_step)
     env.track_extrema(extrema)
-    tr = _Track(orc, name)
+    tr = Track(orc, name)
     _run_launches(env, orc, tr, N, torch, (48, 17, 1, 64), N.POLICY_UNIFORM,
                   lambda: O.policy_actions(orc, O.POLICY_UNIFORM), 3, extrema, what=case)
     env.close()

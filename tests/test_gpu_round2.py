@@ -6,7 +6,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from util import KINDS, assert_bits_equal
+from util import KINDS, Track, assert_bits_equal, compare_stats
 
 pytestmark = pytest.mark.gpu
 
@@ -119,19 +119,26 @@ def test_grid_fast_loop_from_adversarial_entry_states(mods, monkeypatch, shape):
     env.close()
 
 
-@pytest.mark.parametrize("auto_reset,mode", [(True, "1"), (False, "1"), (True, "2"), (True, "3"), (False, "6"), (True, "6")])
+@pytest.mark.parametrize("auto_reset,mode", [(True, "1"), (False, "1"), (True, "2"), (True, "3"), (False, "6"), (True, "6"),
+                                             (True, None), (False, None), (True, "4"), (False, "4"), (True, "0"), (False, "0")])
 def test_grid_persistent_step_kernel_from_adversarial_states_and_actions(mods, monkeypatch, auto_reset, mode):
     """PowerGrid-v0 single step at a population large enough for the dedicated persistent kernel (lean in-place step with
     per-step guards, generic step_core as the per-warp fallback): out-of-range / non-finite / signed-zero states, NaN /
     infinite / over-range actions, generation-limit violations, envs on the brink of truncation, done latches (auto_reset
     off): rewards, flags, violation masks, states, episode words and counters equal to the oracle's, bit for bit, step after
-    step; and to the one-tile kernel (NIG_GRID_STEP=0) through the same oracle."""
+    step, with the statistics window (episode statistics and fp64 return sums too) after every step; and to the one-tile
+    kernel (NIG_GRID_STEP=0) through the same oracle. The dedicated kernel runs from three tiles per resident CTA: with the
+    default shape (256 threads, two CTAs per SM) from 888 tiles = 227,073 envs on 148 SMs (test_gpu_step_flavours.py's
+    dispatch witness checks that these n reach it)."""
     ni, N, O, torch = mods
-    monkeypatch.setenv("NIG_GRID_STEP", mode)          # CTA shape / table replication of the dedicated kernel
+    if mode is None:                                   # unset: the default shape, as "1"
+        monkeypatch.delenv("NIG_GRID_STEP", raising=False)
+    else:
+        monkeypatch.setenv("NIG_GRID_STEP", mode)      # CTA shape / table replication of the dedicated kernel, "0": off
     rng = np.random.default_rng(17)
-    n, T = 180_011, 7      # (>= 3 tiles of 192 envs per resident CTA: the dedicated kernel)
+    n, T = 262_147, 7      # 1,025 tiles of 256 envs (1,366 of 192, 683 of 384, 2,049 of 128): every shape's dedicated kernel
     env = ni.NativeEnv(N.ENV_POWER_GRID, n, device=0, seed=5, env_id_offset=3, auto_reset=auto_reset)
-    orc = O.OracleEnv(O.GRID, n, seed=5, env_id0=3, exp_mode=1, auto_reset=auto_reset, threads=8)
+    orc = O.OracleEnv(O.GRID, n, seed=5, env_id0=3, exp_mode=1, auto_reset=auto_reset, threads=O.max_threads())
     s0 = env.reset_host()
     assert_bits_equal(s0, orc.reset(), "reset")
     st = s0.copy()
@@ -152,8 +159,10 @@ def test_grid_persistent_step_kernel_from_adversarial_states_and_actions(mods, m
     env.set_state_host(st, ep_step, np.zeros(n, np.int32), np.zeros(n, np.uint8))
     orc.state[:] = st
     orc.ep_step[:] = ep_step
+    tr = Track(orc, "grid")
     dev = env.torch_device()
     rew, fl, vm = env.empty(), env.empty(dtype=torch.uint8), env.empty(dtype=torch.uint8)
+    episodes = 0
     for t in range(T):
         a = rng.uniform(-1.3, 1.3, (n, env.A)).astype(np.float32)
         i = some(50); a[i, rng.integers(0, 8, 50)] = rng.choice([np.nan, np.inf, -np.inf, -0.0, 5.0], 50).astype(np.float32)
@@ -163,7 +172,7 @@ def test_grid_persistent_step_kernel_from_adversarial_states_and_actions(mods, m
         d_a[:, :n] = torch.from_numpy(np.ascontiguousarray(a.T)).to(dev)
         env.step_device(d_a, reward=rew, flags=fl, viol_mask=vm)
         torch.cuda.synchronize()
-        _, o_r, o_fl, o_vm = orc.step(a, want_next_obs=False)
+        _, o_r, o_fl, o_vm = tr.step(a, want_next_obs=False)
         assert_bits_equal(fl[:n].cpu().numpy(), o_fl, f"flags t={t}")
         assert_bits_equal(vm[:n].cpu().numpy(), o_vm, f"viol t={t}")
         g_r = rew[:n].cpu().numpy()
@@ -177,8 +186,12 @@ def test_grid_persistent_step_kernel_from_adversarial_states_and_actions(mods, m
         orc.state[nan_both] = g_st[nan_both]
         _compare(env, orc, N, f"t={t}")
         orc.state[:] = keep
-    d = env.stats_dict()
-    assert d["steps"] > 0 and d["episodes"] > 0
+        counters, sums = env.read_stats()
+        compare_stats(N, counters, sums, tr, 3, False, f"statistics t={t}", reward_sum=False)
+        episodes += int(counters[N.ST_EPISODES])
+        env.clear_stats()
+        tr.clear()
+    assert episodes > 0
     env.close()
 
 
@@ -297,46 +310,56 @@ def test_set_state_restarts_the_episode_return(mods):
 
 
 @pytest.mark.parametrize("n", [1, 130])
-def test_zero_copy_step_writes_nothing_past_n(mods, n):
+def test_zero_copy_step_writes_nothing_past_n(mods, monkeypatch, n):
     """nig_step_host with page-locked buffers runs the kernel directly on them: a C caller may pack reward[n], flags[n],
-    viol_mask[n], next_obs[n][S] back to back in ONE nig_host_alloc block -- nothing may be written past element n - 1 of
-    any of them (ADVICE r01: the padding lanes up to pitch used to store 0.0 rewards / INACTIVE flags over the neighbours)."""
+    viol_mask[n], terminated[n], truncated[n], next_obs[n][S] back to back in ONE nig_host_alloc block -- nothing may be
+    written past element n - 1 of any of them (ADVICE r01: the padding lanes up to pitch used to store 0.0 rewards / INACTIVE
+    flags over the neighbours), whatever NIG_STEP_VEC says (the vector flavours store up to the pitch: AoS calls must not
+    take them)."""
     ni, N, O, torch = mods
     S, A = 12, 3
-    env = ni.NativeEnv(N.ENV_CHEMICAL_REACTOR, n, device=0, seed=2)
-    env.reset_host()
     lib = N.lib()
-    nbytes = 4 * n * A + 4 * n + n + n + 4 * n * S + 4 * n * S + 6 * (64 + 16)
-    block = C.c_void_p()
-    N.check(lib.nig_host_alloc(nbytes, C.byref(block)))
-    buf = np.ctypeslib.as_array(C.cast(block, C.POINTER(C.c_uint8)), shape=(nbytes,))
-    buf[:] = 0xA5
-    off = [0]
+    for vec in (None, "2", "4"):
+        if vec is None:
+            monkeypatch.delenv("NIG_STEP_VEC", raising=False)
+        else:
+            monkeypatch.setenv("NIG_STEP_VEC", vec)         # (read by nig_create)
+        env = ni.NativeEnv(N.ENV_CHEMICAL_REACTOR, n, device=0, seed=2)
+        env.reset_host()
+        nbytes = 4 * n * A + 4 * n + 4 * n + 4 * n * S + 4 * n * S + 8 * (64 + 16)
+        block = C.c_void_p()
+        N.check(lib.nig_host_alloc(nbytes, C.byref(block)))
+        buf = np.ctypeslib.as_array(C.cast(block, C.POINTER(C.c_uint8)), shape=(nbytes,))
+        buf[:] = 0xA5
+        off = [0]
 
-    def carve(count, dtype):
-        a = buf[off[0]:off[0] + count * np.dtype(dtype).itemsize].view(dtype)
-        off[0] += count * np.dtype(dtype).itemsize + 64            # >= 64 canary bytes after every array ...
-        off[0] = (off[0] + 15) // 16 * 16                          # ... and every array aligned like a C caller's would be
-        return a
-    act, rew, fl, vm = carve(n * A, np.float32), carve(n, np.float32), carve(n, np.uint8), carve(n, np.uint8)
-    obs, nxt = carve(n * S, np.float32), carve(n * S, np.float32)
-    act[:] = np.random.default_rng(0).uniform(-1, 1, n * A).astype(np.float32)
-    io = N.StepIO()
-    io.actions, io.reward, io.flags, io.viol_mask = act.ctypes.data, rew.ctypes.data, fl.ctypes.data, vm.ctypes.data
-    io.obs, io.next_obs = obs.ctypes.data, nxt.ctypes.data
-    io.action_layout, io.aux_layout = N.LAYOUT_AOS, N.LAYOUT_AOS
-    launches0 = env.launch_count
-    for _ in range(3):
-        N.check(lib.nig_step_host(env._h, C.byref(io)))
-    assert env.launch_count - launches0 == 3                       # the zero-copy path: one launch per call, no staging kernels
-    used = np.zeros(nbytes, bool)
-    for a in (act, rew, fl, vm, obs, nxt):
-        start = a.ctypes.data - buf.ctypes.data
-        used[start:start + a.nbytes] = True
-    assert (buf[~used] == 0xA5).all(), "bytes outside the caller's arrays were overwritten"
-    assert np.isfinite(rew).all() and (fl != 0xA5).all()
-    N.check(lib.nig_host_free(block))
-    env.close()
+        def carve(count, dtype):
+            a = buf[off[0]:off[0] + count * np.dtype(dtype).itemsize].view(dtype)
+            off[0] += count * np.dtype(dtype).itemsize + 64            # >= 64 canary bytes after every array ...
+            off[0] = (off[0] + 15) // 16 * 16                          # ... and every array aligned like a C caller's would be
+            return a
+        act, rew, fl, vm = carve(n * A, np.float32), carve(n, np.float32), carve(n, np.uint8), carve(n, np.uint8)
+        term, trunc = carve(n, np.uint8), carve(n, np.uint8)
+        obs, nxt = carve(n * S, np.float32), carve(n * S, np.float32)
+        act[:] = np.random.default_rng(0).uniform(-1, 1, n * A).astype(np.float32)
+        io = N.StepIO()
+        io.actions, io.reward, io.flags, io.viol_mask = act.ctypes.data, rew.ctypes.data, fl.ctypes.data, vm.ctypes.data
+        io.terminated, io.truncated = term.ctypes.data, trunc.ctypes.data
+        io.obs, io.next_obs = obs.ctypes.data, nxt.ctypes.data
+        io.action_layout, io.aux_layout = N.LAYOUT_AOS, N.LAYOUT_AOS
+        launches0 = env.launch_count
+        for _ in range(3):
+            N.check(lib.nig_step_host(env._h, C.byref(io)))
+        assert env.launch_count - launches0 == 3                       # the zero-copy path: one launch per call, no staging kernels
+        used = np.zeros(nbytes, bool)
+        for a in (act, rew, fl, vm, term, trunc, obs, nxt):
+            start = a.ctypes.data - buf.ctypes.data
+            used[start:start + a.nbytes] = True
+        assert (buf[~used] == 0xA5).all(), f"NIG_STEP_VEC={vec}: bytes outside the caller's arrays were overwritten"
+        assert np.isfinite(rew).all() and (fl != 0xA5).all()
+        assert np.array_equal(term, (fl & 1) != 0) and np.array_equal(trunc, (fl & 2) != 0), vec
+        N.check(lib.nig_host_free(block))
+        env.close()
 
 
 def test_seeded_reset_is_reproducible(mods):
