@@ -142,9 +142,8 @@ struct nig_env {
     int64_t launches;
     int step_vec;              // 0 = auto
     int rollout_block;         // 0 = 128
-    int rollout_ws;            // warp-specialised reactor rollout kernel (NIG_ROLLOUT_WS)
     int rollout_pair;          // two envs per thread + packed f32x2 (NIG_ROLLOUT_PAIR)
-    int grid_fast;             // PowerGrid-v0 dedicated rollout kernel: 0 off, 1 default shape, 2.. other CTA shapes (NIG_GRID_FAST)
+    bool grid_fast;            // PowerGrid-v0 dedicated rollout kernel (NIG_GRID_FAST = 0: off)
     int zero_copy;             // 1 (default): small-population *_host steps run in place on page-locked host buffers
     int step_pipe;             // 1 (default): large plain SoA steps take the persistent TMA-pipelined kernel
     PFN_encodeTiled encode_tiled;
@@ -436,13 +435,12 @@ int rollout_range(nig_env* e, const nig_rollout_t* r, cudaStream_t stream, int64
     // on the SMs, measured 7.82 / 7.93 / 7.98e10 env-steps/s for 128 / 64 / 32 threads per CTA at 8 slices of 8,192 envs
     cfg.block = e->rollout_block ? e->rollout_block : (e->kind == NIG_ENV_CHEMICAL_REACTOR && ns <= 16384 ? 32 : 128);
     cfg.extrema = e->track_extrema;
-    cfg.ws = e->rollout_ws != 0 && e->kind == NIG_ENV_CHEMICAL_REACTOR && e->cfg.auto_reset != 0;
     // two envs per thread + packed f32x2 arithmetic: measured +7 .. 8 % from 262,144 envs per launch up, -11 % at 65,536
     // (half the warps: profiles/r02_e_pair_f32x2_ab.txt); NIG_ROLLOUT_PAIR = 0 / 1 forces it off / on
     cfg.pair = (e->rollout_pair == 1 || (e->rollout_pair < 0 && ns >= 131072)) && e->kind == NIG_ENV_CHEMICAL_REACTOR &&
                e->cfg.auto_reset != 0 && (i0 % 2) == 0;
-    // PowerGrid-v0: the dedicated lean kernel (NIG_GRID_FAST = 0 falls back to the generic one, 2.. pick another CTA shape)
-    cfg.grid_fast = (e->kind == NIG_ENV_POWER_GRID && e->cfg.auto_reset != 0) ? e->grid_fast : 0;
+    // PowerGrid-v0: the dedicated lean kernel (NIG_GRID_FAST = 0 falls back to the generic one)
+    cfg.grid_fast = e->grid_fast && e->kind == NIG_ENV_POWER_GRID && e->cfg.auto_reset != 0;
     e->launches++;
     const int64_t extent = (ns + 127) / 128 * 128;          // launch extent; <= the rows' pitch because slices start at multiples of 128
     NIG_CUDA(nig::launch_rollout(e->kind, cfg, extent, a, map, stream));
@@ -684,12 +682,10 @@ int nig_create(const nig_config_t* cfg, nig_env_t** out)
     e->key = RngKey{(uint32_t)cfg->seed, (uint32_t)(cfg->seed >> 32)};
     if (const char* v = getenv("NIG_STEP_VEC")) e->step_vec = atoi(v);
     if (const char* v = getenv("NIG_ROLLOUT_BLOCK")) e->rollout_block = atoi(v);
-    e->rollout_ws = 0;
-    if (const char* v = getenv("NIG_ROLLOUT_WS")) e->rollout_ws = atoi(v);
     e->rollout_pair = -1;            // auto
     if (const char* v = getenv("NIG_ROLLOUT_PAIR")) e->rollout_pair = atoi(v);
-    e->grid_fast = 1;
-    if (const char* v = getenv("NIG_GRID_FAST")) e->grid_fast = atoi(v);
+    e->grid_fast = true;
+    if (const char* v = getenv("NIG_GRID_FAST")) e->grid_fast = atoi(v) != 0;
     e->host_graph_enable = 1;
     if (const char* v = getenv("NIG_HOST_GRAPH")) e->host_graph_enable = atoi(v);
     e->host_direct = 3;

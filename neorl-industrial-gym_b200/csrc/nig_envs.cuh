@@ -103,12 +103,9 @@ struct Reactor {
     // the reactor (7.0 -> 6.8 -> 6.3e10 env-steps/s at 1M envs for 4 / 6 / 8 CTAs)
     static constexpr int ROLLOUT_MIN_CTAS = 1;
     static constexpr bool TAB_SMEM = false;          // 2 normals per step: the L1-cached global table is as fast, no staging prologue
-#ifndef NIG_REACTOR_ROLLOUT_TAB_SMEM
-#define NIG_REACTOR_ROLLOUT_TAB_SMEM 1
-#endif
     // the fused rollout reads a shared-memory copy of the table: LEA.HI + LDS.128 [R.X16] instead of LEA.HI + IMAD.WIDE (a
     // quarter-rate instruction) + LDG per normal; measured +5 % at 65,536 envs, +1.4 % at 1M (gpurun_out r2_ab1)
-    static constexpr bool ROLLOUT_TAB_SMEM = NIG_REACTOR_ROLLOUT_TAB_SMEM != 0;
+    static constexpr bool ROLLOUT_TAB_SMEM = true;
     static constexpr int STEP_MIN_CTAS = 1;
     __device__ static __forceinline__ void reset_from_normals(const float (&z)[8], float (&s)[S])
     {
@@ -415,10 +412,7 @@ struct Robot {
     static constexpr bool FAST_DIV = false;          // fp64 divisions only
     static constexpr bool COOP_RESET = false;
     static constexpr int COOP_BLOCKS = 0;
-#ifndef NIG_ROBOT_COOP_FK
-#define NIG_ROBOT_COOP_FK 1
-#endif
-    static constexpr bool COOP_FK = NIG_ROBOT_COOP_FK != 0;   // warp-cooperative forward kinematics of the reset (coop_reset_fk)
+    static constexpr bool COOP_FK = true;            // warp-cooperative forward kinematics of the reset (coop_reset_fk)
     static constexpr bool TAB_SMEM = false;          // normals only in reset / policy draws
     static constexpr bool ROLLOUT_TAB_SMEM = false;
     static constexpr int ROLLOUT_MIN_CTAS = 4;       // 177 -> 128 registers: 1.76 -> 2.05e10 env-steps/s at 1M envs

@@ -1317,10 +1317,6 @@ __device__ __forceinline__ void policy_baseline(const Rng& key, const nig_baseli
 // in the same order -> bit-identical results (tests/test_gpu_parity.py compares with the oracle, which knows nothing of
 // this). If a guard fails (never observed: it takes |T' - 320| > 120 K, a pressure outside [1e3, 1e7] Pa or a denormal
 // heat balance) the warp leaves the loop WITHOUT committing the step and the generic loop carries on from there.
-#ifndef NIG_FAST_UNROLL
-#define NIG_FAST_UNROLL 1
-#endif
-constexpr int kFastUnroll = NIG_FAST_UNROLL;
 __device__ __forceinline__ float cdiv_noguard(float x, float c, float rc)
 {
     const float q = __fmul_rn(x, rc);
@@ -1608,17 +1604,13 @@ __device__ __forceinline__ int reactor_fast_steps_v(Src& src, const Rng& key, co
     // normals and the action scaling leave the head of the step's dependency chain and fill the physics' issue gaps instead.
     // Measured +6.3 % at 65,536 envs (3.5 warps per sub-partition: latency shows), -12 % in the two-env flavour (12 more live
     // registers), so one env per thread only (profiles/r02_h_draw_ahead_ab.txt)
-#ifdef NIG_NO_DRAW_AHEAD
-    constexpr bool kAhead = false;
-#else
     constexpr bool kAhead = Src::kPure && N == 1;
-#endif
     StepDraw nxt[N];
     if constexpr (kAhead) {
 #pragma unroll
         for (int k = 0; k < N; ++k) nxt[k] = src.get(0, k);
     }
-#pragma unroll kFastUnroll
+#pragma unroll 1
     for (; t < n_steps; ++t) {
         const uint32_t tick = tick0 + (uint32_t)t;
         V nz0, nz1, hp, cadj, fadj, apen;
@@ -2410,66 +2402,9 @@ __global__ void __launch_bounds__(kThreads, Env::ROLLOUT_MIN_CTAS) rollout_kerne
     rollout_epilogue<Env, EXTREMA>(p, bs, sfl, sext, valid, i, s, ep_st, ep_vi, latched, ep_ret, rsum, acc, r_lo, r_hi);
 }
 
-// ================================================================================================
-// fused K-step rollout, warp-specialised flavour (ChemicalReactor-v0, the benchmark's configuration)
-// ================================================================================================
-// 65,536 envs are 2,048 warps on 592 SM sub-partitions: 3.5 warps each, every one a long dependent chain (Philox rounds ->
-// table normal -> heat balance -> T' -> T'/T -> P' -> relief valve -> reward sum), and the issue slots stay ~30 % empty.
-// The random inputs of a step depend on nothing but (env, tick), so they are split off: in every 96-thread CTA warp 0 is a
-// PRODUCER that draws, for the CTA's 64 envs (two per lane), the step's Philox block, the two table normals and the three
-// uniform actions and stores the six derived values (StepDraw) into a shared-memory ring; warps 1 and 2 are CONSUMERS that
-// run the invariant-specialised physics loop (reactor_fast_steps) with their draws read back from the ring (3 LDS.64 per
-// step). Producer and consumers meet at two mbarriers per ring slot (kWsG steps): `full` (32 producer lanes arrive after
-// their stores) and `empty` (the consumer lanes arrive after their loads). That makes 3,072 resident warps for the same
-// envs (5.2 per sub-partition), takes the longest-latency chain (Philox -> normals) off the consumers' critical path, and
-// the arithmetic is untouched: the same StepDraw values, bit for bit, reach the same instructions.
-// A consumer warp whose envs do not satisfy the loop invariants (or that leaves the loop on a failed guard) steps through
-// the generic path with its own in-place draws, like in rollout_kernel.
-constexpr int kWsG = 4;            // steps per ring slot
-constexpr int kWsSlots = 2;        // ring slots
-constexpr int kWsEnvs = 64;        // envs per CTA
-constexpr int kWsThreads = 96;     // producer warp + two consumer warps
-
-struct DrawFromRing {
-    static constexpr bool kPure = false, kUserActions = false;
-    const float2* lane_base;       // ring + this consumer lane's env index within the CTA; layout [slot][g][3][kWsEnvs]
-    uint64_t* full; uint64_t* empty;
-    __device__ __forceinline__ void wait_full(int t) const
-    {
-        const int q = t / kWsG;
-        mbar_wait(&full[q % kWsSlots], (uint32_t)((q / kWsSlots) & 1));
-    }
-    __device__ __forceinline__ void arrive_empty(int t) const
-    {
-        asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&empty[(t / kWsG) % kWsSlots])) : "memory");
-    }
-    __device__ __forceinline__ StepDraw get(int t, int) const
-    {
-        const int g = t % kWsG;
-        if (g == 0) wait_full(t);
-        const float2* b = lane_base + (((t / kWsG) % kWsSlots) * kWsG + g) * 3 * kWsEnvs;
-        const float2 v0 = b[0], v1 = b[kWsEnvs], v2 = b[2 * kWsEnvs];
-        StepDraw d;
-        d.hp = v0.x; d.cadj = v0.y; d.fadj = v1.x; d.apen = v1.y; d.nz0 = v2.x; d.nz1 = v2.y;
-        return d;
-    }
-    __device__ __forceinline__ void done(int t, int n_steps) const
-    {
-        if (t % kWsG == kWsG - 1 || t == n_steps - 1) arrive_empty(t);
-    }
-    // keep the handshake going without computing (a consumer that left the fast loop at step t_from, whose draw it had
-    // already fetched): the producer runs a fixed schedule and must not be left waiting for a slot
-    __device__ __forceinline__ void drain(int t_from, int n_steps) const
-    {
-        for (int t = t_from; t < n_steps; ++t) {
-            if (t != t_from && t % kWsG == 0) wait_full(t);
-            done(t, n_steps);
-        }
-    }
-};
-
 // one generic step of the uniform-random rollout with in-place draws: the loop body of rollout_kernel for POLICY_UNIFORM
-// (envs without a block-cooperative reset), used by the warp-specialised kernel where a warp cannot take the fast loop
+// (envs without a block-cooperative reset), used by rollout_grid_kernel and rollout_reactor_pair_kernel where a warp cannot
+// take the fast loop
 template <class Env, int CONS, bool EXTREMA>
 __device__ __forceinline__ void rollout_generic_uniform_step(const RolloutArgs& p, const Rng& key, uint32_t env, uint32_t tick, uint32_t epoch, bool valid,
                                                              float (&s)[Env::S], uint32_t& ep_st, uint32_t& ep_vi, bool& latched,
@@ -2519,104 +2454,6 @@ __device__ __forceinline__ void rollout_generic_uniform_step(const RolloutArgs& 
             for (int k = 0; k < S; ++k) s[k] = ns[k];
         }
     }
-}
-
-template <bool EXTREMA>
-__global__ void __launch_bounds__(kWsThreads, 7) rollout_reactor_ws_kernel(const __grid_constant__ RolloutArgs p)
-{
-    using Env = Reactor;
-    constexpr int S = Env::S;
-    __shared__ unsigned int sstat[NIG_STATS_SLOTS];
-    __shared__ double sfl[4];
-    __shared__ unsigned long long sext[2];
-    __shared__ float4 s_tab[NIG_NORMAL_TAB_N];
-    __shared__ alignas(16) float2 ring[kWsSlots * kWsG * 3 * kWsEnvs];
-    __shared__ alignas(8) uint64_t full[kWsSlots], empty[kWsSlots];
-    __shared__ int fast_warp[2];
-    BlockStats bs;
-    if (threadIdx.x < 4) sfl[threadIdx.x] = 0.0;
-    if constexpr (EXTREMA) { if (threadIdx.x < 2) sext[threadIdx.x] = 0ull; }
-    normal_table_to_smem(s_tab);
-    const Rng key(p.key, s_tab);
-    bs.init(sstat);                              // (synchronises the CTA)
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const bool producer = warp == 0;
-    const uint32_t tick0 = load_tick(p.tick_dev, p.tick) + base_tick(p.tick_base);
-    const uint32_t epoch = p.epoch + base_epoch(p.tick_base);
-    // consumer (warp 1, 2): env blockIdx * 64 + (warp - 1) * 32 + lane; the producer's values below are unused
-    const int64_t i = (int64_t)blockIdx.x * kWsEnvs + (producer ? 0 : (warp - 1) * 32) + lane;
-    const bool valid = !producer && i < p.n;
-    const int64_t ic = valid ? i : 0;
-    const uint32_t env = p.env0 + (uint32_t)ic;
-
-    float s[S];
-    uint32_t ep_st = 0, ep_vi = 0;
-    bool latched = false;
-    float ep_ret = 0.0f, rsum = 0.0f, r_lo = INFINITY, r_hi = -INFINITY;
-    RolloutAcc acc;
-#pragma unroll
-    for (int k = 0; k < NIG_MAX_CONSTRAINTS; ++k) acc.c_con[k] = 0;
-    bool fast = false;
-    if (!producer) {
-#pragma unroll
-        for (int k = 0; k < S; ++k) s[k] = p.state[k * p.pitch + ic];
-        const uint32_t w0 = p.ep_word[ic];
-        ep_st = epw_step(w0); ep_vi = epw_viol(w0);
-        latched = (w0 >> 31) != 0u;
-        ep_ret = (float)p.ep_return[ic];
-        const bool inv = valid && !latched && p.auto_reset != 0 && __float_as_uint(s[8]) == 0u &&
-                         (__float_as_uint(s[9]) == 0u || __float_as_uint(s[9]) == 0x3f800000u) &&
-                         s[0] >= 200.0f && s[0] <= 350.0f && s[1] <= 506625.0f && s[5] >= 1e-30f && s[5] <= 1e30f &&
-                         ep_st < (uint32_t)p.max_steps;
-        fast = __all_sync(0xffffffffu, inv);
-        if (lane == 0) fast_warp[warp - 1] = fast ? 1 : 0;
-    } else {
-#pragma unroll
-        for (int k = 0; k < S; ++k) s[k] = 0.0f;
-    }
-    __syncthreads();
-    const int n_fast = fast_warp[0] + fast_warp[1];
-    if (threadIdx.x == 0) {
-#pragma unroll
-        for (int k = 0; k < kWsSlots; ++k) { mbar_init(&full[k], 32); mbar_init(&empty[k], 32 * (n_fast > 0 ? n_fast : 1)); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-
-    if (producer) {
-        if (n_fast > 0) {
-            const uint32_t env_a = p.env0 + (uint32_t)((int64_t)blockIdx.x * kWsEnvs + lane), env_b = env_a + 32u;
-            const int n_slots = (p.n_steps + kWsG - 1) / kWsG;
-#pragma unroll 1
-            for (int q = 0; q < n_slots; ++q) {
-                const int slot = q % kWsSlots;
-                if (q >= kWsSlots) mbar_wait(&empty[slot], (uint32_t)(((q / kWsSlots) - 1) & 1));
-#pragma unroll 1
-                for (int g = 0; g < kWsG; ++g) {
-                    const int t = q * kWsG + g;
-                    if (t >= p.n_steps) break;
-                    float2* b = ring + (slot * kWsG + g) * 3 * kWsEnvs + lane;
-                    const StepDraw da = reactor_step_draw(key, env_a, tick0 + (uint32_t)t);
-                    const StepDraw db = reactor_step_draw(key, env_b, tick0 + (uint32_t)t);
-                    b[0] = make_float2(da.hp, da.cadj); b[kWsEnvs] = make_float2(da.fadj, da.apen); b[2 * kWsEnvs] = make_float2(da.nz0, da.nz1);
-                    b[32] = make_float2(db.hp, db.cadj); b[kWsEnvs + 32] = make_float2(db.fadj, db.apen); b[2 * kWsEnvs + 32] = make_float2(db.nz0, db.nz1);
-                }
-                asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&full[slot])) : "memory");
-            }
-        }
-    } else {
-        int t_begin = 0;
-        if (fast) {
-            DrawFromRing src{ring + (warp - 1) * 32 + lane, full, empty};
-            t_begin = reactor_fast_steps<EXTREMA>(src, key, env, tick0, epoch, p.n_steps, p.max_steps, s, ep_st, ep_vi, ep_ret, rsum, acc, r_lo, r_hi);
-            if (t_begin < p.n_steps) src.drain(t_begin, p.n_steps);
-        }
-#pragma unroll 1
-        for (int t = t_begin; t < p.n_steps; ++t)
-            rollout_generic_uniform_step<Env, CONS_DEFAULT, EXTREMA>(p, key, env, tick0 + (uint32_t)t, epoch, valid, s, ep_st, ep_vi, latched, ep_ret, rsum, acc, r_lo, r_hi);
-    }
-    rollout_epilogue<Env, EXTREMA>(p, bs, sfl, sext, valid, i, s, ep_st, ep_vi, latched, ep_ret, rsum, acc, r_lo, r_hi);
 }
 
 // ================================================================================================

@@ -1,7 +1,6 @@
 // nig_launch.h -- kernel launchers, one translation unit per kernel family so the library builds in parallel
 // (nig_step.cu, nig_rollout_{reactor,grid,robot}.cu, nig_dataset.cu, nig_misc.cu). nig_api.cu holds no kernels.
 #pragma once
-#include <cstdlib>
 #include "nig_kernels.cuh"
 
 namespace nig {
@@ -14,8 +13,7 @@ struct RolloutLaunch {
     int block;         // threads per CTA: 32, 64 or 128
     bool extrema;      // nig_track_extrema: the kernel flavour that also keeps return_min / return_max
     bool pair;         // ChemicalReactor-v0, uniform policy, default constraints: two envs per thread, packed f32x2 arithmetic
-    bool ws;           // ChemicalReactor-v0, uniform policy, default constraints: the warp-specialised kernel (producer / consumers)
-    int grid_fast;     // PowerGrid-v0, uniform policy, default constraints, auto-reset: 0 = generic kernel, 1 + shape = rollout_grid_kernel
+    bool grid_fast;    // PowerGrid-v0, uniform policy, default constraints, auto-reset: rollout_grid_kernel instead of the generic kernel
 };
 
 cudaError_t launch_step(int kind, int vec, int cons, int64_t pitch, const StepArgs& a, cudaStream_t st, bool plain);
@@ -41,16 +39,15 @@ cudaError_t launch_selftest_division(RngKey key, int iters, int blocks, unsigned
 inline unsigned grid_for(int64_t items, int block = kThreads) { return (unsigned)((items + block - 1) / block); }
 
 // launch of a kernel that executes griddepcontrol.wait before its first dependent read (rollout_pdl_sync): programmatic
-// stream serialisation lets its prologue overlap the tail of the previous launch on the stream (NIG_ROLLOUT_PDL=0: off)
+// stream serialisation lets its prologue overlap the tail of the previous launch on the stream
 template <class Kern, class... Args>
 cudaError_t launch_pdl(Kern kern, unsigned grid, unsigned block, size_t smem, cudaStream_t st, const Args&... args)
 {
-    static const bool pdl = [] { const char* v = getenv("NIG_ROLLOUT_PDL"); return v ? atoi(v) != 0 : true; }();
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(grid); cfg.blockDim = dim3(block); cfg.dynamicSmemBytes = smem; cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = pdl ? 1 : 0;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kern, args...);
 }

@@ -1,10 +1,12 @@
 // fused K-step rollout kernels of Grid (see nig_kernels.cuh)
 #include "nig_rollout_launch.cuh"
-#include <cstdlib>
 namespace nig {
-template <bool EXTREMA, int THREADS, int MAXREG>
-static cudaError_t grid_fast_go(int64_t pitch, const RolloutArgs& a, cudaStream_t st)
+// 192 threads per CTA x 168 registers per thread: two CTAs / SM, 12 warps, no spills, the fastest of the CTA shapes measured
+// at 1M envs (profiles/r02_f_grid_rollout_ab.txt)
+template <bool EXTREMA>
+static cudaError_t grid_fast(int64_t pitch, const RolloutArgs& a, cudaStream_t st)
 {
+    constexpr int THREADS = 192, MAXREG = 168;
     auto kern = rollout_grid_kernel<EXTREMA, THREADS, MAXREG>;
     constexpr size_t smem = grid_rollout_smem<THREADS>();
     static bool attr_set[64] = {false};           // the attribute is per function and per device: set once for each
@@ -18,21 +20,10 @@ static cudaError_t grid_fast_go(int64_t pitch, const RolloutArgs& a, cudaStream_
     }
     return launch_pdl(kern, grid_for(pitch, THREADS), (unsigned)THREADS, smem, st, a);
 }
-template <bool EXTREMA>
-static cudaError_t grid_fast(int shape, int64_t pitch, const RolloutArgs& a, cudaStream_t st)
-{
-    switch (shape) {                              // (threads per CTA, registers per thread): resident CTAs follow from both
-    case 1: return grid_fast_go<EXTREMA, 512, 128>(pitch, a, st);
-    case 2: return grid_fast_go<EXTREMA, 384, 168>(pitch, a, st);
-    case 3: return grid_fast_go<EXTREMA, 640, 96>(pitch, a, st);
-    case 4: return grid_fast_go<EXTREMA, 256, 128>(pitch, a, st);
-    default: return grid_fast_go<EXTREMA, 192, 168>(pitch, a, st);      // two CTAs / SM, 12 warps, no spills: the fastest measured
-    }
-}
 cudaError_t launch_rollout_grid(const RolloutLaunch& cfg, int64_t pitch, const RolloutArgs& a, const CUtensorMap& map, cudaStream_t st)
 {
     if (cfg.grid_fast && cfg.policy == NIG_POLICY_UNIFORM && cfg.cons == CONS_DEFAULT && !cfg.tma && !cfg.tf_noise)
-        return cfg.extrema ? grid_fast<true>(cfg.grid_fast - 1, pitch, a, st) : grid_fast<false>(cfg.grid_fast - 1, pitch, a, st);
+        return cfg.extrema ? grid_fast<true>(pitch, a, st) : grid_fast<false>(pitch, a, st);
     return rollout_env<Grid>(cfg, pitch, a, map, st);
 }
 } // namespace nig

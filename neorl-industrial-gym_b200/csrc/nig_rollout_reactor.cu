@@ -8,12 +8,6 @@ cudaError_t launch_rollout_reactor(const RolloutLaunch& cfg, int64_t pitch, cons
         return cfg.extrema ? launch_pdl(rollout_reactor_pair_kernel<true>, grid, (unsigned)cfg.block, 0, st, a)
                            : launch_pdl(rollout_reactor_pair_kernel<false>, grid, (unsigned)cfg.block, 0, st, a);
     }
-    if (cfg.ws && cfg.policy == NIG_POLICY_UNIFORM && cfg.cons == CONS_DEFAULT && !cfg.tma && !cfg.tf_noise) {
-        const unsigned grid = (unsigned)((pitch + kWsEnvs - 1) / kWsEnvs);
-        if (cfg.extrema) rollout_reactor_ws_kernel<true><<<grid, kWsThreads, 0, st>>>(a);
-        else rollout_reactor_ws_kernel<false><<<grid, kWsThreads, 0, st>>>(a);
-        return cudaGetLastError();
-    }
     return rollout_env<Reactor>(cfg, pitch, a, map, st);
 }
 } // namespace nig

@@ -12,12 +12,11 @@ cudaError_t go(int cons, int64_t pitch, const StepArgs& a, cudaStream_t st, bool
         if (plain && cons == CONS_DEFAULT) {
             // launched with programmatic stream serialisation: back-to-back steps (a captured graph of them above all) overlap
             // the launch latency and prologue of step t + 1 with the tail of step t (griddepcontrol.wait in the kernel)
-            static const bool pdl = [] { const char* v = getenv("NIG_STEP_PDL"); return v ? atoi(v) != 0 : true; }();
             cudaLaunchConfig_t cfg{};
             cfg.gridDim = dim3(g); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = 0; cfg.stream = st;
             cudaLaunchAttribute attr[1];
             attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-            attr[0].val.programmaticStreamSerializationAllowed = pdl ? 1 : 0;
+            attr[0].val.programmaticStreamSerializationAllowed = 1;
             cfg.attrs = attr; cfg.numAttrs = 1;
             return cudaLaunchKernelEx(&cfg, step_kernel<Env, 1, CONS_DEFAULT, true>, a);
         }
@@ -63,12 +62,16 @@ cudaError_t go_pipe_t(int64_t pitch, const StepArgs& a, cudaStream_t st, bool* u
     return cudaGetLastError();
 }
 
-// PowerGrid-v0: the dedicated persistent single-step kernel (NIG_GRID_STEP = 0: off, 1 / unset: the default shape, 2.. other
-// CTA shapes / table replications, see go_grid); gridDim = the CTAs resident on the device
-template <int THREADS, int REGS, int REP>
-cudaError_t go_grid_t(int64_t pitch, const StepArgs& a, cudaStream_t st, bool* used)
+// PowerGrid-v0: the dedicated persistent single-step kernel (NIG_GRID_STEP = 0: off); gridDim = the CTAs resident on the
+// device. CTA shapes <threads, registers, normal-table replication> measured at 1M / 4M envs, us per launch
+// (profiles/r02_f_grid_step_ab.txt): <256, 128, 4> 82.9 / 280 (two CTAs per SM, 16 warps, 8 B of spills), <128, 168, 4>
+// 87.0 / 308 (three CTAs per SM, 12 warps, table copies shared by lane pairs), <192, 168, 4> 89.1, <192, 168, 8>
+// 89.1 / 304 (two CTAs per SM, 12 warps), <384, 168, 8> 93.2 / 313 (one CTA per SM, 12 warps). The first is the one built.
+cudaError_t go_grid(int64_t pitch, const StepArgs& a, cudaStream_t st, bool* used)
 {
-    static const bool pdl = [] { const char* v = getenv("NIG_STEP_PDL"); return v ? atoi(v) != 0 : true; }();
+    const char* const v = getenv("NIG_GRID_STEP");         // (read per launch: the tests switch kernels inside one process)
+    if (v && atoi(v) == 0) return cudaSuccess;
+    constexpr int THREADS = 256, REGS = 128, REP = 4;
     static int cache[64] = {0};
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
@@ -89,23 +92,10 @@ cudaError_t go_grid_t(int64_t pitch, const StepArgs& a, cudaStream_t st, bool* u
     cfg.gridDim = dim3((unsigned)cache[dev]); cfg.blockDim = dim3(THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = pdl ? 1 : 0;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
     *used = true;
     return cudaLaunchKernelEx(&cfg, kern, a);
-}
-cudaError_t go_grid(int64_t pitch, const StepArgs& a, cudaStream_t st, bool* used)
-{
-    const char* const v = getenv("NIG_GRID_STEP");         // (read per launch: the tests switch shapes inside one process)
-    const int mode = v ? atoi(v) : 1;
-    if (mode == 0) return cudaSuccess;
-    switch (mode) {                   // measured at 1M / 4M envs (profiles/r02_f_grid_step_ab.txt): us per launch
-    case 2: return go_grid_t<384, 168, 8>(pitch, a, st, used);      // 93.2 / 313   one CTA per SM, 12 warps
-    case 3: return go_grid_t<128, 168, 4>(pitch, a, st, used);      // 87.0 / 308   three CTAs per SM, 12 warps, table copies shared by lane pairs
-    case 4: return go_grid_t<192, 168, 4>(pitch, a, st, used);      // 89.1
-    case 6: return go_grid_t<192, 168, 8>(pitch, a, st, used);      // 89.1 / 304   two CTAs per SM, 12 warps
-    default: return go_grid_t<256, 128, 4>(pitch, a, st, used);     // 82.9 / 280   two CTAs per SM, 16 warps (8 B of spills)
-    }
 }
 
 template <class Env, int VEC>
@@ -140,7 +130,7 @@ cudaError_t launch_step_pipelined(int kind, int cons, int64_t pitch, const StepA
     default:
         // PowerGrid (23 Gaussian draws per step, block-cooperative reset buffer) is latency-bound at the pipeline's two
         // resident CTAs per SM (115 -> 136 us at 1M envs): with the env's default constraints it takes its own persistent
-        // kernel (lean in-place step, 8 x replicated normal table), otherwise step_kernel.
+        // kernel (lean in-place step, 4 x replicated normal table), otherwise step_kernel.
         *used = false;
         if (cons == CONS_DEFAULT) return go_grid(pitch, a, st, used);
         return cudaSuccess;

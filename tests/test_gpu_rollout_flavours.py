@@ -1,10 +1,10 @@
 """Fused-rollout kernel flavours that only a size, an environment variable, a policy or a constraint set selects: the
 two-env packed f32x2 reactor kernel (chosen by default from 131,072 envs per launch, also inside nig_rollout_steps and
 nig_rollout_host slices and CUDA graphs), NIG_POLICY_ZERO, the in-kernel baseline controllers with return extrema and
-appended bounds, the warp-specialised reactor kernel, the PowerGrid CTA shape NIG_GRID_FAST=5 and 64-thread CTAs of the
-generic kernel. Every result is compared with the CPU oracle (spec-exp mode) bit for bit; the fp64 statistics to the
-tolerances of tests/test_gpu_parity.py. A dispatch witness records kernel names so that these tests cannot lose their
-target silently when a dispatch threshold moves."""
+appended bounds, and 64-thread CTAs of the generic kernel; also the default reactor and PowerGrid kernels from
+adversarial populations with return extrema. Every result is compared with the CPU oracle (spec-exp mode) bit for bit;
+the fp64 statistics to the tolerances of tests/test_gpu_parity.py. A dispatch witness records kernel names so that these
+tests cannot lose their target silently when a dispatch threshold moves."""
 import numpy as np
 import pytest
 
@@ -302,10 +302,8 @@ def test_dispatch_witness(mods, monkeypatch):
     assert not has(off, "rollout_reactor_pair_kernel") and has(off, "rollout_kernel"), sorted(off)
     sliced = names_of(N.ENV_CHEMICAL_REACTOR, (1 << 20) - 1_000, lambda e: e.rollout_steps_device(64, 64, N.POLICY_UNIFORM))
     assert has(sliced, "rollout_reactor_pair_kernel") and has(sliced, "rollout_kernel"), sorted(sliced)
-    ws = names_of(N.ENV_CHEMICAL_REACTOR, 4_133, one, NIG_ROLLOUT_WS="1")
-    assert has(ws, "rollout_reactor_ws_kernel"), sorted(ws)
-    grid = names_of(N.ENV_POWER_GRID, 4_133, one, NIG_GRID_FAST="5")
-    assert any("rollout_grid_kernel" in x and "256" in x for x in grid), sorted(grid)
+    grid = names_of(N.ENV_POWER_GRID, 4_133, one)
+    assert any("rollout_grid_kernel" in x and "192" in x for x in grid), sorted(grid)
     small = names_of(N.ENV_CHEMICAL_REACTOR, 4_133, one, NIG_ROLLOUT_PAIR="1", NIG_ROLLOUT_BLOCK="32")
     assert has(small, "rollout_reactor_pair_kernel"), sorted(small)
 
@@ -408,15 +406,16 @@ def test_pid_mpc_baselines_with_extrema_and_bound_vs_host_agents(mods, name, kin
     env.close()
 
 
-# 7. opt-in kernel shapes
+# 7. default and opt-in kernel shapes
 @pytest.mark.parametrize("extrema", [False, True])
-@pytest.mark.parametrize("case", ["reactor_ws", "grid_fast5", "grid_block64", "robot_block64"])
+@pytest.mark.parametrize("case", ["reactor_default", "grid_default", "grid_block64", "robot_block64"])
 def test_opt_in_shapes_vs_oracle(mods, monkeypatch, case, extrema):
-    """NIG_ROLLOUT_WS=1 (warp-specialised reactor kernel), NIG_GRID_FAST=5 (PowerGrid kernel, 256-thread CTAs) and
-    NIG_ROLLOUT_BLOCK=64 (generic kernel of the grid and the robot) from adversarial populations == the oracle."""
+    """The default dispatch of the reactor (rollout_kernel<Reactor>, one-warp CTAs at this size) and of PowerGrid
+    (rollout_grid_kernel, 192-thread CTAs), and NIG_ROLLOUT_BLOCK=64 (generic kernel of the grid and the robot), from
+    adversarial populations == the oracle."""
     ni, N, O, torch = mods
-    name, envvars = {"reactor_ws": ("reactor", {"NIG_ROLLOUT_WS": "1"}),
-                     "grid_fast5": ("grid", {"NIG_GRID_FAST": "5"}),
+    name, envvars = {"reactor_default": ("reactor", {}),
+                     "grid_default": ("grid", {}),
                      "grid_block64": ("grid", {"NIG_GRID_FAST": "0", "NIG_ROLLOUT_BLOCK": "64"}),
                      "robot_block64": ("robot", {"NIG_ROLLOUT_BLOCK": "64"})}[case]
     for k, v in envvars.items():

@@ -73,13 +73,13 @@ def test_reactor_fast_loop_from_adversarial_entry_states(mods):
     env.close()
 
 
-@pytest.mark.parametrize("shape", ["1", "2", "3", "4", "0"])
+@pytest.mark.parametrize("shape", ["1", "0"])
 def test_grid_fast_loop_from_adversarial_entry_states(mods, monkeypatch, shape):
     """PowerGrid-v0: the dedicated lean rollout kernel (in-place step, min / max trees for the voltage ranges, max / min
     clamps, 8 x replicated normal table, rank-dealt cooperative reset) enters its loop per warp only when every env of the
     warp satisfies the invariants; these populations mix such warps with warps holding out-of-range / non-finite / signed-zero
-    states and episodes about to be truncated. Everything must be the oracle's, bit for bit, for every CTA shape and for the
-    generic kernel (NIG_GRID_FAST=0) alike; per-env sums, counters and episode statistics included."""
+    states and episodes about to be truncated. Everything must be the oracle's, bit for bit, for the dedicated kernel and
+    for the generic kernel (NIG_GRID_FAST=0) alike; per-env sums, counters and episode statistics included."""
     ni, N, O, torch = mods
     monkeypatch.setenv("NIG_GRID_FAST", shape)
     rng = np.random.default_rng(11)
@@ -119,24 +119,23 @@ def test_grid_fast_loop_from_adversarial_entry_states(mods, monkeypatch, shape):
     env.close()
 
 
-@pytest.mark.parametrize("auto_reset,mode", [(True, "1"), (False, "1"), (True, "2"), (True, "3"), (False, "6"), (True, "6"),
-                                             (True, None), (False, None), (True, "4"), (False, "4"), (True, "0"), (False, "0")])
+@pytest.mark.parametrize("auto_reset,mode", [(True, "1"), (False, "1"), (True, None), (False, None), (True, "0"), (False, "0")])
 def test_grid_persistent_step_kernel_from_adversarial_states_and_actions(mods, monkeypatch, auto_reset, mode):
     """PowerGrid-v0 single step at a population large enough for the dedicated persistent kernel (lean in-place step with
     per-step guards, generic step_core as the per-warp fallback): out-of-range / non-finite / signed-zero states, NaN /
     infinite / over-range actions, generation-limit violations, envs on the brink of truncation, done latches (auto_reset
     off): rewards, flags, violation masks, states, episode words and counters equal to the oracle's, bit for bit, step after
     step, with the statistics window (episode statistics and fp64 return sums too) after every step; and to the one-tile
-    kernel (NIG_GRID_STEP=0) through the same oracle. The dedicated kernel runs from three tiles per resident CTA: with the
-    default shape (256 threads, two CTAs per SM) from 888 tiles = 227,073 envs on 148 SMs (test_gpu_step_flavours.py's
+    kernel (NIG_GRID_STEP=0) through the same oracle. The dedicated kernel runs from three tiles per resident CTA: with
+    256-thread CTAs, two per SM, from 888 tiles = 227,073 envs on 148 SMs (test_gpu_step_flavours.py's
     dispatch witness checks that these n reach it)."""
     ni, N, O, torch = mods
-    if mode is None:                                   # unset: the default shape, as "1"
+    if mode is None:                                   # unset: the dedicated kernel, as "1"
         monkeypatch.delenv("NIG_GRID_STEP", raising=False)
     else:
-        monkeypatch.setenv("NIG_GRID_STEP", mode)      # CTA shape / table replication of the dedicated kernel, "0": off
+        monkeypatch.setenv("NIG_GRID_STEP", mode)      # "0": off
     rng = np.random.default_rng(17)
-    n, T = 262_147, 7      # 1,025 tiles of 256 envs (1,366 of 192, 683 of 384, 2,049 of 128): every shape's dedicated kernel
+    n, T = 262_147, 7      # 1,025 tiles of 256 envs: the dedicated kernel
     env = ni.NativeEnv(N.ENV_POWER_GRID, n, device=0, seed=5, env_id_offset=3, auto_reset=auto_reset)
     orc = O.OracleEnv(O.GRID, n, seed=5, env_id0=3, exp_mode=1, auto_reset=auto_reset, threads=O.max_threads())
     s0 = env.reset_host()

@@ -1,5 +1,5 @@
 """PowerGrid-v0 / RobotAssembly-v0 fused rollout throughput (uniform policy, K = 64, 256 steps per pass):
-   python tools/grid_ab.py [kind=1] [n_envs ...]    (NIG_GRID_FAST = 0 generic kernel / 1.. CTA shapes of the dedicated kernel)"""
+   python tools/grid_ab.py [kind=1] [n_envs ...]    (NIG_GRID_FAST = 0 generic kernel / 1 the dedicated kernel)"""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "neorl-industrial-gym_b200")]

@@ -1,5 +1,5 @@
 """The single-step kernel at the BASELINE population (65,536 reactor envs): eager and graph-replayed launch time.
-   env knobs: NIG_STEP_VEC (1/2/4), NIG_STEP_PDL (0/1); argv: [n_envs] [track_returns 0/1] [step_counters 0/1]"""
+   env knob: NIG_STEP_VEC (1/2/4); argv: [n_envs] [track_returns 0/1] [step_counters 0/1]"""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "neorl-industrial-gym_b200")]
@@ -38,5 +38,5 @@ for _ in range(10):
     g.replay()
 e1.record(); torch.cuda.synchronize()
 graph = e0.elapsed_time(e1)
-print(f"tick_mode={mode} n={n} vec={os.environ.get('NIG_STEP_VEC', 'auto')} pdl={os.environ.get('NIG_STEP_PDL', '1')} track_returns={track} step_counters={counters}: "
+print(f"tick_mode={mode} n={n} vec={os.environ.get('NIG_STEP_VEC', 'auto')} track_returns={track} step_counters={counters}: "
       f"eager {eager:.3f} us/launch, graph {graph:.3f} us/launch", flush=True)
