@@ -150,7 +150,7 @@ struct nig_env {
     int64_t *d_len, *d_off, *d_total;   // dataset: per-episode lengths, offsets, total
     int64_t d_len_cap;
     uint32_t dataset_gen;      // datasets generated so far (each one draws from a fresh derived key)
-    struct { int64_t n_episodes; int32_t n_steps, policy; nig_policy_params_t pp; ConsParams cons; uint32_t gen; int64_t total; bool valid; } probe;
+    struct { int64_t n_episodes; int32_t n_steps, policy; nig_policy_params_t pp; ConsParams cons; RngKey key; int64_t total; bool valid; } probe;
 };
 
 namespace {
@@ -1247,15 +1247,17 @@ int dataset_args(nig_env* e, int64_t n_episodes, int32_t n_steps, int32_t policy
     return NIG_OK;
 }
 
-// pass 1 + scan; the result is cached so that nig_dataset() right after nig_dataset_size() does not repeat it
+// pass 1 + scan; the result is cached so that nig_dataset() right after nig_dataset_size() does not repeat it. The cache is
+// keyed on the derived key, not on the handle's seed or dataset count, so that whatever changes the random streams
+// (nig_set_seed, a dataset written in between) also misses it.
 int dataset_probe(nig_env* e, int64_t n_episodes, int32_t n_steps, int32_t policy, const nig_policy_params_t* pp, DatasetArgs* a,
                   int64_t* total, cudaStream_t st)
 {
     int rc;
     if ((rc = dataset_args(e, n_episodes, n_steps, policy, pp, a)) != NIG_OK) return rc;
     auto& c = e->probe;
-    const bool hit = c.valid && c.n_episodes == n_episodes && c.n_steps == n_steps && c.policy == policy && c.gen == e->dataset_gen &&
-                     memcmp(&c.pp, &a->pp, sizeof c.pp) == 0 && memcmp(&c.cons, &e->cons, sizeof c.cons) == 0;
+    const bool hit = c.valid && c.n_episodes == n_episodes && c.n_steps == n_steps && c.policy == policy && c.key.k0 == a->key.k0 &&
+                     c.key.k1 == a->key.k1 && memcmp(&c.pp, &a->pp, sizeof c.pp) == 0 && memcmp(&c.cons, &e->cons, sizeof c.cons) == 0;
     if (!hit) {
         if ((rc = launch_dataset<false>(e, *a, st)) != NIG_OK) return rc;
         e->launches++;
@@ -1263,7 +1265,7 @@ int dataset_probe(nig_env* e, int64_t n_episodes, int32_t n_steps, int32_t polic
         int64_t t = 0;
         NIG_CUDA(cudaMemcpyAsync(&t, e->d_total, sizeof t, cudaMemcpyDeviceToHost, st));
         NIG_CUDA(cudaStreamSynchronize(st));
-        c.n_episodes = n_episodes; c.n_steps = n_steps; c.policy = policy; c.pp = a->pp; c.cons = e->cons; c.gen = e->dataset_gen;
+        c.n_episodes = n_episodes; c.n_steps = n_steps; c.policy = policy; c.pp = a->pp; c.cons = e->cons; c.key = a->key;
         c.total = t; c.valid = true;
     }
     *total = c.total;

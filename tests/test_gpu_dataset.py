@@ -6,7 +6,7 @@ import time
 import numpy as np
 import pytest
 
-from util import ENV_IDS, KINDS, assert_bits_equal
+from util import ENV_IDS, KINDS, assert_bits_equal, oracle_dataset
 
 pytestmark = pytest.mark.gpu
 
@@ -21,32 +21,6 @@ def mods():
 
 
 ENV_CLASS = {"reactor": "ChemicalReactorEnv", "grid": "PowerGridEnv", "robot": "RobotAssemblyEnv"}
-
-
-def oracle_dataset(O, kind, n_ep, n_steps, policy, pp, seed, gen, env0, incl_trunc):
-    """Episode-contiguous transitions from the oracle, replaying the dataset kernels' documented RNG keying."""
-    k0 = (seed & 0xFFFFFFFF) ^ ((0x9E3779B9 * (gen + 1)) & 0xFFFFFFFF)
-    k1 = ((seed >> 32) & 0xFFFFFFFF) ^ 0x85EBCA6B
-    orc = O.OracleEnv(kind, n_ep, env_id0=env0, seed=k0 | (k1 << 32), exp_mode=1, auto_reset=False)
-    orc.epoch = -1        # the dataset kernels draw the initial states with epoch 0
-    orc.reset()
-    opp = O.copy_policy_params(pp)
-    obs, act, rew, term, nxt, saf, live = [], [], [], [], [], [], []
-    for t in range(n_steps):
-        active = orc.done_latch == 0
-        if not active.any():
-            break
-        a = O.policy_actions(orc, policy, opp)
-        if pp.store_clip > 0:
-            a = np.clip(a, np.float32(-pp.store_clip), np.float32(pp.store_clip))
-        s0 = orc.state.copy()
-        ns, r, fl, vm = orc.step(a)
-        obs.append(s0); act.append(a); rew.append(r); nxt.append(ns); saf.append(vm); live.append(active)
-        term.append(((fl & 3) > 0) if incl_trunc else ((fl & 1) > 0))
-    live = np.stack(live, 1)                       # [episode, t]
-    sel = lambda xs: np.stack(xs, 1)[live]         # episode-major, time-minor == episode-contiguous rows
-    return {"observations": sel(obs), "actions": sel(act), "rewards": sel(rew), "terminals": sel(term),
-            "next_observations": sel(nxt), "safety": sel(saf)}, live.sum(1)
 
 
 @pytest.mark.parametrize("name,quality,n_ep", [("reactor", "mixed", 300), ("reactor", "expert", 100), ("reactor", "random", 200),

@@ -8,7 +8,7 @@ tests cannot lose their target silently when a dispatch threshold moves."""
 import numpy as np
 import pytest
 
-from util import KINDS, Track, adversarial, assert_bits_equal, compare_state, compare_stats
+from util import KINDS, Track, adversarial, assert_bits_equal, compare_state, compare_stats, kernel_names
 
 pytestmark = pytest.mark.gpu
 
@@ -267,15 +267,6 @@ def test_pair_kernel_graph_replay_vs_eager_and_oracle(mods, mode):
 
 
 # 5. dispatch witness
-def _kernel_names(torch, fn):
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        fn()
-        torch.cuda.synchronize()
-    return {e.name for e in prof.events()}
-
-
 def test_dispatch_witness(mods, monkeypatch):
     """The kernels the tests above and below are written for are the ones that run: recorded by name with torch.profiler."""
     ni, N, O, torch = mods
@@ -285,7 +276,7 @@ def test_dispatch_witness(mods, monkeypatch):
             monkeypatch.setenv(k, v)
         env = ni.NativeEnv(kind, n, device=0, seed=1)
         env.reset_device()
-        got = _kernel_names(torch, lambda: call(env))
+        got = kernel_names(torch, lambda: call(env))
         env.close()
         for k in envvars:
             monkeypatch.delenv(k)

@@ -8,12 +8,11 @@ tests/test_gpu_rollout_flavours.py. The dedicated PowerGrid step kernel at its r
 tests/test_gpu_round2.py::test_grid_persistent_step_kernel_from_adversarial_states_and_actions. A dispatch witness records
 kernel names so that these tests cannot lose their target silently when a dispatch threshold moves."""
 import ctypes as C
-import re
 
 import numpy as np
 import pytest
 
-from util import KINDS, Track, adversarial, assert_bits_equal, compare_state, compare_stats
+from util import KINDS, Track, adversarial, assert_bits_equal, compare_state, compare_stats, kernel_names, template_args
 
 pytestmark = pytest.mark.gpu
 
@@ -146,25 +145,6 @@ def _step(env, tr, N, torch, a, ncons, what, *, noise=None, reset_states=None, h
 
 # ---------------------------------------------------------------------------------------------------------------------
 # 1. dispatch witness
-def _kernel_names(torch, fn):
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        fn()
-        torch.cuda.synchronize()
-    return {e.name for e in prof.events()}
-
-
-def _targs(names, kernel):
-    """Template arguments of every recorded instantiation of `kernel`, e.g. ("Reactor", "2", "1", "false")."""
-    out = set()
-    for x in names:
-        m = re.search(r"\b" + kernel + r"<([^>]*)>", x)
-        if m:
-            out.add(tuple(re.sub(r"^(nig::|\(\w+\))", "", s.strip()) for s in m.group(1).split(",")))
-    return out
-
-
 def test_step_dispatch_witness(mods, monkeypatch):
     """The single-step kernels the tests of this file (and the PowerGrid one of test_gpu_round2.py) are written for are the
     ones that run: recorded by name with torch.profiler."""
@@ -179,7 +159,7 @@ def test_step_dispatch_witness(mods, monkeypatch):
                 monkeypatch.setenv(k, v)
         env = ni.NativeEnv(kind, n, device=0, seed=1, constraints=constraints)
         env.reset_device()
-        got = _kernel_names(torch, lambda: call(env))
+        got = kernel_names(torch, lambda: call(env))
         env.close()
         for k in envvars:
             monkeypatch.delenv(k, raising=False)
@@ -192,26 +172,26 @@ def test_step_dispatch_witness(mods, monkeypatch):
     grid = names_of(N.ENV_POWER_GRID, GRID_N, plain, NIG_GRID_STEP=None)
     if not grid:
         pytest.skip("torch.profiler recorded no CUDA kernel in this process (no CUPTI activity records)")
-    assert _targs(grid, "step_grid_kernel") == {("256", "128", "4")} and not _targs(grid, "step_kernel"), sorted(grid)
+    assert template_args(grid, "step_grid_kernel") == {("256", "128", "4")} and not template_args(grid, "step_kernel"), sorted(grid)
     g0 = names_of(N.ENV_POWER_GRID, GRID_N, plain, NIG_GRID_STEP="0")
-    assert not _targs(g0, "step_grid_kernel") and _targs(g0, "step_kernel") == {("Grid", "1", "1", "true")}, sorted(g0)
+    assert not template_args(g0, "step_grid_kernel") and template_args(g0, "step_kernel") == {("Grid", "1", "1", "true")}, sorted(g0)
 
     for name, env_t, vec in (("reactor", "Reactor", "2"), ("robot", "Robot", "1")):
         kind = KINDS[name]
         bound = make_constraint(N.CON_BOUND, si=0, lo=-1.0, hi=1.0, penalty=-5.0)
         pre = names_of(kind, PIPE_N[name], plain, constraints=_builtins(N, kind) + [bound])
-        assert _targs(pre, "step_pipe_kernel") == {(env_t, vec, str(CONS_PREFIX))} and not _targs(pre, "step_kernel"), sorted(pre)
+        assert template_args(pre, "step_pipe_kernel") == {(env_t, vec, str(CONS_PREFIX))} and not template_args(pre, "step_kernel"), sorted(pre)
         gen = names_of(kind, PIPE_N[name], plain, constraints=_builtins(N, kind, (1, 0, 2)) + [bound])
-        assert _targs(gen, "step_pipe_kernel") == {(env_t, vec, str(CONS_GENERIC))}, sorted(gen)
+        assert template_args(gen, "step_pipe_kernel") == {(env_t, vec, str(CONS_GENERIC))}, sorted(gen)
 
     R = N.ENV_CHEMICAL_REACTOR
     soa_obs = names_of(R, VEC2_N, lambda e: plain(e, obs=e.empty(e.S)))
-    assert _targs(soa_obs, "step_kernel") == {("Reactor", "2", "1", "false")}, sorted(soa_obs)
-    assert _targs(names_of(R, VEC2_N, plain), "step_pipe_kernel") == {("Reactor", "2", "1")}
+    assert template_args(soa_obs, "step_kernel") == {("Reactor", "2", "1", "false")}, sorted(soa_obs)
+    assert template_args(names_of(R, VEC2_N, plain), "step_pipe_kernel") == {("Reactor", "2", "1")}
     off8 = names_of(R, VEC2_N, lambda e: plain(e, 2))          # 8-byte aligned actions: no TMA pipeline, two envs per thread
-    assert _targs(off8, "step_kernel") == {("Reactor", "2", "1", "false")} and not _targs(off8, "step_pipe_kernel"), sorted(off8)
+    assert template_args(off8, "step_kernel") == {("Reactor", "2", "1", "false")} and not template_args(off8, "step_pipe_kernel"), sorted(off8)
     off4 = names_of(R, VEC2_N, lambda e: plain(e, 1))          # 4-byte aligned: one env per thread
-    assert _targs(off4, "step_kernel") == {("Reactor", "1", "1", "true")}, sorted(off4)
+    assert template_args(off4, "step_kernel") == {("Reactor", "1", "1", "true")}, sorted(off4)
 
     def aos_calls(e):              # nig_step_host on page-locked [n] arrays, and an AoS step_device call on the torch stream
         e.step_host(np.zeros((e.n, e.A), np.float32))
@@ -219,7 +199,7 @@ def test_step_dispatch_witness(mods, monkeypatch):
                       action_layout=N.LAYOUT_AOS, aux_layout=N.LAYOUT_AOS)
     for vec in ("2", "4"):
         aos = names_of(R, 130, aos_calls, NIG_STEP_VEC=vec)
-        assert {t[1] for t in _targs(aos, "step_kernel")} == {"1"}, (vec, sorted(aos))
+        assert {t[1] for t in template_args(aos, "step_kernel")} == {"1"}, (vec, sorted(aos))
 
 
 # ---------------------------------------------------------------------------------------------------------------------

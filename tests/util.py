@@ -2,6 +2,7 @@
 import glob
 import io
 import os
+import re
 
 import numpy as np
 
@@ -80,7 +81,28 @@ ENV_IDS = {"reactor": "ChemicalReactor-v0", "grid": "PowerGrid-v0", "robot": "Ro
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# oracle tracking shared by the kernel-flavour tests (test_gpu_rollout_flavours.py, test_gpu_step_flavours.py)
+# dispatch witness and oracle tracking shared by the kernel-flavour tests (test_gpu_rollout_flavours.py,
+# test_gpu_step_flavours.py, test_gpu_dataset_flavours.py)
+def kernel_names(torch, fn):
+    """Names of the CUDA kernels fn() runs, recorded with torch.profiler (empty when CUPTI records no activity)."""
+    from torch.profiler import ProfilerActivity, profile
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        fn()
+        torch.cuda.synchronize()
+    return {e.name for e in prof.events()}
+
+
+def template_args(names, kernel):
+    """Template arguments of every recorded instantiation of `kernel`, e.g. ("Reactor", "2", "1", "false")."""
+    out = set()
+    for x in names:
+        m = re.search(r"\b" + kernel + r"<([^>]*)>", x)
+        if m:
+            out.add(tuple(re.sub(r"^(nig::|\(\w+\))", "", s.strip()) for s in m.group(1).split(",")))
+    return out
+
+
 def popcount8(v):
     return np.unpackbits(np.ascontiguousarray(v, np.uint8)[:, None], axis=1).sum(1, dtype=np.int64)
 
@@ -186,6 +208,43 @@ def compare_stats(N, counters, sums, tr, ncons, extrema, what, lohi=None, reward
         else:
             tol = 1e-15 if tr.reactor else 1e-6
             np.testing.assert_allclose([lo, hi], [tr.lo, tr.hi], rtol=tol, atol=0 if tr.reactor else 1e-3, err_msg=what)
+
+
+DATASET_KEYS = ("observations", "actions", "rewards", "terminals", "next_observations", "safety")
+
+
+def oracle_dataset(O, kind, n_ep, n_steps, policy, pp, seed, gen, env0, incl_trunc, *, builtin=True, extra_cons=(),
+                   max_episode_steps=None, threads=1):
+    """Episode-contiguous transitions from the oracle, replaying the dataset kernels' documented RNG keying: episode e is
+    the env env0 + e of its own, reset with epoch 0 and stepped without auto-reset until it is done or n_steps ran out.
+    builtin / extra_cons / max_episode_steps configure the oracle like a handle's constraint set and episode cap. The live
+    rows of each step are kept with their episode index and put in episode-major order by one stable sort, so no
+    [n_ep, n_steps, S] stack is built. Returns the arrays of DATASET_KEYS and the episode lengths."""
+    k0 = (seed & 0xFFFFFFFF) ^ ((0x9E3779B9 * (gen + 1)) & 0xFFFFFFFF)
+    k1 = ((seed >> 32) & 0xFFFFFFFF) ^ 0x85EBCA6B
+    orc = O.OracleEnv(kind, n_ep, env_id0=env0, seed=k0 | (k1 << 32), exp_mode=1, auto_reset=False, builtin=builtin,
+                      extra_cons=extra_cons, max_episode_steps=max_episode_steps, threads=threads)
+    orc.epoch = -1        # the dataset kernels draw the initial states with epoch 0
+    orc.reset()
+    opp = O.copy_policy_params(pp)
+    rows = {k: [] for k in DATASET_KEYS}
+    eps = []
+    for t in range(n_steps):
+        live = np.flatnonzero(orc.done_latch == 0)
+        if not live.size:
+            break
+        a = O.policy_actions(orc, policy, opp)
+        if pp.store_clip > 0:
+            a = np.clip(a, np.float32(-pp.store_clip), np.float32(pp.store_clip))
+        s0 = orc.state[live]
+        ns, r, fl, vm = orc.step(a)
+        term = ((fl & 3) > 0) if incl_trunc else ((fl & 1) > 0)
+        for k, v in zip(DATASET_KEYS, (s0, a[live], r[live], term[live], ns[live], vm[live])):
+            rows[k].append(v)
+        eps.append(live)
+    ep = np.concatenate(eps)
+    order = np.argsort(ep, kind="stable")          # stable: time-minor inside an episode
+    return {k: np.concatenate(v)[order] for k, v in rows.items()}, np.bincount(ep, minlength=n_ep)
 
 
 def adversarial(O, kind, rng, s0, n, max_steps, clean_from=None):
