@@ -36,7 +36,7 @@ extern "C" {
 #define NIG_API
 #endif
 
-#define NIG_ABI_VERSION 4
+#define NIG_ABI_VERSION 5
 #define NIG_MAX_CONSTRAINTS 8
 #define NIG_MAX_STATE_DIM 32
 #define NIG_MAX_ACTION_DIM 8
@@ -139,8 +139,37 @@ enum {
                                 the reference's timing harness performance_benchmark.py:106-133) */
     NIG_POLICY_ZERO = 2,
     NIG_POLICY_PCTRL = 3,    /* get_dataset's "PID-like" P-controller mixes (chemical_reactor.py:364-390) */
-    NIG_POLICY_BASELINE = 4  /* the benchmark baseline controllers (benchmarks/baseline_agents.py:28-114), nig_baseline_t */
+    NIG_POLICY_BASELINE = 4, /* the benchmark baseline controllers (benchmarks/baseline_agents.py:28-114), nig_baseline_t */
+    NIG_POLICY_MLP = 5       /* a deterministic MLP actor (nig_set_mlp_policy) evaluated by the tensor cores in the kernel */
 };
+
+/* NIG_POLICY_MLP: the deterministic actor of an offline-RL agent (TD3+BC / IQL / CQL style), evaluated inside the fused
+ * rollout by tcgen05 MMAs, 128 envs per tile, one env per accumulator row. Network family and numeric contract:
+ *  - input: the observation the env hands the policy, i.e. the pre-step state s (base.py:201). Optional normalisation
+ *    x = (s - obs_mean) * obs_inv_std in fp32 (round to nearest, no contraction); NULL mean / inv_std = 0 / 1.
+ *  - n_hidden = 1 or 2 hidden layers, each of width 64, 128 or 256, ReLU (NaN-propagating, like torch.relu);
+ *    then an output layer of width A followed by tanh or identity. The env clips the action to [-1, 1] as always.
+ *  - weights and every layer's INPUT are rounded to bf16 (nearest even); products are accumulated in fp32 by the tensor
+ *    core in the hardware's order; biases and activations are applied in fp32. Inputs are zero-padded to a multiple of 16
+ *    (reactor 12 -> 16, robot 24 -> 32), the output to 16 columns; the padding is invisible.
+ *  - actions are therefore specified to a tolerance against an fp64 forward pass of the bf16-rounded network, not bit for
+ *    bit; everything downstream of the action keeps the bit-exact contract. Env i's action depends only on its own
+ *    observation and the weights (row i mod 128 of its tile), not on the population, slicing or launch shape.
+ * Not supported (NIG_ERR_INVALID): more layers, other widths, other activations; stochastic actors; fp16 / fp8 / tf32 weights
+ * (the ABI takes fp32, the library rounds to bf16). */
+enum { NIG_MLP_OUT_IDENTITY = 0, NIG_MLP_OUT_TANH = 1 };
+typedef struct nig_mlp {
+    int32_t n_hidden;           /* hidden layers: 1 or 2 */
+    int32_t hidden[2];          /* hidden widths (64, 128 or 256); hidden[1] ignored when n_hidden == 1 */
+    int32_t output_activation;  /* NIG_MLP_OUT_* */
+    int32_t in_dim;             /* must equal the env's state_dim */
+    int32_t out_dim;            /* must equal the env's action_dim */
+    const float* weight[3];     /* host fp32 [out][in] (torch nn.Linear order): the hidden layers, then the output layer
+                                   (weight[1] is the output layer when n_hidden == 1) */
+    const float* bias[3];       /* host fp32 [out] per layer, same order; NULL = zeros */
+    const float* obs_mean;      /* host fp32 [in_dim] or NULL */
+    const float* obs_inv_std;   /* host fp32 [in_dim] or NULL */
+} nig_mlp_t;
 
 /* Baseline controllers evaluated inside the fused rollout kernel (benchmarks/baseline_agents.py). The reference
  * computes them in numpy float64 from the float32 observation; so does the kernel (fp64 registers), then the action
@@ -296,6 +325,15 @@ typedef struct nig_rollout_host {
 } nig_rollout_host_t;
 NIG_API int nig_rollout_host(nig_env_t* env, const nig_rollout_host_t* r);
 
+/* NIG_POLICY_MLP's network: validated against the env's S / A, converted and packed once into a handle-owned device buffer.
+ * A network that fails validation leaves the previous one in place. Otherwise the call synchronises the device (a rollout
+ * still running on any stream finishes with the old network), then drops the old network and the captured nig_rollout_steps /
+ * nig_rollout_host graphs before it touches the device buffer; if the upload then fails (NIG_ERR_CUDA) the handle has no
+ * network. The network is copied: changing the caller's arrays afterwards changes nothing. nig_rollout, nig_rollout_steps and nig_rollout_host then accept
+ * NIG_POLICY_MLP (NIG_ERR_INVALID before a network is set; NIG_ERR_UNSUPPORTED with teacher-forced noise); nig_dataset and
+ * nig_dataset_size do not (NIG_ERR_UNSUPPORTED). */
+NIG_API int nig_set_mlp_policy(nig_env_t* env, const nig_mlp_t* mlp);
+
 /* zero the persistent controller state of NIG_POLICY_BASELINE / NIG_BASELINE_PID (integral, previous error) */
 NIG_API int nig_reset_policy_state(nig_env_t* env, void* stream);
 
@@ -407,6 +445,10 @@ NIG_API int nig_selftest_normal(int device, uint32_t first, uint32_t stride, int
  * its PID integral / previous error across the n_steps rows like one agent object does. */
 NIG_API int nig_selftest_policy(int device, int32_t env_kind, int32_t policy, const nig_policy_params_t* pp, int64_t n, int32_t n_steps,
                                 const float* states, const float* coin, const float* z, const float* u, float* actions);
+
+/* test hook of NIG_POLICY_MLP: the handle's network evaluated by the rollout's own device function and 128-row tiling on
+ * HOST arrays: obs [n][S] -> actions [n][A] (before the env's clip). Synchronous. */
+NIG_API int nig_selftest_mlp(nig_env_t* env, const float* obs, int64_t n, float* actions);
 
 #ifdef __cplusplus
 }

@@ -151,6 +151,9 @@ struct nig_env {
     int64_t d_len_cap;
     uint32_t dataset_gen;      // datasets generated so far (each one draws from a fresh derived key)
     struct { int64_t n_episodes; int32_t n_steps, policy; nig_policy_params_t pp; ConsParams cons; RngKey key; int64_t total; bool valid; } probe;
+    void* mlp_blob;            // NIG_POLICY_MLP: the packed network (nig_set_mlp_policy; MlpParams::blob)
+    size_t mlp_cap;            // bytes allocated at mlp_blob
+    MlpParams mlp;             // blob null until a network is set
 };
 
 namespace {
@@ -373,7 +376,8 @@ int rollout_checks(nig_env* e, const nig_rollout_t* r)
     if (r->noise && e->NZ == 0) return fail(NIG_ERR_INVALID, "nig_rollout: env kind %d has no process noise", e->kind);
     if (r->noise && r->policy != NIG_POLICY_ACTIONS)
         return fail(NIG_ERR_UNSUPPORTED, "nig_rollout: teacher-forced noise is only available together with teacher-forced actions (NIG_POLICY_ACTIONS)");
-    if (r->policy < NIG_POLICY_ACTIONS || r->policy > NIG_POLICY_BASELINE) return fail(NIG_ERR_INVALID, "unknown rollout policy %d", r->policy);
+    if (r->policy < NIG_POLICY_ACTIONS || r->policy > NIG_POLICY_MLP) return fail(NIG_ERR_INVALID, "unknown rollout policy %d", r->policy);
+    if (r->policy == NIG_POLICY_MLP && !e->mlp.blob) return fail(NIG_ERR_INVALID, "nig_rollout: NIG_POLICY_MLP needs a network (nig_set_mlp_policy)");
     if (r->noise && e->track_extrema)
         return fail(NIG_ERR_UNSUPPORTED, "nig_rollout: teacher-forced noise has no return-extrema kernel flavour (nig_track_extrema(env, 0) first)");
     if (r->policy == NIG_POLICY_BASELINE) {
@@ -441,6 +445,8 @@ int rollout_range(nig_env* e, const nig_rollout_t* r, cudaStream_t stream, int64
                e->cfg.auto_reset != 0 && (i0 % 2) == 0;
     // PowerGrid-v0: the dedicated lean kernel (NIG_GRID_FAST = 0 falls back to the generic one)
     cfg.grid_fast = e->grid_fast && e->kind == NIG_ENV_POWER_GRID && e->cfg.auto_reset != 0;
+    cfg.mlp = e->mlp;
+    cfg.mlp.extrema = e->track_extrema ? 1 : 0;
     e->launches++;
     const int64_t extent = (ns + 127) / 128 * 128;          // launch extent; <= the rows' pitch because slices start at multiples of 128
     NIG_CUDA(nig::launch_rollout(e->kind, cfg, extent, a, map, stream));
@@ -743,6 +749,7 @@ int nig_destroy(nig_env_t* e)
     cudaFree(e->h_reward); cudaFree(e->h_hostmask); cudaFree(e->h_flags); cudaFree(e->h_viol); cudaFree(e->h_mask);
     cudaFree(e->h_terminated); cudaFree(e->h_truncated);
     cudaFree(e->h_i32a); cudaFree(e->h_i32b); cudaFree(e->pid_state); cudaFree(e->tick_dev); cudaFree(e->cons_masks); cudaFree(e->extrema); cudaFree(e->d_len); cudaFree(e->d_off); cudaFree(e->d_total);
+    cudaFree(e->mlp_blob);
     for (int b = 0; b < 2; ++b) {
         cudaFree(e->r_act[b]); cudaFree(e->r_nz[b]);
         if (e->r_ev_copy[b]) cudaEventDestroy(e->r_ev_copy[b]);
@@ -1026,6 +1033,112 @@ plain_enqueue:
     return rc ? rc : jrc;
 }
 
+} // extern "C"
+
+// ---- NIG_POLICY_MLP ------------------------------------------------------------------------------------------------------
+namespace {
+uint16_t bf16_rne(float x)
+{
+    uint32_t u;
+    memcpy(&u, &x, 4);
+    if ((u & 0x7fffffffu) > 0x7f800000u) return (uint16_t)((u >> 16) | 0x40u);      // NaN stays a (quiet) NaN
+    u += 0x7fffu + ((u >> 16) & 1u);
+    return (uint16_t)(u >> 16);
+}
+// [n_out][n_in] fp32 (nn.Linear order) -> bf16 [n_rows][k_pad] in the canonical layout of MlpParams, zero-padded
+void pack_weight(uint8_t* dst, const float* w, int n_out, int n_in, int n_rows, int k_pad)
+{
+    for (int n = 0; n < n_rows; ++n)
+        for (int k = 0; k < k_pad; ++k) {
+            const uint16_t v = (n < n_out && k < n_in) ? bf16_rne(w[(size_t)n * n_in + k]) : (uint16_t)0;
+            memcpy(dst + (size_t)(k / 8) * n_rows * 16 + (size_t)n * 16 + (k % 8) * 2, &v, 2);
+        }
+}
+} // namespace
+
+extern "C" {
+
+int nig_set_mlp_policy(nig_env_t* e, const nig_mlp_t* m)
+{
+    NIG_CHECK_ENV(e);
+    if (!m) return fail(NIG_ERR_INVALID, "nig_set_mlp_policy: null network");
+    if (m->n_hidden != 1 && m->n_hidden != 2) return fail(NIG_ERR_INVALID, "nig_set_mlp_policy: %d hidden layers (1 or 2 are supported)", m->n_hidden);
+    for (int l = 0; l < m->n_hidden; ++l)
+        if (m->hidden[l] != 64 && m->hidden[l] != 128 && m->hidden[l] != 256)
+            return fail(NIG_ERR_INVALID, "nig_set_mlp_policy: hidden width %d (64, 128 or 256 are supported)", m->hidden[l]);
+    if (m->output_activation != NIG_MLP_OUT_IDENTITY && m->output_activation != NIG_MLP_OUT_TANH)
+        return fail(NIG_ERR_INVALID, "nig_set_mlp_policy: unknown output activation %d", m->output_activation);
+    if (m->in_dim != e->S || m->out_dim != e->A)
+        return fail(NIG_ERR_INVALID, "nig_set_mlp_policy: network maps %d -> %d, the env needs %d -> %d", m->in_dim, m->out_dim, e->S, e->A);
+    for (int l = 0; l <= m->n_hidden; ++l)
+        if (!m->weight[l]) return fail(NIG_ERR_INVALID, "nig_set_mlp_policy: null weight of layer %d", l);
+    MlpParams p;
+    memset(&p, 0, sizeof p);
+    p.layers = m->n_hidden; p.h1 = m->hidden[0]; p.h2 = m->n_hidden == 2 ? m->hidden[1] : m->hidden[0];
+    p.out_tanh = m->output_activation == NIG_MLP_OUT_TANH ? 1 : 0;
+    const MlpLayout L = mlp_layout(e->S, p);
+    p.blob_bytes = L.blob;
+    uint8_t* h = (uint8_t*)calloc(L.blob, 1);
+    if (!h) return fail(NIG_ERR_INVALID, "out of host memory");
+    const int widths[3] = {p.h1, p.layers == 2 ? p.h2 : kMlpOut, kMlpOut};
+    const int rows[3] = {p.h1, p.layers == 2 ? p.h2 : kMlpOut, kMlpOut};
+    const int ins[3] = {e->S, p.h1, p.h2};
+    const uint32_t woff[3] = {L.w1, p.layers == 2 ? L.w2 : L.w3, L.w3};
+    const uint32_t boff[3] = {L.b1, p.layers == 2 ? L.b2 : L.b3, L.b3};
+    for (int l = 0; l <= p.layers; ++l) {
+        const bool last = l == p.layers;
+        const int n_out = last ? e->A : widths[l];
+        pack_weight(h + woff[l], m->weight[l], n_out, ins[l], rows[l], l == 0 ? L.sp : ins[l]);
+        if (m->bias[l]) memcpy(h + boff[l], m->bias[l], (size_t)n_out * sizeof(float));
+    }
+    float* mean = (float*)(h + L.mean);
+    float* istd = (float*)(h + L.istd);
+    for (int k = 0; k < L.sp; ++k) {
+        mean[k] = (m->obs_mean && k < e->S) ? m->obs_mean[k] : 0.0f;
+        istd[k] = (m->obs_inv_std && k < e->S) ? m->obs_inv_std[k] : 1.0f;
+    }
+    // a rollout still running on any stream keeps reading the old blob: finish it before the buffer is reused or freed
+    cudaError_t ce = cudaDeviceSynchronize();
+    // from here on the old network is gone, whether or not the upload below succeeds: no launch and no replay of a captured
+    // nig_rollout_steps / nig_rollout_host graph (the network is baked into them) may read the buffer until the new one is
+    // complete. A failed upload leaves the handle without a network (NIG_POLICY_MLP then fails with NIG_ERR_INVALID).
+    e->mlp.blob = nullptr;
+    e->config_version++;
+    if (e->steps_graph) { cudaGraphExecDestroy(e->steps_graph); e->steps_graph = nullptr; }
+    if (e->host_graph) { cudaGraphExecDestroy(e->host_graph); e->host_graph = nullptr; }
+    if (ce == cudaSuccess && L.blob > e->mlp_cap) {
+        cudaFree(e->mlp_blob);
+        e->mlp_blob = nullptr; e->mlp_cap = 0;
+        ce = cudaMalloc(&e->mlp_blob, L.blob);
+        if (ce == cudaSuccess) e->mlp_cap = L.blob;
+    }
+    if (ce == cudaSuccess) ce = cudaMemcpyAsync(e->mlp_blob, h, L.blob, cudaMemcpyHostToDevice, e->stream);
+    if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
+    free(h);
+    if (ce != cudaSuccess) return fail(NIG_ERR_CUDA, "nig_set_mlp_policy: %s", cudaGetErrorString(ce));
+    p.blob = e->mlp_blob;
+    e->mlp = p;
+    return NIG_OK;
+}
+
+int nig_selftest_mlp(nig_env_t* e, const float* obs, int64_t n, float* actions)
+{
+    NIG_CHECK_ENV(e);
+    if (!e->mlp.blob) return fail(NIG_ERR_INVALID, "nig_selftest_mlp: no network set (nig_set_mlp_policy)");
+    if (n <= 0 || !obs || !actions) return fail(NIG_ERR_INVALID, "nig_selftest_mlp: bad arguments");
+    if (int hrc = host_entry(e)) return hrc;
+    float *d_obs = nullptr, *d_act = nullptr;
+    cudaError_t ce = cudaMalloc((void**)&d_obs, (size_t)n * e->S * sizeof(float));
+    if (ce == cudaSuccess) ce = cudaMalloc((void**)&d_act, (size_t)n * e->A * sizeof(float));
+    if (ce == cudaSuccess) ce = cudaMemcpyAsync(d_obs, obs, (size_t)n * e->S * sizeof(float), cudaMemcpyHostToDevice, e->stream);
+    if (ce == cudaSuccess) { e->launches++; ce = nig::launch_selftest_mlp(e->kind, e->mlp, d_obs, d_act, n, e->stream); }
+    if (ce == cudaSuccess) ce = cudaMemcpyAsync(actions, d_act, (size_t)n * e->A * sizeof(float), cudaMemcpyDeviceToHost, e->stream);
+    if (ce == cudaSuccess) ce = cudaStreamSynchronize(e->stream);
+    cudaFree(d_obs); cudaFree(d_act);
+    if (ce != cudaSuccess) return fail(NIG_ERR_CUDA, "nig_selftest_mlp: %s", cudaGetErrorString(ce));
+    return NIG_OK;
+}
+
 int nig_reset_policy_state(nig_env_t* e, void* stream)
 {
     NIG_CHECK_ENV(e);
@@ -1222,6 +1335,7 @@ int dataset_args(nig_env* e, int64_t n_episodes, int32_t n_steps, int32_t policy
 {
     if (n_episodes <= 0 || n_episodes > (1LL << 31)) return fail(NIG_ERR_INVALID, "n_episodes %lld outside [1, 2^31]", (long long)n_episodes);
     if (n_steps <= 0) return fail(NIG_ERR_INVALID, "n_steps must be positive (got %d)", n_steps);
+    if (policy == NIG_POLICY_MLP) return fail(NIG_ERR_UNSUPPORTED, "the dataset kernels have no NIG_POLICY_MLP flavour");
     if (policy != NIG_POLICY_UNIFORM && policy != NIG_POLICY_ZERO && policy != NIG_POLICY_PCTRL)
         return fail(NIG_ERR_INVALID, "dataset policy must be UNIFORM, ZERO or PCTRL (got %d)", policy);
     if (policy == NIG_POLICY_PCTRL && !pp) return fail(NIG_ERR_INVALID, "NIG_POLICY_PCTRL needs policy parameters");

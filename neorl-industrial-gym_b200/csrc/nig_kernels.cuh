@@ -2339,6 +2339,9 @@ __global__ void __launch_bounds__(kThreads, Env::ROLLOUT_MIN_CTAS) rollout_kerne
             } else ng.get(key, env, tick, nz);
         } else nz[0] = 0.0f;
 
+        // this step-and-bookkeeping block is repeated statement for statement in rollout_step_generic (nig_rollout_mlp.cu,
+        // the MLP policy's kernel) and, for the uniform policy, in rollout_generic_uniform_step: a change here goes there too
+        // (moving it into a shared function changed ptxas' schedule of this kernel's reactor instantiations)
         const bool active = valid && !latched;
         uint32_t st2, vi2, f, vm;
         acc_t r;

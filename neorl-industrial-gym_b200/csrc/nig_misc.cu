@@ -68,6 +68,7 @@ cudaError_t launch_selftest_policy(int kind, const PolicyTestArgs& a, cudaStream
 }
 cudaError_t launch_rollout(int kind, const RolloutLaunch& cfg, int64_t pitch, const RolloutArgs& a, const CUtensorMap& map, cudaStream_t st)
 {
+    if (cfg.policy == NIG_POLICY_MLP) return launch_rollout_mlp(kind, cfg, pitch, a, st);
     switch (kind) {
     case NIG_ENV_CHEMICAL_REACTOR: return launch_rollout_reactor(cfg, pitch, a, map, st);
     case NIG_ENV_POWER_GRID: return launch_rollout_grid(cfg, pitch, a, map, st);

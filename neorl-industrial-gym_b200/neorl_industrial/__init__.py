@@ -13,10 +13,11 @@ from .safety import BoundConstraint, SafetyWrapper
 from .utils import evaluate_with_safety, make
 from .vector import NativeEnv
 from .torch_env import TorchIndustrialEnv
+from .policies import MLPPolicy
 from ._native import build_native
 
 __all__ = [
     "__version__", "DatasetQuality", "IndustrialState", "SafetyConstraint", "SafetyMetrics", "BatchedSafetyMetrics",
     "IndustrialEnv", "ChemicalReactorEnv", "PowerGridEnv", "RobotAssemblyEnv", "SafetyWrapper", "BoundConstraint",
-    "make", "evaluate_with_safety", "NativeEnv", "TorchIndustrialEnv", "build_native",
+    "make", "evaluate_with_safety", "NativeEnv", "TorchIndustrialEnv", "MLPPolicy", "build_native",
 ]

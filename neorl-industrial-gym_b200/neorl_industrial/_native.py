@@ -16,7 +16,7 @@ _ROOT = os.path.dirname(_PKG_DIR)                       # neorl-industrial-gym_b
 LIB_PATH = os.environ.get("NIG_LIB_PATH") or os.path.join(_ROOT, "libnig_b200.so")   # (override: A/B builds, tools/ab_build.sh)
 CSRC_DIR = os.path.join(_ROOT, "csrc")
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 MAX_CONSTRAINTS = 8
 STATS_SLOTS = 32
 
@@ -25,7 +25,8 @@ ENV_CHEMICAL_REACTOR, ENV_POWER_GRID, ENV_ROBOT_ASSEMBLY = 0, 1, 2
 CON_BUILTIN, CON_BOUND, CON_HOSTMASK = 0, 1, 2
 F_TERMINATED, F_TRUNCATED, F_CRITICAL, F_RESET, F_INACTIVE = 1, 2, 4, 8, 128
 LAYOUT_SOA, LAYOUT_AOS = 0, 1
-POLICY_ACTIONS, POLICY_UNIFORM, POLICY_ZERO, POLICY_PCTRL, POLICY_BASELINE = 0, 1, 2, 3, 4
+POLICY_ACTIONS, POLICY_UNIFORM, POLICY_ZERO, POLICY_PCTRL, POLICY_BASELINE, POLICY_MLP = 0, 1, 2, 3, 4, 5
+MLP_OUT_IDENTITY, MLP_OUT_TANH = 0, 1
 BASELINE_RANDOM, BASELINE_PID, BASELINE_MPC, BASELINE_CONSTANT = 0, 1, 2, 3
 ROLLOUT_USE_TMA = 1
 ROLLOUT_ACCUMULATE = 2
@@ -92,6 +93,12 @@ class DatasetOut(C.Structure):
                 ("reserved", C.c_int32)]
 
 
+class Mlp(C.Structure):
+    _fields_ = [("n_hidden", C.c_int32), ("hidden", C.c_int32 * 2), ("output_activation", C.c_int32), ("in_dim", C.c_int32),
+                ("out_dim", C.c_int32), ("weight", C.c_void_p * 3), ("bias", C.c_void_p * 3), ("obs_mean", C.c_void_p),
+                ("obs_inv_std", C.c_void_p)]
+
+
 # every symbol include/nig_b200.h declares: (restype, argtypes)
 _VP, _I32, _I64, _U32, _U64 = C.c_void_p, C.c_int32, C.c_int64, C.c_uint32, C.c_uint64
 SYMBOLS = {
@@ -112,6 +119,8 @@ SYMBOLS = {
     "nig_rollout_steps": (C.c_int, [_VP, _VP, C.c_int32, _VP]),
     "nig_rollout_host": (C.c_int, [_VP, C.POINTER(RolloutHost)]),
     "nig_reset_policy_state": (C.c_int, [_VP, _VP]),
+    "nig_set_mlp_policy": (C.c_int, [_VP, C.POINTER(Mlp)]),
+    "nig_selftest_mlp": (C.c_int, [_VP, _VP, _I64, _VP]),
     "nig_dataset": (C.c_int, [_VP, _I64, _I32, _I32, C.POINTER(PolicyParams), C.POINTER(DatasetOut), C.POINTER(_I64), _VP]),
     "nig_dataset_size": (C.c_int, [_VP, _I64, _I32, _I32, C.POINTER(PolicyParams), C.POINTER(_I64), _VP]),
     "nig_get_state": (C.c_int, [_VP, _VP, _I32, _VP, _VP, _VP, _VP]),

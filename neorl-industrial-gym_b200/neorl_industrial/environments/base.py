@@ -17,6 +17,7 @@ import numpy as np
 
 from .. import _native as N
 from ..core.types import BatchedSafetyMetrics, SafetyConstraint, SafetyMetrics
+from ..policies import MLPPolicy
 from ..spaces import Box
 from ..vector import NativeEnv, make_constraint
 
@@ -331,7 +332,7 @@ class IndustrialEnv:
 
         ``policy``: "random" (= ``action_space.sample()`` per step, drawn in-kernel), "zero", "dataset" with ``params``
         (the get_dataset controllers), a ``benchmarks.baseline_agents`` controller object (PID / MPC / constant / random,
-        evaluated in-kernel), or "actions" with ``actions`` [T, num_envs, A] (and optionally ``noise``
+        evaluated in-kernel), an ``MLPPolicy`` (a learned actor, evaluated in-kernel on the tensor cores), or "actions" with ``actions`` [T, num_envs, A] (and optionally ``noise``
         [T, num_envs, NZ]) teacher-forcing every step. Returns per-env ``reward_sum`` / ``violations`` / ``episodes``,
         the final ``obs`` and the lifetime ``stats`` (the evaluate_with_safety aggregates)."""
         nat = self.native
@@ -349,6 +350,9 @@ class IndustrialEnv:
                 noise = np.ascontiguousarray(z.transpose(0, 2, 1))
         elif hasattr(policy, "device_policy"):                 # benchmarks.baseline_agents controllers, in-kernel
             pid, params = policy.device_policy()
+        elif isinstance(policy, MLPPolicy):                    # a learned actor on the tensor cores, in-kernel
+            nat.use_mlp_policy(policy)
+            pid = N.POLICY_MLP
         elif policy == "dataset":
             if params is None:
                 raise ValueError("policy='dataset' needs PolicyParams (see datasets.policy_params)")

@@ -3,7 +3,7 @@
 
 Two flavours:
   * ``evaluate_policy_device``: the policy runs inside the fused rollout kernel (uniform random, zero, the
-    get_dataset P-controllers) -- no host round trips; aggregates come from the device stats block, which
+    get_dataset P-controllers, a learned ``MLPPolicy``) -- no host round trips; aggregates come from the device stats block, which
     ``distributed.allreduce_stats`` can sum across GPUs.
   * ``evaluate_agent_batched``: an arbitrary ``agent.predict(obs, deterministic=True)`` callback drives the
     batched ``env.step`` (host arrays).
@@ -17,6 +17,7 @@ from typing import Any, Dict, Optional
 import numpy as np
 
 from . import _native as N
+from .policies import MLPPolicy
 
 
 def metrics_from_stats(stats: Dict[str, Any], n_constraints: int, critical_flags) -> Dict[str, Any]:
@@ -44,8 +45,12 @@ def evaluate_policy_device(env, n_steps: int, policy: int = N.POLICY_UNIFORM, pa
                            reduce_fn=None) -> Dict[str, Any]:
     """Run ``n_steps`` env-steps per env with an in-kernel policy (auto-reset on) and return the reference's
     evaluation keys over every episode that finished. ``reduce_fn(counters, sums) -> (counters, sums)`` hooks in the
-    cross-GPU all-reduce (see distributed.allreduce_stats)."""
+    cross-GPU all-reduce (see distributed.allreduce_stats). ``policy`` may also be an ``MLPPolicy``: the learned actor runs
+    inside the kernel (NIG_POLICY_MLP), uploaded once per network object."""
     nat = env.native
+    if isinstance(policy, MLPPolicy):
+        nat.use_mlp_policy(policy)
+        policy = N.POLICY_MLP
     nat.clear_stats()
     nat.track_extrema(True)            # the kernel flavour that also keeps return_min / return_max
     try:

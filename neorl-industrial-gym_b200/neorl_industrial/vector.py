@@ -150,6 +150,23 @@ class NativeEnv:
         """Zero the device-resident PID controller state (= constructing a new PIDControllerAgent)."""
         N.check(N.lib().nig_reset_policy_state(self._h, self._stream(stream)))
 
+    def set_mlp_policy(self, mlp):
+        """Upload an ``MLPPolicy`` for NIG_POLICY_MLP (nig_set_mlp_policy: synchronises the device, invalidates captured graphs)."""
+        N.check(N.lib().nig_set_mlp_policy(self._h, C.byref(mlp.native_struct())))
+        self._mlp = mlp
+
+    def use_mlp_policy(self, mlp):
+        """``set_mlp_policy`` unless this very network object is already uploaded (one upload per network object)."""
+        if getattr(self, "_mlp", None) is not mlp:
+            self.set_mlp_policy(mlp)
+
+    def selftest_mlp(self, obs) -> np.ndarray:
+        """The uploaded network evaluated by the rollout's device code on host observations [n, S] -> actions [n, A]."""
+        obs = np.ascontiguousarray(obs, np.float32).reshape(-1, self.S)
+        out = np.empty((obs.shape[0], self.A), np.float32)
+        N.check(N.lib().nig_selftest_mlp(self._h, obs.ctypes.data, obs.shape[0], out.ctypes.data))
+        return out
+
     def sync(self):
         N.check(N.lib().nig_sync(self._h))
 
