@@ -153,7 +153,9 @@ enum {
  *    core in the hardware's order; biases and activations are applied in fp32. Inputs are zero-padded to a multiple of 16
  *    (reactor 12 -> 16, robot 24 -> 32), the output to 16 columns; the padding is invisible.
  *  - actions are therefore specified to a tolerance against an fp64 forward pass of the bf16-rounded network, not bit for
- *    bit; everything downstream of the action keeps the bit-exact contract. Env i's action depends only on its own
+ *    bit (where every layer's exact sum is fp32-representable the order does not matter and the action is exact: bit for
+ *    bit with identity output, within tanhf's 2 ulp with tanh); everything downstream of the action keeps the bit-exact
+ *    contract. Env i's action depends only on its own
  *    observation and the weights (row i mod 128 of its tile), not on the population, slicing or launch shape.
  * Not supported (NIG_ERR_INVALID): more layers, other widths, other activations; stochastic actors; fp16 / fp8 / tf32 weights
  * (the ABI takes fp32, the library rounds to bf16). */

@@ -95,7 +95,8 @@ def assert_within(dev, ref, bound, what):
 
 
 NETS = [((64,), True, False), ((128, 128), False, True), ((256, 256), True, True), ((256, 64), False, False),
-        ((64, 256), True, False)]
+        ((64, 256), True, False), ((128,), False, True), ((256,), True, False), ((64, 64), False, True),
+        ((64, 128), True, True), ((128, 64), True, False), ((128, 256), False, False), ((256, 128), False, True)]
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -212,16 +213,22 @@ def _adversarial_start(env, orc, O, kind, rng, auto_reset=True):
 
 
 def _run(env, orc, tr, N, torch, chunks, ncons, extrema, what):
+    """One comparison per element of chunks: a launch of K steps, or a tuple of launches issued back to back (programmatic
+    dependent launch lets the next one start while the previous one runs) and compared launch by launch."""
     n = orc.n
-    rsum, vcnt, dcnt = env.empty(), env.empty(dtype=torch.int32), env.empty(dtype=torch.int32)
     for K in chunks:
-        env.rollout_device(K, N.POLICY_MLP, reward_sum=rsum, viol_count=vcnt, done_count=dcnt)
+        Ks = K if isinstance(K, tuple) else (K,)
+        outs = [(env.empty(), env.empty(dtype=torch.int32), env.empty(dtype=torch.int32)) for _ in Ks]
         torch.cuda.synchronize()
-        o_rs, o_v, o_d = tr.launch(K, lambda: env.selftest_mlp(orc.state))
-        w = f"{what} after a {K}-step launch"
-        assert_bits_equal(rsum[:n].cpu().numpy(), o_rs, f"{w}: per-env reward sum")
-        assert_bits_equal(vcnt[:n].cpu().numpy().astype(np.int64), o_v, f"{w}: per-env violation count")
-        assert_bits_equal(dcnt[:n].cpu().numpy().astype(np.int64), o_d, f"{w}: per-env done count")
+        for k, (rsum, vcnt, dcnt) in zip(Ks, outs):
+            env.rollout_device(k, N.POLICY_MLP, reward_sum=rsum, viol_count=vcnt, done_count=dcnt)
+        torch.cuda.synchronize()
+        for c, (k, (rsum, vcnt, dcnt)) in enumerate(zip(Ks, outs)):
+            o_rs, o_v, o_d = tr.launch(k, lambda: env.selftest_mlp(orc.state))
+            w = f"{what} after a {K}-step launch" if len(Ks) == 1 else f"{what}, launch {c} of {K} issued back to back"
+            assert_bits_equal(rsum[:n].cpu().numpy(), o_rs, f"{w}: per-env reward sum")
+            assert_bits_equal(vcnt[:n].cpu().numpy().astype(np.int64), o_v, f"{w}: per-env violation count")
+            assert_bits_equal(dcnt[:n].cpu().numpy().astype(np.int64), o_d, f"{w}: per-env done count")
         compare_state(env, orc, w)
         counters, sums = env.read_stats()
         compare_stats(N, counters, sums, tr, ncons, extrema, w, env.read_extrema())
@@ -239,30 +246,53 @@ def _generic_cons(N, kind):
     return [b[2], b[0], b[1], make_constraint(N.CON_BOUND, si=0, ai=0, coef=0.5, lo=lo, hi=hi, penalty=-7.0)]
 
 
-CASES = [  # name, n, cons, auto_reset, episode cap, extrema, launches
-    ("reactor", 1_000, "default", True, None, True, (40, 7)),
-    ("reactor", 4_099, "generic", True, 30, False, (33, 1)),
-    ("reactor", 1, "default", True, 20, True, (45,)),
-    ("reactor", 1_000, "default", False, 25, True, (40,)),
-    ("grid", 1_000, "default", True, None, True, (20, 5)),
-    ("grid", 4_133, "generic", True, 15, True, (20,)),
-    ("grid", 1_000, "default", False, 15, False, (25,)),
-    ("robot", 1_000, "default", True, 30, True, (40, 3)),
-    ("robot", 1_000, "generic", False, 20, True, (30,)),
+CASES = [  # name, n, cons, auto_reset, episode cap, extrema, launches, (hidden, tanh) or None: 128-128 (grid 256-256) tanh
+    ("reactor", 1_000, "default", True, None, True, (40, 7), None),
+    ("reactor", 4_099, "generic", True, 30, False, (33, 1), None),
+    ("reactor", 1, "default", True, 20, True, (45,), None),
+    ("reactor", 1_000, "default", False, 25, True, (40,), None),
+    ("grid", 1_000, "default", True, None, True, (20, 5), None),
+    ("grid", 4_133, "generic", True, 15, True, (20,), None),
+    ("grid", 1_000, "default", False, 15, False, (25,), None),
+    ("robot", 1_000, "default", True, 30, True, (40, 3), None),
+    ("robot", 1_000, "generic", False, 20, True, (30,), None),
+    # one hidden layer, and identity outputs beyond +-1: the env's clip of the action
+    ("reactor", 1_000, "default", True, None, True, (40,), ((64,), False)),
+    ("grid", 1_000, "generic", True, 15, True, (20,), ((256,), False)),
+    ("robot", 1_000, "default", True, 30, True, (30,), ((128,), True)),
+    ("robot", 1_000, "generic", False, 20, False, (25,), ((64, 256), False)),
+    # full tensor-memory occupancy on 148 SMs, two launches issued back to back: 2 CTAs per SM for two waves (256 columns),
+    # and 1 CTA per SM holding all 512 columns, so that a CTA of the second launch waits in tcgen05.alloc behind the first
+    ("reactor", 75_853, "default", True, 40, True, ((5, 3),), None),
+    ("grid", 37_965, "default", True, 30, True, ((4, 3),), None),
 ]
 
 
-@pytest.mark.parametrize("name,n,cons,auto_reset,cap,extrema,chunks", CASES)
-def test_rollout_vs_oracle(mods, name, n, cons, auto_reset, cap, extrema, chunks):
+def _case_id(i, case):
+    """pytest's default id of the first seven fields, then the network where it is not the default one."""
+    name, n, cons, auto_reset, cap, extrema, _, net = case
+    cid = f"{name}-{n}-{cons}-{auto_reset}-{cap}-{extrema}-chunks{i}"
+    return cid if net is None else f"{cid}-{'x'.join(map(str, net[0]))}-{'tanh' if net[1] else 'identity'}"
+
+
+@pytest.mark.parametrize("name,n,cons,auto_reset,cap,extrema,chunks,net", CASES,
+                         ids=[_case_id(i, c) for i, c in enumerate(CASES)])
+def test_rollout_vs_oracle(mods, name, n, cons, auto_reset, cap, extrema, chunks, net):
     """The fused MLP rollout == the oracle driven by nig_selftest_mlp, bit for bit after every launch, from the adversarial
-    start population, for CONS_DEFAULT and CONS_GENERIC, with and without auto-reset, with episode caps below K."""
+    start population, for CONS_DEFAULT and CONS_GENERIC, with and without auto-reset, with episode caps below K, one and two
+    hidden layers, identity outputs clipped by the env, and populations that fill every SM's tensor memory."""
     ni, N, O, torch = mods
     kind = KINDS[name]
     cs = None if cons == "default" else _generic_cons(N, kind)
-    env, orc = _start(ni, N, O, kind, n, seed=21, env_id_offset=5, max_episode_steps=cap, auto_reset=auto_reset, constraints=cs)
+    env, orc = _start(ni, N, O, kind, n, seed=21, env_id_offset=5, max_episode_steps=cap, auto_reset=auto_reset, constraints=cs,
+                      threads=O.max_threads() if n > 10_000 else 1)
     rng = np.random.default_rng(n)
     _adversarial_start(env, orc, O, kind, rng, auto_reset)
-    env.set_mlp_policy(make_mlp(ni, rng, env.S, env.A, (128, 128) if name != "grid" else (256, 256), True))
+    hidden, tanh = net or ((128, 128) if name != "grid" else (256, 256), True)
+    env.set_mlp_policy(make_mlp(ni, rng, env.S, env.A, hidden, tanh))
+    if not tanh:
+        a = env.selftest_mlp(orc.state)
+        assert (np.abs(a) > 1).mean() > 0.05, "the identity network's actions should exercise the clip"
     env.track_extrema(extrema)
     tr = Track(orc, name)
     _run(env, orc, tr, N, torch, chunks, 3 if cs is None else 4, extrema, f"{name} n={n} {cons}")
