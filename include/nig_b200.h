@@ -19,6 +19,10 @@
  *    `pitch` apart); host arrays are exact-size.
  *  - Envs are identified by a global id = env_id_offset + local index; all random streams are
  *    keyed by (seed, global id, tick) so a sharded run reproduces the unsharded one bit-for-bit.
+ *    Global ids are 32-bit: env_id_offset + n_envs (or + n_episodes of nig_dataset) must not exceed 2^32.
+ *  - The tick (one per batched step) is a uint32 Philox counter word and wraps modulo 2^32: stepping across the wrap is
+ *    the same as anywhere else. Explicit resets draw with the counter word (epoch << 8) | j, so the draws of epoch e and
+ *    e + 2^24 at the same tick coincide: a period of 2^24 explicit resets (auto-resets reuse the current epoch).
  */
 #ifndef NIG_B200_H
 #define NIG_B200_H
@@ -42,6 +46,11 @@ extern "C" {
 #define NIG_MAX_ACTION_DIM 8
 #define NIG_MAX_NOISE_DIM 23
 #define NIG_STATS_SLOTS 32
+/* Most steps one fused launch may run (nig_rollout_t.n_steps; nig_rollout_host caps steps_per_launch at it). A CTA counts
+ * its statistics in 32-bit registers and shared slots before it adds them to the int64 block: the largest is
+ * 256 envs x NIG_MAX_CONSTRAINTS x K violations (the two-env reactor kernel's 128-thread CTAs), < 2^31 at K = 2^20, and so
+ * are a one-warp CTA's 32 x 8 x K and every env's int32 viol_count of one launch. Above it the counters would wrap. */
+#define NIG_MAX_LAUNCH_STEPS (1 << 20)
 
 typedef struct nig_env nig_env_t; /* opaque */
 
@@ -94,7 +103,7 @@ typedef struct nig_config {
     int32_t env_kind;
     int32_t device;            /* CUDA device ordinal */
     int64_t n_envs;            /* envs owned by THIS handle (this GPU's shard) */
-    int64_t env_id_offset;     /* global id of local env 0 */
+    int64_t env_id_offset;     /* global id of local env 0; >= 0 and env_id_offset + n_envs <= 2^32 */
     uint64_t seed;
     int32_t max_episode_steps; /* 0 = env default; <= 65535 */
     int32_t auto_reset;        /* 1: a finished env is re-initialised inside the same step call */
@@ -215,7 +224,7 @@ enum {
 };
 
 typedef struct nig_rollout {
-    int32_t n_steps;            /* K */
+    int32_t n_steps;            /* K, 1 .. NIG_MAX_LAUNCH_STEPS (NIG_ERR_INVALID above) */
     int32_t policy;             /* NIG_POLICY_* */
     int32_t flags;              /* NIG_ROLLOUT_* */
     int32_t reserved;
@@ -311,7 +320,9 @@ NIG_API int nig_rollout_steps(nig_env_t* env, const nig_rollout_t* r, int32_t to
  * double-buffered so the copy of chunk c+1 overlaps the launch of chunk c). */
 typedef struct nig_rollout_host {
     int32_t n_steps;            /* T: total steps per env */
-    int32_t steps_per_launch;   /* K fused steps per kernel launch; 0 = T */
+    int32_t steps_per_launch;   /* K fused steps per kernel launch; 0 = T; either way at most NIG_MAX_LAUNCH_STEPS (a longer
+                                   horizon runs as several launches, whose fp32 reward sums are added launch by launch, as
+                                   for any K < T) */
     int32_t policy;             /* NIG_POLICY_* */
     int32_t reset_first;        /* 1: IndustrialEnv.reset() of every env before stepping (drawn, or init_states) */
     const float* init_states;   /* in  [n][S] AoS or NULL */
@@ -348,7 +359,11 @@ NIG_API int nig_dataset(nig_env_t* env, int64_t n_episodes, int32_t n_steps, int
 NIG_API int nig_dataset_size(nig_env_t* env, int64_t n_episodes, int32_t n_steps, int32_t policy,
                              const nig_policy_params_t* pp, int64_t* n_transitions, void* stream);
 
-/* checkpoint / teacher forcing: env.state, env.current_step, env.violation_count (base.py:50-57) */
+/* checkpoint / teacher forcing: env.state, env.current_step, env.violation_count (base.py:50-57). The episode word keeps the
+ * step in 16 bits and the violation count in 15, saturating at 32,767 (the kernels saturate a running count the same way; the
+ * per-env viol_count of the rollouts and the statistics block count every violation). Ranges of an import: ep_step in
+ * [0, 65535], ep_viol >= 0 (above 32,767 it saturates). nig_set_state_host rejects values outside them (NIG_ERR_INVALID,
+ * nothing imported); nig_set_state, whose arrays are on the device, clamps them into range. */
 NIG_API int nig_get_state(nig_env_t* env, float* state_dev, int32_t layout, int32_t* ep_step_dev, int32_t* ep_viol_dev, uint8_t* done_dev, void* stream);
 NIG_API int nig_set_state(nig_env_t* env, const float* state_dev, int32_t layout, const int32_t* ep_step_dev, const int32_t* ep_viol_dev, const uint8_t* done_dev, void* stream);
 NIG_API int nig_get_state_host(nig_env_t* env, float* state_aos, int32_t* ep_step, int32_t* ep_viol, uint8_t* done);

@@ -371,7 +371,8 @@ int reset_range(nig_env* e, const float* init_aos, int64_t i0, int64_t ns, uint3
 int rollout_checks(nig_env* e, const nig_rollout_t* r)
 {
     if (!r) return fail(NIG_ERR_INVALID, "nig_rollout: null descriptor");
-    if (r->n_steps <= 0) return fail(NIG_ERR_INVALID, "nig_rollout: n_steps must be positive (got %d)", r->n_steps);
+    if (r->n_steps <= 0 || r->n_steps > NIG_MAX_LAUNCH_STEPS)
+        return fail(NIG_ERR_INVALID, "nig_rollout: n_steps %d outside [1, NIG_MAX_LAUNCH_STEPS = %d]", r->n_steps, NIG_MAX_LAUNCH_STEPS);
     if (r->policy == NIG_POLICY_ACTIONS && !r->actions) return fail(NIG_ERR_INVALID, "nig_rollout: NIG_POLICY_ACTIONS needs an actions tensor");
     if (r->noise && e->NZ == 0) return fail(NIG_ERR_INVALID, "nig_rollout: env kind %d has no process noise", e->kind);
     if (r->noise && r->policy != NIG_POLICY_ACTIONS)
@@ -661,6 +662,8 @@ int nig_create(const nig_config_t* cfg, nig_env_t** out)
     if (cfg->n_envs <= 0) return fail(NIG_ERR_INVALID, "n_envs must be positive (got %lld)", (long long)cfg->n_envs);
     if (cfg->n_envs > (1LL << 31)) return fail(NIG_ERR_INVALID, "n_envs %lld exceeds 2^31", (long long)cfg->n_envs);
     if (cfg->max_episode_steps < 0 || cfg->max_episode_steps > 65535) return fail(NIG_ERR_INVALID, "max_episode_steps %d outside [0, 65535]", cfg->max_episode_steps);
+    if (cfg->env_id_offset < 0 || cfg->env_id_offset > (1LL << 32) - cfg->n_envs)      // global env ids are 32-bit
+        return fail(NIG_ERR_INVALID, "env ids env_id_offset %lld + [0, %lld) outside [0, 2^32)", (long long)cfg->env_id_offset, (long long)cfg->n_envs);
     int ndev = 0;
     if (nig_device_count(&ndev) != NIG_OK || ndev == 0) {
         char why[256];
@@ -953,6 +956,8 @@ int nig_rollout_steps(nig_env_t* e, const nig_rollout_t* r, int32_t total_steps,
     NIG_CHECK_ENV(e);
     if (!r) return fail(NIG_ERR_INVALID, "nig_rollout_steps: null descriptor");
     if (total_steps <= 0 || r->n_steps <= 0) return fail(NIG_ERR_INVALID, "nig_rollout_steps: total_steps and n_steps must be positive");
+    if (r->n_steps > NIG_MAX_LAUNCH_STEPS)
+        return fail(NIG_ERR_INVALID, "nig_rollout_steps: n_steps %d exceeds NIG_MAX_LAUNCH_STEPS = %d", r->n_steps, NIG_MAX_LAUNCH_STEPS);
     if (r->policy == NIG_POLICY_ACTIONS) return fail(NIG_ERR_UNSUPPORTED, "nig_rollout_steps: in-kernel policies only (teacher-forced actions: nig_rollout per chunk)");
     cudaStream_t st = (cudaStream_t)stream;
     note_device_work(e, st);
@@ -1158,7 +1163,8 @@ int nig_rollout_host(nig_env_t* e, const nig_rollout_host_t* r)
     if (r->noise && e->NZ == 0) return fail(NIG_ERR_INVALID, "nig_rollout_host: env kind %d has no process noise", e->kind);
     int rc;
     const size_t n = (size_t)e->n, cap = (size_t)e->pitch;
-    const int32_t T = r->n_steps, K = r->steps_per_launch > 0 && r->steps_per_launch < T ? r->steps_per_launch : T;
+    const int32_t T = r->n_steps;
+    const int32_t K = std::min(std::min(r->steps_per_launch > 0 ? r->steps_per_launch : T, T), (int32_t)NIG_MAX_LAUNCH_STEPS);
     cudaStream_t st = e->stream;
     const bool forced = r->policy == NIG_POLICY_ACTIONS;
     if (forced) {
@@ -1334,6 +1340,8 @@ int launch_dataset(nig_env* e, const DatasetArgs& a, cudaStream_t st)
 int dataset_args(nig_env* e, int64_t n_episodes, int32_t n_steps, int32_t policy, const nig_policy_params_t* pp, DatasetArgs* a)
 {
     if (n_episodes <= 0 || n_episodes > (1LL << 31)) return fail(NIG_ERR_INVALID, "n_episodes %lld outside [1, 2^31]", (long long)n_episodes);
+    if (e->cfg.env_id_offset > (1LL << 32) - n_episodes)          // episode e is the env of global id env_id_offset + e
+        return fail(NIG_ERR_INVALID, "episode ids env_id_offset %lld + [0, %lld) exceed 2^32", (long long)e->cfg.env_id_offset, (long long)n_episodes);
     if (n_steps <= 0) return fail(NIG_ERR_INVALID, "n_steps must be positive (got %d)", n_steps);
     if (policy == NIG_POLICY_MLP) return fail(NIG_ERR_UNSUPPORTED, "the dataset kernels have no NIG_POLICY_MLP flavour");
     if (policy != NIG_POLICY_UNIFORM && policy != NIG_POLICY_ZERO && policy != NIG_POLICY_PCTRL)
@@ -1457,6 +1465,10 @@ int nig_set_state_host(nig_env_t* e, const float* state_aos, const int32_t* st, 
     if (int hrc = host_entry(e)) return hrc;
     int rc;
     const size_t n = (size_t)e->n, cap = (size_t)e->pitch;
+    for (size_t i = 0; st && i < n; ++i)           // the episode word holds 16 bits of episode step
+        if (st[i] < 0 || st[i] > 65535) return fail(NIG_ERR_INVALID, "nig_set_state_host: ep_step[%zu] = %d outside [0, 65535]", i, st[i]);
+    for (size_t i = 0; vi && i < n; ++i)           // (above 32,767 it saturates like the kernels' running count)
+        if (vi[i] < 0) return fail(NIG_ERR_INVALID, "nig_set_state_host: ep_viol[%zu] = %d is negative", i, vi[i]);
     float* ds = nullptr; int32_t *dst = nullptr, *dvi = nullptr; uint8_t* ddn = nullptr;
     if (state_aos) {
         if ((rc = dev_alloc(&e->h_obs, cap * e->S)) != NIG_OK) return rc;

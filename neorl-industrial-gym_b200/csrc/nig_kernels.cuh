@@ -1108,9 +1108,10 @@ static __global__ void __launch_bounds__(kThreads) state_io_kernel(const __grid_
         if (p.ext_viol) p.ext_viol[i] = (int32_t)epw_viol(w);
         if (p.ext_done) p.ext_done[i] = (uint8_t)(w >> 31);
     } else if (p.ext_step || p.ext_viol || p.ext_done) {
+        // imported counters are clamped to what the word holds: step to [0, 65535], violations to [0, 32767] (epw_make)
         const uint32_t w = p.ep_word[i];
-        const uint32_t st = p.ext_step ? (uint32_t)p.ext_step[i] : epw_step(w);
-        const uint32_t vi = p.ext_viol ? (uint32_t)p.ext_viol[i] : epw_viol(w);
+        const uint32_t st = p.ext_step ? (uint32_t)min(max(p.ext_step[i], 0), 65535) : epw_step(w);
+        const uint32_t vi = p.ext_viol ? (uint32_t)max(p.ext_viol[i], 0) : epw_viol(w);
         const uint32_t dn = p.ext_done ? (uint32_t)(p.ext_done[i] != 0) : (w >> 31);
         p.ep_word[i] = epw_make(st, vi, dn);
         if (p.ep_return) p.ep_return[i] = 0.0;

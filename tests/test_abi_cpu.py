@@ -79,6 +79,28 @@ def test_no_gpu_means_loud_failure():
         ni.make("ChemicalReactor-v0", device="cpu")
 
 
+def test_create_rejects_env_ids_beyond_32_bits():
+    """Global env ids are 32-bit: nig_create refuses env_id_offset < 0 and env_id_offset + n_envs > 2^32 before it looks
+    for a device, so the range check answers NIG_ERR_INVALID with or without a GPU; the last valid offset passes it."""
+    lib = N.lib()
+
+    def create(n, off):
+        cfg = N.Config()
+        cfg.env_kind, cfg.device, cfg.n_envs, cfg.env_id_offset, cfg.n_constraints = N.ENV_CHEMICAL_REACTOR, 0, n, off, -1
+        h = C.c_void_p()
+        rc = lib.nig_create(C.byref(cfg), C.byref(h))
+        if h.value:
+            lib.nig_destroy(h)
+        return rc
+    for n, off in ((100, (1 << 32) - 99), (1, 1 << 32), (1 << 31, (1 << 31) + 1), (5, -1), (5, -(1 << 40))):
+        assert create(n, off) == N.ERR_INVALID, (n, off)
+        assert "2^32" in N.lib().nig_last_error().decode(), (n, off)
+    for n, off in ((100, (1 << 32) - 100), (1, (1 << 32) - 1)):
+        assert create(n, off) in (N.OK, N.ERR_NO_DEVICE), (n, off)
+    with pytest.raises(ValueError, match="2\\^32"):
+        ni.NativeEnv(N.ENV_POWER_GRID, 10, env_id_offset=(1 << 32) - 9)
+
+
 def test_product_never_imports_oracle():
     """The oracle is test infrastructure: nothing in the product may import, include, link or dlopen it."""
     pkg = os.path.join(ROOT, "neorl-industrial-gym_b200")

@@ -8,7 +8,8 @@ tests cannot lose their target silently when a dispatch threshold moves."""
 import numpy as np
 import pytest
 
-from util import KINDS, Track, adversarial, assert_bits_equal, compare_state, compare_stats, kernel_names
+from util import (KINDS, Track, adversarial, assert_bits_equal, compare_state, compare_stats, kernel_names, set_population,
+                  start_pair)
 
 pytestmark = pytest.mark.gpu
 
@@ -27,30 +28,6 @@ def mods():
 def _compare_window(env, N, tr, ncons, extrema, what):
     counters, sums = env.read_stats()
     compare_stats(N, counters, sums, tr, ncons, extrema, what, env.read_extrema())
-
-
-def _start(ni, N, O, kind, n, *, seed, env_id_offset=0, max_episode_steps=None, auto_reset=True, constraints=None,
-           threads=1):
-    env = ni.NativeEnv(kind, n, device=0, seed=seed, env_id_offset=env_id_offset, max_episode_steps=max_episode_steps,
-                       auto_reset=auto_reset, constraints=constraints)
-    kw = {}
-    if constraints is not None:
-        kw = {"builtin": False, "extra_cons": [O.Con(c.kind, c.id, c.si, c.ai, c.coef, c.lo, c.hi, c.penalty, c.critical)
-                                               for c in constraints]}
-    orc = O.OracleEnv(kind, n, auto_reset=auto_reset, seed=seed, env_id0=env_id_offset, exp_mode=1,
-                      max_episode_steps=max_episode_steps, threads=threads, **kw)
-    assert_bits_equal(env.reset_host(), orc.reset(), "reset draw")
-    return env, orc
-
-
-def _set_population(env, orc, st, ep_step, done=None):
-    n = orc.n
-    done = np.zeros(n, np.uint8) if done is None else done
-    env.set_state_host(st, ep_step, np.zeros(n, np.int32), done)
-    orc.state[:] = st
-    orc.ep_step[:] = ep_step
-    orc.ep_viol[:] = 0
-    orc.done_latch[:] = done
 
 
 def _run_launches(env, orc, tr, N, torch, chunks, policy_id, policy, ncons, extrema, params=None, what=""):
@@ -103,10 +80,10 @@ def test_pair_kernel_default_dispatch_vs_oracle(mods, extrema, max_steps):
     ends and auto-resets episodes inside the packed loop) == the oracle stepped one tick at a time."""
     ni, N, O, torch = mods
     n = PAIR_MIN + 4_099
-    env, orc = _start(ni, N, O, O.REACTOR, n, seed=6060, env_id_offset=1_001, max_episode_steps=max_steps,
-                      threads=O.max_threads())
+    env, orc = start_pair(ni, O, O.REACTOR, n, seed=6060, env_id_offset=1_001, max_episode_steps=max_steps,
+                          threads=O.max_threads())
     st, ep_step = _pair_population(O, np.random.default_rng(12), orc.state.copy(), n, env.max_episode_steps)
-    _set_population(env, orc, st, ep_step)
+    set_population(env, orc, st, ep_step)
     env.track_extrema(extrema)
     tr = Track(orc, "reactor")
     _run_launches(env, orc, tr, N, torch, (64, 17, 1, 70), N.POLICY_UNIFORM,
@@ -125,12 +102,12 @@ def test_pair_kernel_forced_small_vs_oracle(mods, monkeypatch, block, extrema, a
     monkeypatch.setenv("NIG_ROLLOUT_PAIR", "1")
     monkeypatch.setenv("NIG_ROLLOUT_BLOCK", str(block))
     n = 4_096 + 37
-    env, orc = _start(ni, N, O, O.REACTOR, n, seed=77, env_id_offset=333, max_episode_steps=60, auto_reset=auto_reset)
+    env, orc = start_pair(ni, O, O.REACTOR, n, seed=77, env_id_offset=333, max_episode_steps=60, auto_reset=auto_reset)
     rng = np.random.default_rng(block)
     st, ep_step = adversarial(O, O.REACTOR, rng, orc.state.copy(), n, 60)
     st[2 * 700, 8] = 1.0; st[2 * 900 + 1, 9] = 0.5; st[64 * 40:64 * 41, 8] = 1.0
     done = None if auto_reset else (rng.random(n) < 0.05).astype(np.uint8)
-    _set_population(env, orc, st, ep_step, done)
+    set_population(env, orc, st, ep_step, done)
     env.track_extrema(extrema)
     tr = Track(orc, "reactor")
     _run_launches(env, orc, tr, N, torch, (64, 17, 1, 70), N.POLICY_UNIFORM,
@@ -145,7 +122,7 @@ def test_pair_kernel_in_sliced_device_rollout_vs_oracle(mods):
     replay): per-env sums in the device's chunked fp32 order, states, counters and statistics == the oracle."""
     ni, N, O, torch = mods
     n, T, K = (1 << 20) - 1_000, 150, 64
-    env, orc = _start(ni, N, O, O.REACTOR, n, seed=2027, env_id_offset=5, max_episode_steps=100, threads=O.max_threads())
+    env, orc = start_pair(ni, O, O.REACTOR, n, seed=2027, env_id_offset=5, max_episode_steps=100, threads=O.max_threads())
     tr = Track(orc, "reactor")
     policy = lambda: O.policy_actions(orc, O.POLICY_UNIFORM)
     rsum, vcnt, dcnt = env.empty(), env.empty(dtype=torch.int32), env.empty(dtype=torch.int32)
@@ -178,7 +155,7 @@ def test_pair_kernel_in_host_rollout_vs_oracle(mods, monkeypatch, direct):
     monkeypatch.setenv("NIG_HOST_DIRECT", "3" if direct else "0")
     monkeypatch.setenv("NIG_HOST_DIRECT_MAX_MB", "1e9")
     n, T, K = (1 << 18) + 77, 150, 64
-    env, orc = _start(ni, N, O, O.REACTOR, n, seed=88, env_id_offset=3, max_episode_steps=100, threads=O.max_threads())
+    env, orc = start_pair(ni, O, O.REACTOR, n, seed=88, env_id_offset=3, max_episode_steps=100, threads=O.max_threads())
     tr = Track(orc, "reactor")
     policy = lambda: O.policy_actions(orc, O.POLICY_UNIFORM)
     for call in range(2):
@@ -318,7 +295,7 @@ def test_zero_policy_vs_oracle(mods, name, extrema, cons):
     ni, N, O, torch = mods
     kind, n = KINDS[name], 3_000
     cs = None if cons == "default" else _bound_cons(N, kind)
-    env, orc = _start(ni, N, O, kind, n, seed=44, env_id_offset=17, max_episode_steps=50, constraints=cs)
+    env, orc = start_pair(ni, O, kind, n, seed=44, env_id_offset=17, max_episode_steps=50, constraints=cs)
     env.track_extrema(extrema)
     tr = Track(orc, name)
     _run_launches(env, orc, tr, N, torch, (70, 33), N.POLICY_ZERO, lambda: O.policy_actions(orc, O.POLICY_ZERO),
@@ -360,7 +337,7 @@ def test_random_baseline_vs_oracle(mods, name, extrema):
     from neorl_industrial.benchmarks import BaselineAgentFactory
     kind, n = KINDS[name], 3_000
     lo, hi = -0.3, 0.55
-    env, orc = _start(ni, N, O, kind, n, seed=13, env_id_offset=9, max_episode_steps=50)
+    env, orc = start_pair(ni, O, kind, n, seed=13, env_id_offset=9, max_episode_steps=50)
     pid, pp = BaselineAgentFactory.create("random", env.S, env.A, action_low=lo, action_high=hi).device_policy()
     assert pid == N.POLICY_BASELINE and pp.baseline.kind == N.BASELINE_RANDOM
     mid, half = np.float32(0.5 * (lo + hi)), np.float32(0.5 * (hi - lo))
@@ -387,7 +364,7 @@ def test_pid_mpc_baselines_with_extrema_and_bound_vs_host_agents(mods, name, kin
         sp = {"reactor": [320.0, 253312.0, 50.0], "grid": [0.0] + [1.0] * 7, "robot": [0.3, 0.0, 0.4, 0, 0, 0, 1.0]}[name]
         kw = {"kp": 0.05, "ki": 0.001, "kd": 0.02, "setpoint": np.array(sp, np.float64)}
     cs = _bound_cons(N, ek)
-    env, orc = _start(ni, N, O, ek, n, seed=5, env_id_offset=2, max_episode_steps=30, constraints=cs)
+    env, orc = start_pair(ni, O, ek, n, seed=5, env_id_offset=2, max_episode_steps=30, constraints=cs)
     pid, pp = Factory.create(kind, env.S, env.A, **kw).device_policy()
     agents = [Factory.create(kind, env.S, env.A, **kw) for _ in range(n)]
     env.track_extrema(True)
@@ -412,9 +389,9 @@ def test_opt_in_shapes_vs_oracle(mods, monkeypatch, case, extrema):
     for k, v in envvars.items():
         monkeypatch.setenv(k, v)
     kind, n = KINDS[name], 4_096 + 37
-    env, orc = _start(ni, N, O, kind, n, seed=21, env_id_offset=96, max_episode_steps=60 if name == "reactor" else None)
+    env, orc = start_pair(ni, O, kind, n, seed=21, env_id_offset=96, max_episode_steps=60 if name == "reactor" else None)
     st, ep_step = adversarial(O, kind, np.random.default_rng(kind + 3), orc.state.copy(), n, env.max_episode_steps)
-    _set_population(env, orc, st, ep_step)
+    set_population(env, orc, st, ep_step)
     env.track_extrema(extrema)
     tr = Track(orc, name)
     _run_launches(env, orc, tr, N, torch, (48, 17, 1, 64), N.POLICY_UNIFORM,

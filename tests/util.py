@@ -171,6 +171,33 @@ class Track:
         return rsum, vcnt, dcnt
 
 
+def start_pair(ni, O, kind, n, *, seed, env_id_offset=0, max_episode_steps=None, auto_reset=True, constraints=None,
+               threads=1):
+    """A NativeEnv and the oracle configured alike (constraint set, episode cap, ids), from the same checked reset draw."""
+    env = ni.NativeEnv(kind, n, device=0, seed=seed, env_id_offset=env_id_offset, max_episode_steps=max_episode_steps,
+                       auto_reset=auto_reset, constraints=constraints)
+    kw = {}
+    if constraints is not None:
+        kw = {"builtin": False, "extra_cons": [O.Con(c.kind, c.id, c.si, c.ai, c.coef, c.lo, c.hi, c.penalty, c.critical)
+                                               for c in constraints]}
+    orc = O.OracleEnv(kind, n, auto_reset=auto_reset, seed=seed, env_id0=env_id_offset, exp_mode=1,
+                      max_episode_steps=max_episode_steps, threads=threads, **kw)
+    assert_bits_equal(env.reset_host(), orc.reset(), "reset draw")
+    return env, orc
+
+
+def set_population(env, orc, st, ep_step, done=None, ep_viol=None):
+    """Imports the same states and episode counters on both sides."""
+    n = orc.n
+    done = np.zeros(n, np.uint8) if done is None else done
+    ep_viol = np.zeros(n, np.int32) if ep_viol is None else ep_viol
+    env.set_state_host(st, ep_step, ep_viol, done)
+    orc.state[:] = st
+    orc.ep_step[:] = ep_step
+    orc.ep_viol[:] = ep_viol
+    orc.done_latch[:] = done
+
+
 def _close(got, want, rtol, atol, what):
     if np.isnan(want):
         assert np.isnan(got), (what, got, want)
