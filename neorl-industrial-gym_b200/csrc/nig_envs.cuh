@@ -76,14 +76,16 @@ struct Reactor {
         }
     };
     // action_space.sample() (performance_benchmark.py:118) from words z, w of the step's block: a0 / a1 from bits 21..0 of
-    // z / w, a2 from the two 10-bit tops; the bits go straight into the mantissa of a float in [1, 2) (one LOP3 each, no
-    // int -> float conversion) and one exact fma maps it to [-1, 1): a0, a1 = v * 2^-21 - 1, a2 = v * 2^-19 - 1
+    // z / w, a2 from the two 10-bit tops; the bits go straight into the mantissa of a float in [4, 6) / [16, 18) (one LOP3
+    // each, no int -> float conversion) and one exact add maps it to [-1, 1): a0, a1 = v * 2^-21 - 1, a2 = v * 2^-19 - 1.
+    // (The same values as fma(1 + v * 2^-23, 4 or 16, -5 or -17): the sums are multiples of 2^-21 / 2^-19 below 2 in
+    // magnitude, exact in binary32, and an add needs no second constant in a register.)
     __device__ static __forceinline__ void uniform_from_words(uint32_t wz, uint32_t ww, float (&a)[A])
     {
-        a[0] = __fmaf_rn(__uint_as_float((wz & 0x3fffffu) | 0x3f800000u), 4.0f, -5.0f);
-        a[1] = __fmaf_rn(__uint_as_float((ww & 0x3fffffu) | 0x3f800000u), 4.0f, -5.0f);
+        a[0] = __fadd_rn(__uint_as_float((wz & 0x3fffffu) | 0x40800000u), -5.0f);
+        a[1] = __fadd_rn(__uint_as_float((ww & 0x3fffffu) | 0x40800000u), -5.0f);
         const uint32_t v2 = __funnelshift_l(ww, wz >> 22, 10);          // (wz[31:22] << 10) | ww[31:22]
-        a[2] = __fmaf_rn(__uint_as_float(v2 | 0x3f800000u), 16.0f, -17.0f);
+        a[2] = __fadd_rn(__uint_as_float(v2 | 0x41800000u), -17.0f);
     }
     __device__ static __forceinline__ void uniform_actions(const Rng& key, uint32_t env, uint32_t tick, float (&a)[A])
     {
