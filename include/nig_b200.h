@@ -40,7 +40,7 @@ extern "C" {
 #define NIG_API
 #endif
 
-#define NIG_ABI_VERSION 5
+#define NIG_ABI_VERSION 6
 #define NIG_MAX_CONSTRAINTS 8
 #define NIG_MAX_STATE_DIM 32
 #define NIG_MAX_ACTION_DIM 8
@@ -295,6 +295,31 @@ NIG_API int nig_step_host(nig_env_t* env, const nig_step_io_t* io);
 /* K fused steps with state in registers: the `for step: action = policy(obs); env.step(action)` loops of
  * performance_benchmark.py:106-133, utils.evaluate_with_safety (utils.py:82-125) and get_dataset */
 NIG_API int nig_rollout(nig_env_t* env, const nig_rollout_t* r, void* stream);
+/* nig_rollout that also records every step: the per-step tuple (obs, action, reward, terminated, truncated, info) of
+ * `for t in range(K): env.step(policy(obs))` -- the caller's own gym vector-env loop that stores each step -- written by the one
+ * fused launch into time-major device arrays. Everything nig_rollout does, the call does too, bit for bit, with the same
+ * descriptor: state, episode words and returns, tick (+K), per-env reward_sum / viol_count / done_count (NIG_ROLLOUT_ACCUMULATE
+ * included), the statistics block, the return extrema and the PID controller state; recording is a side output. Validation is
+ * nig_rollout's (same statuses for the same descriptor); out == NULL is NIG_ERR_INVALID, a descriptor whose fields are all NULL
+ * records nothing. NIG_ROLLOUT_USE_TMA is accepted and has no effect. One launch on `stream`; the device tick modes of
+ * nig_use_device_tick apply as for nig_rollout (the call can be captured into a CUDA graph). Row (t, i) holds exactly what
+ * nig_step writes for env i stepped with the recorded action at the same tick: obs[t] is nig_step's post-auto-reset obs of
+ * step t - 1 (row 0: the state at the call); an inactive env (auto_reset == 0, already finished) keeps its state, reward 0,
+ * flags NIG_F_INACTIVE, viol_mask 0. The kernel runs rollout_kernel's generic loop (or the MLP rollout's), not the
+ * specialised throughput loops of nig_rollout. */
+typedef struct nig_trajectory {
+    /* device arrays, time-major, exact-size rows ([K][n][dim]: row t * n + i is env i at step t of this call, the layout of a
+     * contiguous torch tensor [K, n, dim]); NULL = not recorded. Offsets are 64-bit: K * n * S may exceed 2^31. */
+    float*   obs;         /* [K][n][S] s_t: the observation the policy acted on (row 0 = the state at the call) */
+    float*   actions;     /* [K][n][A] the action handed to the env at step t, BEFORE the env's clip to [-1, 1] */
+    float*   rewards;     /* [K][n]    */
+    uint8_t* flags;       /* [K][n]    NIG_F_* bits */
+    uint8_t* viol_mask;   /* [K][n]    bit k = constraint k violated on s_t */
+    uint8_t* terminated;  /* [K][n]    0/1 */
+    uint8_t* truncated;   /* [K][n]    0/1 */
+    float*   next_obs;    /* [K][n][S] s' of the transition, before auto-reset (gym's final_observation) */
+} nig_trajectory_t;
+NIG_API int nig_rollout_record(nig_env_t* env, const nig_rollout_t* r, const nig_trajectory_t* out, void* stream);
 /* total_steps steps of every env as ceil(total_steps / r->n_steps) fused launches (in-kernel policies only). On a large
  * population the envs are split into slices that advance on internal streams forked from and joined back to `stream`
  * (NIG_HOST_SLICES, default 8, >= 8,192 envs per slice): a slice's next launch fills the SMs another slice's tail leaves

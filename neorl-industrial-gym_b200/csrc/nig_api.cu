@@ -411,8 +411,10 @@ int host_slices(const nig_env* e, bool forced, int want = 4)
     return want < 1 ? 1 : want;
 }
 
-// one fused launch over envs [i0, i0 + ns) at an explicit tick (validation and e->tick bookkeeping are the callers')
-int rollout_range(nig_env* e, const nig_rollout_t* r, cudaStream_t stream, int64_t i0, int64_t ns, uint32_t tick)
+// one fused launch over envs [i0, i0 + ns) at an explicit tick (validation and e->tick bookkeeping are the callers'); with
+// `record` (nig_rollout_record: whole population only) the recording kernels instead of nig_rollout's
+int rollout_range(nig_env* e, const nig_rollout_t* r, cudaStream_t stream, int64_t i0, int64_t ns, uint32_t tick,
+                  const nig_trajectory_t* record = nullptr)
 {
     RolloutArgs a;
     memset(&a, 0, sizeof a);
@@ -450,7 +452,8 @@ int rollout_range(nig_env* e, const nig_rollout_t* r, cudaStream_t stream, int64
     cfg.mlp.extrema = e->track_extrema ? 1 : 0;
     e->launches++;
     const int64_t extent = (ns + 127) / 128 * 128;          // launch extent; <= the rows' pitch because slices start at multiples of 128
-    NIG_CUDA(nig::launch_rollout(e->kind, cfg, extent, a, map, stream));
+    if (record) NIG_CUDA(nig::launch_rollout_record(e->kind, cfg, extent, a, *record, stream));
+    else NIG_CUDA(nig::launch_rollout(e->kind, cfg, extent, a, map, stream));
     return NIG_OK;
 }
 
@@ -947,6 +950,17 @@ int nig_rollout(nig_env_t* e, const nig_rollout_t* r, void* stream)
     if (int crc = rollout_checks(e, r)) return crc;
     note_device_work(e, (cudaStream_t)stream);
     if (int rc = rollout_range(e, r, (cudaStream_t)stream, 0, e->n, e->tick)) return rc;
+    e->tick += (uint32_t)r->n_steps;
+    return NIG_OK;
+}
+
+int nig_rollout_record(nig_env_t* e, const nig_rollout_t* r, const nig_trajectory_t* out, void* stream)
+{
+    NIG_CHECK_ENV(e);
+    if (!out) return fail(NIG_ERR_INVALID, "nig_rollout_record: null trajectory descriptor");
+    if (int crc = rollout_checks(e, r)) return crc;
+    note_device_work(e, (cudaStream_t)stream);
+    if (int rc = rollout_range(e, r, (cudaStream_t)stream, 0, e->n, e->tick, out)) return rc;
     e->tick += (uint32_t)r->n_steps;
     return NIG_OK;
 }

@@ -578,8 +578,8 @@ __device__ __forceinline__ void store_rows(float* base, int64_t pitch, int64_t n
 // AoS rows ([n][D] row-major: the layout of the host and torch APIs) through a per-warp shared-memory transpose, so
 // that the global accesses of a warp are D fully coalesced 128-byte requests instead of D requests that each touch 32
 // sectors (measured at 4M envs with obs + next_obs outputs, tools/aos_vs_soa.py: reactor 340 -> 197 us, grid 1553 -> 652 us).
-// One env per lane.
-template <int D>
+// One env per lane. STREAM: evict-first stores (__stcs) for outputs nothing in the kernel reads again (nig_rollout_record).
+template <int D, bool STREAM = false>
 __device__ __forceinline__ void store_aos_warp(float* base, int64_t n, int64_t i, const float (&v)[D], float* tile)
 {
     const int lane = threadIdx.x & 31;
@@ -591,7 +591,10 @@ __device__ __forceinline__ void store_aos_warp(float* base, int64_t n, int64_t i
     for (int it = 0; it < D; ++it) {
         const int j = it * 32 + lane;           // float index inside the warp's [32][D] block
         const int e = j / D, k = j - e * D;
-        if (env0 + e < n) base[env0 * D + j] = tile[e * (D + 1) + k];
+        if (env0 + e < n) {
+            if constexpr (STREAM) __stcs(base + env0 * D + j, tile[e * (D + 1) + k]);
+            else base[env0 * D + j] = tile[e * (D + 1) + k];
+        }
     }
     __syncwarp();
 }
@@ -2343,8 +2346,8 @@ __global__ void __launch_bounds__(kThreads, Env::ROLLOUT_MIN_CTAS) rollout_kerne
             } else ng.get(key, env, tick, nz);
         } else nz[0] = 0.0f;
 
-        // this step-and-bookkeeping block is repeated statement for statement in rollout_step_generic (nig_rollout_mlp.cu,
-        // the MLP policy's kernel) and, for the uniform policy, in rollout_generic_uniform_step: a change here goes there too
+        // this step-and-bookkeeping block is repeated statement for statement in rollout_step_generic (nig_mlp.cuh, the
+        // kernels of the MLP policy and of nig_rollout_record) and, for the uniform policy, in rollout_generic_uniform_step: a change here goes there too
         // (moving it into a shared function changed ptxas' schedule of this kernel's reactor instantiations)
         const bool active = valid && !latched;
         uint32_t st2, vi2, f, vm;

@@ -1,5 +1,5 @@
 // nig_launch.h -- kernel launchers, one translation unit per kernel family so the library builds in parallel
-// (nig_step.cu, nig_rollout_{reactor,grid,robot}.cu, nig_dataset.cu, nig_misc.cu). nig_api.cu holds no kernels.
+// (nig_step.cu, nig_rollout_{reactor,grid,robot,mlp,record}.cu, nig_dataset.cu, nig_misc.cu). nig_api.cu holds no kernels.
 #pragma once
 #include "nig_kernels.cuh"
 
@@ -69,6 +69,8 @@ cudaError_t launch_rollout_reactor(const RolloutLaunch& cfg, int64_t pitch, cons
 cudaError_t launch_rollout_grid(const RolloutLaunch& cfg, int64_t pitch, const RolloutArgs& a, const CUtensorMap& map, cudaStream_t st);
 cudaError_t launch_rollout_robot(const RolloutLaunch& cfg, int64_t pitch, const RolloutArgs& a, const CUtensorMap& map, cudaStream_t st);
 cudaError_t launch_rollout_mlp(int kind, const RolloutLaunch& cfg, int64_t pitch, const RolloutArgs& a, cudaStream_t st);
+cudaError_t launch_rollout_record(int kind, const RolloutLaunch& cfg, int64_t pitch, const RolloutArgs& a, const nig_trajectory_t& out,
+                                  cudaStream_t st);
 cudaError_t launch_selftest_mlp(int kind, const MlpParams& m, const float* obs, float* act, int64_t n, cudaStream_t st);
 cudaError_t launch_dataset(int kind, int cons, bool write, const DatasetArgs& a, cudaStream_t st);
 cudaError_t launch_reset(int kind, const ResetArgs& a, cudaStream_t st);

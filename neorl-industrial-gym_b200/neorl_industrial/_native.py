@@ -16,7 +16,7 @@ _ROOT = os.path.dirname(_PKG_DIR)                       # neorl-industrial-gym_b
 LIB_PATH = os.environ.get("NIG_LIB_PATH") or os.path.join(_ROOT, "libnig_b200.so")   # (override: A/B builds, tools/ab_build.sh)
 CSRC_DIR = os.path.join(_ROOT, "csrc")
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 MAX_CONSTRAINTS = 8
 STATS_SLOTS = 32
 
@@ -79,6 +79,12 @@ class Rollout(C.Structure):
                 ("reward_sum", C.c_void_p), ("viol_count", C.c_void_p), ("done_count", C.c_void_p)]
 
 
+class Trajectory(C.Structure):
+    """nig_trajectory_t: the per-step device arrays of nig_rollout_record, time-major [K][n][dim] (NULL = not recorded)."""
+    _fields_ = [("obs", C.c_void_p), ("actions", C.c_void_p), ("rewards", C.c_void_p), ("flags", C.c_void_p),
+                ("viol_mask", C.c_void_p), ("terminated", C.c_void_p), ("truncated", C.c_void_p), ("next_obs", C.c_void_p)]
+
+
 class RolloutHost(C.Structure):
     _fields_ = [("n_steps", C.c_int32), ("steps_per_launch", C.c_int32), ("policy", C.c_int32), ("reset_first", C.c_int32),
                 ("init_states", C.c_void_p), ("actions", C.c_void_p), ("noise", C.c_void_p), ("pp", PolicyParams),
@@ -116,6 +122,7 @@ SYMBOLS = {
     "nig_step": (C.c_int, [_VP, C.POINTER(StepIO), _VP]),
     "nig_step_host": (C.c_int, [_VP, C.POINTER(StepIO)]),
     "nig_rollout": (C.c_int, [_VP, C.POINTER(Rollout), _VP]),
+    "nig_rollout_record": (C.c_int, [_VP, C.POINTER(Rollout), C.POINTER(Trajectory), _VP]),
     "nig_rollout_steps": (C.c_int, [_VP, _VP, C.c_int32, _VP]),
     "nig_rollout_host": (C.c_int, [_VP, C.POINTER(RolloutHost)]),
     "nig_reset_policy_state": (C.c_int, [_VP, _VP]),

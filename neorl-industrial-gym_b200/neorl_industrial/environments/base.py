@@ -17,7 +17,7 @@ import numpy as np
 
 from .. import _native as N
 from ..core.types import BatchedSafetyMetrics, SafetyConstraint, SafetyMetrics
-from ..policies import MLPPolicy
+from ..rollouts import resolve_policy
 from ..spaces import Box
 from ..vector import NativeEnv, make_constraint
 
@@ -322,8 +322,6 @@ class IndustrialEnv:
             return obs.copy(), reward.copy(), terminated, truncated, info
         return obs, reward, terminated, truncated, info
 
-    _POLICY_IDS = {"random": N.POLICY_UNIFORM, "uniform": N.POLICY_UNIFORM, "zero": N.POLICY_ZERO}
-
     def rollout(self, n_steps: int, policy="random", *, steps_per_launch: int = 64, reset: bool = False, init_states=None,
                 actions=None, noise=None, params=None) -> Dict[str, Any]:
         """The reference's timing / evaluation loop -- ``for _ in range(n_steps): env.step(policy(obs))`` with reset on done
@@ -339,30 +337,13 @@ class IndustrialEnv:
         if self._host_constraints():
             raise NotImplementedError("callable safety constraints cannot run inside the fused rollout kernel; "
                                       "use BoundConstraint / built-in constraints, or step()")
-        if actions is not None or policy == "actions":
-            if actions is None:
-                raise ValueError("policy='actions' needs an actions array [T, num_envs, A]")
-            pid = N.POLICY_ACTIONS
+        pid, params = resolve_policy(nat, policy, params, actions)
+        if pid == N.POLICY_ACTIONS:
             a = np.asarray(actions, np.float32).reshape(int(n_steps), self.num_envs, self.action_dim)
             actions = np.ascontiguousarray(a.transpose(0, 2, 1))            # [T, A, n]: what the kernel streams
             if noise is not None:
                 z = np.asarray(noise, np.float32).reshape(int(n_steps), self.num_envs, nat.NZ)
                 noise = np.ascontiguousarray(z.transpose(0, 2, 1))
-        elif hasattr(policy, "device_policy"):                 # benchmarks.baseline_agents controllers, in-kernel
-            pid, params = policy.device_policy()
-        elif isinstance(policy, MLPPolicy):                    # a learned actor on the tensor cores, in-kernel
-            nat.use_mlp_policy(policy)
-            pid = N.POLICY_MLP
-        elif policy == "dataset":
-            if params is None:
-                raise ValueError("policy='dataset' needs PolicyParams (see datasets.policy_params)")
-            pid = N.POLICY_PCTRL
-        else:
-            try:
-                pid = self._POLICY_IDS[policy]
-            except KeyError:
-                raise ValueError(f"unknown rollout policy {policy!r}; expected one of "
-                                 f"{sorted(self._POLICY_IDS) + ['dataset', 'actions']}") from None
         out = nat.rollout_host(n_steps, pid, steps_per_launch=steps_per_launch, params=params, init_states=init_states,
                                reset_first=reset or self._state is None, actions=actions, noise=noise)
         self._state = out["obs"]

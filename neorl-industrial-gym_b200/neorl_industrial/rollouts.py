@@ -20,6 +20,34 @@ from . import _native as N
 from .policies import MLPPolicy
 
 
+ROLLOUT_POLICY_IDS = {"random": N.POLICY_UNIFORM, "uniform": N.POLICY_UNIFORM, "zero": N.POLICY_ZERO}
+
+
+def resolve_policy(nat, policy, params=None, actions=None):
+    """The ``policy`` argument of ``IndustrialEnv.rollout`` and ``TorchIndustrialEnv.rollout`` -> (NIG_POLICY_* id, params):
+    "random" / "uniform" / "zero", "dataset" with ``params`` (the get_dataset controllers), a ``benchmarks.baseline_agents``
+    controller object, an ``MLPPolicy`` (uploaded to ``nat`` once per network object), or teacher-forced ``actions``
+    (``policy="actions"`` or any policy with ``actions`` given; the caller lays them out for the kernel)."""
+    if actions is not None or policy == "actions":
+        if actions is None:
+            raise ValueError("policy='actions' needs an actions array [T, num_envs, A]")
+        return N.POLICY_ACTIONS, params
+    if hasattr(policy, "device_policy"):                   # benchmarks.baseline_agents controllers, in-kernel
+        return policy.device_policy()
+    if isinstance(policy, MLPPolicy):                      # a learned actor on the tensor cores, in-kernel
+        nat.use_mlp_policy(policy)
+        return N.POLICY_MLP, params
+    if policy == "dataset":
+        if params is None:
+            raise ValueError("policy='dataset' needs PolicyParams (see datasets.policy_params)")
+        return N.POLICY_PCTRL, params
+    try:
+        return ROLLOUT_POLICY_IDS[policy], params
+    except KeyError:
+        raise ValueError(f"unknown rollout policy {policy!r}; expected one of "
+                         f"{sorted(ROLLOUT_POLICY_IDS) + ['dataset', 'actions']}") from None
+
+
 def metrics_from_stats(stats: Dict[str, Any], n_constraints: int, critical_flags) -> Dict[str, Any]:
     """Reference result dict (utils.py:128-152) from summed device counters."""
     ep = max(int(stats["episodes"]), 1)

@@ -5,13 +5,15 @@ signature of the reference (environments/base.py:133-213) with a leading env axi
 the env's device (``obs [n, S]`` fp32, ``reward [n]`` fp32, ``terminated`` / ``truncated [n]`` bool), and each call is
 exactly one kernel launch on torch's current stream. Auto-reset is on: a finished env is re-initialised inside the
 same launch; ``info["final_observation"]`` holds s' of the finished transition. ``capture_graph()`` records K steps
-driven by a policy callable into a CUDA graph (device-resident tick) and returns a replay function.
+driven by a policy callable into a CUDA graph (device-resident tick) and returns a replay function; ``rollout()`` runs K steps
+of an in-kernel policy (or teacher-forced actions) as one fused launch and returns every step's tuple as [K, n, ...] tensors.
 """
 from __future__ import annotations
 
 from typing import Any, Callable, Dict, Optional, Tuple
 
 from . import _native as N
+from .rollouts import resolve_policy
 from .vector import KIND_BY_ID, NativeEnv
 
 
@@ -67,6 +69,41 @@ class TorchIndustrialEnv:
         if self._final is not None:
             info["final_observation"] = self._final
         return self._obs, self._reward[:n], self._term[:n], self._trunc[:n], info
+
+    # rollout()'s keys -> nig_trajectory_t fields (the names of step()'s return and info)
+    ROLLOUT_KEYS = {"obs": "obs", "actions": "actions", "rewards": "rewards", "terminated": "terminated",
+                    "truncated": "truncated", "final_observation": "next_obs", "flags": "flags", "violation_mask": "viol_mask"}
+
+    def rollout(self, n_steps: int, policy="random", *, params=None, actions=None, out=None) -> Dict[str, Any]:
+        """``n_steps`` iterations of ``obs -> policy(obs) -> step`` recorded step by step in ONE fused kernel launch
+        (nig_rollout_record), continuing from the current state. Returns time-major CUDA tensors: obs [T, n, S] (the
+        observation the policy acted on), actions [T, n, A] (before the env's clip), rewards [T, n], terminated / truncated
+        [T, n] bool, final_observation [T, n, S] (s' before the auto-reset), flags / violation_mask [T, n] uint8 -- what a loop
+        of ``step`` calls that stores every result holds. The observation buffer of ``step`` / ``reset`` then holds the current
+        state, so a following ``step`` carries on seamlessly. ``policy`` as in ``IndustrialEnv.rollout`` and evaluated inside
+        the kernel: "random", "zero", "dataset" with ``params``, a baseline agent, an ``MLPPolicy``; or ``actions`` [T, n, A]
+        teacher-forces every step. ``out`` (optional): preallocated tensors under any of these keys, filled in place."""
+        import torch
+        nat, n, T = self.native, self.num_envs, int(n_steps)
+        pid, params = resolve_policy(nat, policy, params, actions)
+        a_dev = None
+        if pid == N.POLICY_ACTIONS:
+            if not torch.is_tensor(actions) or tuple(actions.shape) != (T, n, self.action_dim):
+                raise ValueError(f"actions must be a tensor of shape ({T}, {n}, {self.action_dim})")
+            a_dev = torch.zeros((T, self.action_dim, nat.pitch), dtype=torch.float32, device=self.device)
+            a_dev[:, :, :n] = actions.to(device=self.device, dtype=torch.float32).transpose(1, 2)   # [T][A][pitch]: the kernel's rows
+        out = dict(out or {})
+        for key in out:
+            if key not in self.ROLLOUT_KEYS:
+                raise ValueError(f"unknown rollout output {key!r}; expected a subset of {sorted(self.ROLLOUT_KEYS)}")
+        shapes = {"obs": (T, n, self.state_dim), "actions": (T, n, self.action_dim), "final_observation": (T, n, self.state_dim)}
+        dtypes = {"terminated": torch.bool, "truncated": torch.bool, "flags": torch.uint8, "violation_mask": torch.uint8}
+        for key in self.ROLLOUT_KEYS:
+            if out.get(key) is None:
+                out[key] = torch.empty(shapes.get(key, (T, n)), dtype=dtypes.get(key, torch.float32), device=self.device)
+        nat.rollout_record_device(T, pid, out={f: out[k] for k, f in self.ROLLOUT_KEYS.items()}, actions=a_dev, params=params)
+        nat.get_state_device(self._obs, layout=N.LAYOUT_AOS)
+        return out
 
     def capture_graph(self, policy: Callable, n_steps: int):
         """Record ``n_steps`` iterations of ``obs -> policy(obs) -> step`` into a CUDA graph (the policy must be

@@ -388,6 +388,45 @@ class NativeEnv:
         r.reward_sum, r.viol_count, r.done_count = N.ptr_of(reward_sum), N.ptr_of(viol_count), N.ptr_of(done_count)
         N.check(N.lib().nig_rollout(self._h, C.byref(r), self._stream(stream)))
 
+    # nig_trajectory_t fields: (per-step width or None for [T, n] rows, accepted torch dtype names)
+    RECORD_FIELDS = {"obs": ("S", ("float32",)), "actions": ("A", ("float32",)), "rewards": (None, ("float32",)),
+                     "flags": (None, ("uint8",)), "viol_mask": (None, ("uint8",)), "terminated": (None, ("uint8", "bool")),
+                     "truncated": (None, ("uint8", "bool")), "next_obs": ("S", ("float32",))}
+
+    def rollout_record_device(self, n_steps: int, policy: int = N.POLICY_UNIFORM, *, out: dict, actions=None, noise=None,
+                              params=None, reward_sum=None, viol_count=None, done_count=None, stream=None):
+        """``rollout_device`` that also records every step (nig_rollout_record, one launch): ``out`` maps any subset of
+        obs / actions / next_obs ([T, n, S | A] fp32), rewards ([T, n] fp32), flags / viol_mask ([T, n] uint8) and
+        terminated / truncated ([T, n] uint8 or bool) to contiguous CUDA tensors on this env's device; row [t, i] is what
+        ``step_device`` writes for env i at step t. ``actions`` [T, A, pitch] / ``noise`` [T, NZ, pitch] teacher-force the run
+        (policy ACTIONS) as in ``rollout_device``. Every tensor is checked before anything is launched (ValueError)."""
+        import torch
+        T, dev = int(n_steps), self.torch_device()
+        tr = N.Trajectory()
+        for name, x in out.items():
+            if name not in self.RECORD_FIELDS:
+                raise ValueError(f"unknown trajectory field {name!r}; expected a subset of {sorted(self.RECORD_FIELDS)}")
+            if x is None:
+                continue
+            width, dtypes = self.RECORD_FIELDS[name]
+            shape = (T, self.n) if width is None else (T, self.n, getattr(self, width))
+            if not isinstance(x, torch.Tensor) or x.device != dev:
+                raise ValueError(f"out[{name!r}] must be a torch tensor on {dev}")
+            if str(x.dtype).replace("torch.", "") not in dtypes:
+                raise ValueError(f"out[{name!r}] must have dtype {' or '.join(dtypes)}, not {x.dtype}")
+            if tuple(x.shape) != shape:
+                raise ValueError(f"out[{name!r}] must have shape {shape}, not {tuple(x.shape)}")
+            if not x.is_contiguous():
+                raise ValueError(f"out[{name!r}] must be contiguous")
+            setattr(tr, name, x.data_ptr())
+        r = N.Rollout()
+        r.n_steps, r.policy = T, int(policy)
+        r.actions, r.noise = N.ptr_of(actions), N.ptr_of(noise)
+        if params is not None:
+            r.pp = params
+        r.reward_sum, r.viol_count, r.done_count = N.ptr_of(reward_sum), N.ptr_of(viol_count), N.ptr_of(done_count)
+        N.check(N.lib().nig_rollout_record(self._h, C.byref(r), C.byref(tr), self._stream(stream)))
+
     def rollout_steps_device(self, total_steps: int, steps_per_launch: int = 64, policy: int = N.POLICY_UNIFORM, *, params=None,
                              reward_sum=None, viol_count=None, done_count=None, accumulate: bool = False, stream=None):
         """``total_steps`` steps of every env in ``steps_per_launch``-step fused launches with an in-kernel policy; large
