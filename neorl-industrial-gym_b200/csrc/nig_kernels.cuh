@@ -1331,7 +1331,7 @@ __device__ __forceinline__ float cdiv_noguard(float x, float c, float rc)
 
 struct RolloutAcc {            // episode / launch statistics of one thread (shared by the fast and the generic loop)
     unsigned int c_steps = 0, c_ep = 0, c_term = 0, c_trunc = 0, c_crit = 0, c_viol = 0, c_succ = 0, c_done = 0;
-    unsigned int c_con[NIG_MAX_CONSTRAINTS];
+    unsigned int c_con[NIG_MAX_CONSTRAINTS] = {};
     unsigned long long len_sum = 0, len_sq = 0;
     double ret_sum = 0.0, ret_sq = 0.0, rew_sum = 0.0;
 };
@@ -2175,6 +2175,115 @@ __device__ __forceinline__ void rollout_stats_flush(const RolloutArgs& p, BlockS
     advance_device_tick(p.tick_dev, (uint32_t)p.n_steps);
 }
 
+// ---- the common head of the fused rollout kernels with one env per thread: the statistics staging zeroed, this CTA's copy of
+// the normal table where the env reads it from shared memory, the shared counters (synchronises the CTA); returns the key of
+// the random streams
+template <class Env>
+__device__ __forceinline__ Rng rollout_cta_init(const RolloutArgs& p, BlockStats& bs, unsigned int* sstat, double* sfl,
+                                                unsigned long long* sext, float4* s_tab, bool extrema)
+{
+    if (threadIdx.x < 4) sfl[threadIdx.x] = 0.0;
+    if (extrema && threadIdx.x < 2) sext[threadIdx.x] = 0ull;
+    if constexpr (Env::ROLLOUT_TAB_SMEM) normal_table_to_smem(s_tab);
+    const Rng key(p.key, Env::ROLLOUT_TAB_SMEM ? s_tab : g_normal_tab);
+    bs.init(sstat);
+    return key;
+}
+
+// the env's state, episode word (unpacked across the K steps) and running return
+template <class Env>
+__device__ __forceinline__ void rollout_load(const RolloutArgs& p, int64_t ic, float (&s)[Env::S], uint32_t& ep_st, uint32_t& ep_vi,
+                                             bool& latched, typename Env::acc_t& ep_ret)
+{
+#pragma unroll
+    for (int k = 0; k < Env::S; ++k) s[k] = p.state[k * p.pitch + ic];
+    const uint32_t w0 = p.ep_word[ic];
+    ep_st = epw_step(w0); ep_vi = epw_viol(w0);
+    latched = (w0 >> 31) != 0u;
+    ep_ret = (typename Env::acc_t)p.ep_return[ic];
+}
+
+// one step of the fused rollouts' generic loop after the policy: step_core, the per-thread statistics, the episode bookkeeping
+// and the auto-reset; must be called convergently (coop resets). rollout_kernel keeps an inline copy (see there). `extrema` is nig_track_extrema (a constant where the kernel
+// has it as a template flag). COOP_RESET = false resets envs with a block-cooperative reset (PowerGrid) per lane, for kernels
+// without a CoopSmem buffer. REC (nig_rollout_record's kernels) also hands out in *rec what nig_step writes for the env in
+// this step.
+template <class Env>
+struct StepRecord {
+    float ns[Env::S];          // s' of the transition, before the auto-reset; an inactive env's unchanged state
+    float r;                   // reward; 0 for an inactive env
+    uint32_t f, vm;            // NIG_F_* flags with NIG_F_RESET / NIG_F_INACTIVE as nig_step sets them; violation mask (0 inactive)
+};
+template <class Env, int CONS, bool CLIP, bool REC = false, bool COOP_RESET = true>
+__device__ __forceinline__ void rollout_step_generic(const RolloutArgs& p, const Rng& key, uint32_t env, uint32_t tick, uint32_t epoch,
+                                                     bool valid, bool extrema, const float (&a)[Env::A],
+                                                     const float (&nz)[Env::NZ > 0 ? Env::NZ : 1], float (&s)[Env::S],
+                                                     uint32_t& ep_st, uint32_t& ep_vi, bool& latched, typename Env::acc_t& ep_ret,
+                                                     float& rsum, RolloutAcc& acc, typename Env::acc_t& r_lo, typename Env::acc_t& r_hi,
+                                                     float* coop_buf, StepRecord<Env>* rec = nullptr)
+{
+    constexpr int S = Env::S;
+    constexpr bool COOP = COOP_RESET && (Env::COOP_BLOCKS > 0 || Env::COOP_FK);
+    using acc_t = typename Env::acc_t;
+    float ns[S];
+    const bool active = valid && !latched;
+    uint32_t st2, vi2, f, vm;
+    acc_t r;
+    bool need_reset = false;
+    step_core_unpacked<Env, CONS, CLIP, true>(p.cons, p.max_steps, s, a, nz, 0u, ep_st, ep_vi, st2, vi2, ns, r, f, vm);
+    if constexpr (REC) {
+        // step_kernel's outputs: the rollout computes r / f / vm for inactive lanes too, nig_step reports them as nothing happened
+        const bool done = (f & (NIG_F_TERMINATED | NIG_F_TRUNCATED)) != 0;
+#pragma unroll
+        for (int k = 0; k < S; ++k) rec->ns[k] = active ? ns[k] : s[k];
+        rec->r = active ? (float)r : 0.0f;
+        rec->f = !active ? (uint32_t)NIG_F_INACTIVE : (done && p.auto_reset) ? (f | (uint32_t)NIG_F_RESET) : f;
+        rec->vm = active ? vm : 0u;
+    }
+    if (active) {
+        const bool done = (f & (NIG_F_TERMINATED | NIG_F_TRUNCATED)) != 0;
+        rsum = add(rsum, (float)r);
+        ep_ret = ep_ret + r;
+        if constexpr (sizeof(acc_t) == 8) acc.rew_sum += r;      // fp32-reward envs: derived from rsum after the loop
+        acc.c_steps += 1; acc.c_viol += __popc(vm);
+        acc.c_crit += (f & NIG_F_CRITICAL) ? 1u : 0u;
+#pragma unroll
+        for (int k = 0; k < Env::NB; ++k) acc.c_con[k] += (vm >> k) & 1u;
+        if constexpr (cons_fast_extras(CONS) > 0) {
+#pragma unroll
+            for (int k = Env::NB; k < Env::NB + cons_fast_extras(CONS); ++k) acc.c_con[k] += (vm >> k) & 1u;
+        } else if constexpr (CONS != CONS_DEFAULT) {
+#pragma unroll
+            for (int k = Env::NB; k < NIG_MAX_CONSTRAINTS; ++k) acc.c_con[k] += (vm >> k) & 1u;
+        }
+        ep_st = st2; ep_vi = vi2;
+        if (done) {
+            const unsigned long long len = st2;
+            acc.c_ep += 1; acc.c_done += 1;
+            acc.c_term += (f & NIG_F_TERMINATED) ? 1u : 0u;
+            acc.c_trunc += (f & NIG_F_TRUNCATED) ? 1u : 0u;
+            acc.c_succ += (ep_ret > (acc_t)0) ? 1u : 0u;
+            acc.len_sum += len; acc.len_sq += len * len;
+            acc.ret_sum += (double)ep_ret; acc.ret_sq += (double)ep_ret * (double)ep_ret;
+            if (extrema) { r_lo = ep_ret < r_lo ? ep_ret : r_lo; r_hi = ep_ret > r_hi ? ep_ret : r_hi; }
+            if (p.auto_reset) {
+                if constexpr (COOP) need_reset = true;
+                else Env::reset(key, env, tick + 1u, epoch, s);
+                ep_st = 0u; ep_vi = 0u; ep_ret = (acc_t)0;
+            } else {
+#pragma unroll
+                for (int k = 0; k < S; ++k) s[k] = ns[k];
+                latched = true;
+            }
+        } else {
+#pragma unroll
+            for (int k = 0; k < S; ++k) s[k] = ns[k];
+        }
+    }
+    if constexpr (COOP && Env::COOP_BLOCKS > 0) coop_reset_blocks<Env>(key, env, tick + 1u, epoch, need_reset, s, coop_buf);
+    else if constexpr (COOP) coop_reset_fk<Env>(key, env, tick + 1u, epoch, need_reset, s, coop_buf);
+}
+
 // TFNOISE: process noise teacher-forced from p.noise (POLICY_ACTIONS only). The LDG flavour of POLICY_ACTIONS
 // prefetches the next step's actions / noise into registers one step ahead, so the L2 latency of the loads is
 // hidden behind a whole step of arithmetic. Block size is a launch parameter (blockDim.x <= kThreads; TMA launches
@@ -2240,8 +2349,6 @@ __global__ void __launch_bounds__(kThreads, Env::ROLLOUT_MIN_CTAS) rollout_kerne
 
     float rsum = 0.0f;
     RolloutAcc acc;
-#pragma unroll
-    for (int k = 0; k < NIG_MAX_CONSTRAINTS; ++k) acc.c_con[k] = 0;
     acc_t r_lo = (acc_t)INFINITY, r_hi = -(acc_t)INFINITY;     // extrema of this thread's finished-episode returns
 
     double pid_i[A], pid_e[A];             // POLICY_BASELINE: the PID agent's integral and previous error
@@ -2346,9 +2453,9 @@ __global__ void __launch_bounds__(kThreads, Env::ROLLOUT_MIN_CTAS) rollout_kerne
             } else ng.get(key, env, tick, nz);
         } else nz[0] = 0.0f;
 
-        // this step-and-bookkeeping block is repeated statement for statement in rollout_step_generic (nig_mlp.cuh, the
-        // kernels of the MLP policy and of nig_rollout_record) and, for the uniform policy, in rollout_generic_uniform_step: a change here goes there too
-        // (moving it into a shared function changed ptxas' schedule of this kernel's reactor instantiations)
+        // rollout_step_generic statement for statement, kept inline: calling the function from here moved ptxas' schedule of
+        // 167 of this kernel's instantiations, and the SafetyWrapper one (ChemicalReactor-v0, CONS_BOUNDS2, uniform policy) ran
+        // 0.8 % slower on a B200 (profiles/r03_d_sass_and_speed.txt). A change here goes there too.
         const bool active = valid && !latched;
         uint32_t st2, vi2, f, vm;
         acc_t r;
@@ -2412,58 +2519,21 @@ __global__ void __launch_bounds__(kThreads, Env::ROLLOUT_MIN_CTAS) rollout_kerne
     rollout_epilogue<Env, EXTREMA>(p, bs, sfl, sext, valid, i, s, ep_st, ep_vi, latched, ep_ret, rsum, acc, r_lo, r_hi);
 }
 
-// one generic step of the uniform-random rollout with in-place draws: the loop body of rollout_kernel for POLICY_UNIFORM
-// (envs without a block-cooperative reset), used by rollout_grid_kernel and rollout_reactor_pair_kernel where a warp cannot
-// take the fast loop
+// one generic step of the uniform-random rollout with in-place draws, used by rollout_grid_kernel and
+// rollout_reactor_pair_kernel where a warp cannot take the fast loop. These kernels have no CoopSmem buffer, so PowerGrid
+// resets per lane here: this is its fallback path only.
 template <class Env, int CONS, bool EXTREMA>
 __device__ __forceinline__ void rollout_generic_uniform_step(const RolloutArgs& p, const Rng& key, uint32_t env, uint32_t tick, uint32_t epoch, bool valid,
                                                              float (&s)[Env::S], uint32_t& ep_st, uint32_t& ep_vi, bool& latched,
                                                              typename Env::acc_t& ep_ret, float& rsum, RolloutAcc& acc,
                                                              typename Env::acc_t& r_lo, typename Env::acc_t& r_hi)
 {
-    // (envs with a block-cooperative reset -- PowerGrid -- reset per lane here: this is their fallback path only)
-    constexpr int S = Env::S, A = Env::A, NZ = Env::NZ, NZA = NZ > 0 ? NZ : 1;
-    using acc_t = typename Env::acc_t;
-    float a[A], nz[NZA], ns[S];
+    constexpr int A = Env::A, NZ = Env::NZ, NZA = NZ > 0 ? NZ : 1;
+    float a[A], nz[NZA];
     policy_uniform<Env>(key, env, tick, a);
     if constexpr (NZ > 0) { typename Env::NoiseGen ng; ng.get(key, env, tick, nz); } else nz[0] = 0.0f;
-    const bool active = valid && !latched;
-    uint32_t st2, vi2, f, vm;
-    acc_t r;
-    step_core_unpacked<Env, CONS, false, true>(p.cons, p.max_steps, s, a, nz, 0u, ep_st, ep_vi, st2, vi2, ns, r, f, vm);
-    if (active) {
-        const bool done = (f & (NIG_F_TERMINATED | NIG_F_TRUNCATED)) != 0;
-        rsum = add(rsum, (float)r);
-        ep_ret = ep_ret + r;
-        if constexpr (sizeof(acc_t) == 8) acc.rew_sum += r;
-        acc.c_steps += 1; acc.c_viol += __popc(vm);
-        acc.c_crit += (f & NIG_F_CRITICAL) ? 1u : 0u;
-#pragma unroll
-        for (int k = 0; k < NIG_MAX_CONSTRAINTS; ++k)
-            if (k < Env::NB || CONS != CONS_DEFAULT) acc.c_con[k] += (vm >> k) & 1u;
-        ep_st = st2; ep_vi = vi2;
-        if (done) {
-            const unsigned long long len = st2;
-            acc.c_ep += 1; acc.c_done += 1;
-            acc.c_term += (f & NIG_F_TERMINATED) ? 1u : 0u;
-            acc.c_trunc += (f & NIG_F_TRUNCATED) ? 1u : 0u;
-            acc.c_succ += (ep_ret > (acc_t)0) ? 1u : 0u;
-            acc.len_sum += len; acc.len_sq += len * len;
-            acc.ret_sum += (double)ep_ret; acc.ret_sq += (double)ep_ret * (double)ep_ret;
-            if constexpr (EXTREMA) { r_lo = ep_ret < r_lo ? ep_ret : r_lo; r_hi = ep_ret > r_hi ? ep_ret : r_hi; }
-            if (p.auto_reset) {
-                Env::reset(key, env, tick + 1u, epoch, s);
-                ep_st = 0u; ep_vi = 0u; ep_ret = (acc_t)0;
-            } else {
-#pragma unroll
-                for (int k = 0; k < S; ++k) s[k] = ns[k];
-                latched = true;
-            }
-        } else {
-#pragma unroll
-            for (int k = 0; k < S; ++k) s[k] = ns[k];
-        }
-    }
+    rollout_step_generic<Env, CONS, false, false, false>(p, key, env, tick, epoch, valid, EXTREMA, a, nz, s, ep_st, ep_vi, latched,
+                                                         ep_ret, rsum, acc, r_lo, r_hi, nullptr);
 }
 
 // ================================================================================================
@@ -2503,17 +2573,13 @@ __global__ void __launch_bounds__(THREADS) __maxnreg__(MAXREG) rollout_grid_kern
     const uint32_t tick0 = load_tick(p.tick_dev, p.tick) + base_tick(p.tick_base);
     const uint32_t epoch = p.epoch + base_epoch(p.tick_base);
     float s[S];
-#pragma unroll
-    for (int k = 0; k < S; ++k) s[k] = p.state[k * p.pitch + ic];
-    const uint32_t w0 = p.ep_word[ic];
-    uint32_t ep_st = epw_step(w0), ep_vi = epw_viol(w0);
-    bool latched = (w0 >> 31) != 0u;
-    double ep_ret = p.ep_return[ic];
+    uint32_t ep_st, ep_vi;
+    bool latched;
+    double ep_ret;
+    rollout_load<Env>(p, ic, s, ep_st, ep_vi, latched, ep_ret);
     float rsum = 0.0f;
     double r_lo = INFINITY, r_hi = -INFINITY;
     RolloutAcc acc;
-#pragma unroll
-    for (int k = 0; k < NIG_MAX_CONSTRAINTS; ++k) acc.c_con[k] = 0;
 
     int t_begin = 0;
     {
@@ -2811,10 +2877,6 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_reactor_pair_kernel(const
     float ep_ret[2] = {(float)er0.x, (float)er0.y}, rsum[2] = {0.0f, 0.0f};
     float r_lo = INFINITY, r_hi = -INFINITY;
     RolloutAcc acc[2];
-#pragma unroll
-    for (int e = 0; e < 2; ++e)
-#pragma unroll
-        for (int k = 0; k < NIG_MAX_CONSTRAINTS; ++k) acc[e].c_con[k] = 0;
 
     bool inv = p.auto_reset != 0;
 #pragma unroll

@@ -1,6 +1,6 @@
-// nig_mlp.cuh -- device code shared by the fused rollouts of nig_rollout_mlp.cu (NIG_POLICY_MLP) and
-// nig_rollout_record.cu (nig_rollout_record): the tcgen05 MLP forward pass, rollout_kernel's generic step as a function, and
-// the launch-side sizing of the MLP kernels' dynamic shared memory.
+// nig_mlp.cuh -- the MLP policy of the fused rollouts of nig_rollout_mlp.cu (NIG_POLICY_MLP) and nig_rollout_record.cu
+// (nig_rollout_record): the tcgen05 helpers, the MLP forward pass, and the launch-side sizing of the MLP kernels' dynamic
+// shared memory.
 #pragma once
 #include <mutex>
 #include <vector>
@@ -197,87 +197,6 @@ __device__ __forceinline__ void mlp_forward(MlpCta& c, const MlpParams& m, const
         const float y = __fadd_rn(v[k], b3[k]);
         a[k] = m.out_tanh ? tanhf(y) : y;
     }
-}
-
-// one step of rollout_kernel's generic loop after the policy: step_core, the per-thread statistics, the episode bookkeeping
-// and the (cooperative) auto-reset, statement for statement; must be called convergently (coop resets). `extrema` is the
-// run-time switch of nig_track_extrema. rollout_kernel keeps its inline copy: calling this function from it changed ptxas'
-// instruction schedule of 24 of its reactor instantiations (the benchmark's among them), and existing kernels stay as measured.
-// REC (nig_rollout_record's kernels; off for the MLP rollout, whose code it leaves as it was) also hands out in *rec what
-// nig_step writes for the env in this step.
-template <class Env>
-struct StepRecord {
-    float ns[Env::S];          // s' of the transition, before the auto-reset; an inactive env's unchanged state
-    float r;                   // reward; 0 for an inactive env
-    uint32_t f, vm;            // NIG_F_* flags with NIG_F_RESET / NIG_F_INACTIVE as nig_step sets them; violation mask (0 inactive)
-};
-template <class Env, int CONS, bool CLIP, bool REC = false>
-__device__ __forceinline__ void rollout_step_generic(const RolloutArgs& p, const Rng& key, uint32_t env, uint32_t tick, uint32_t epoch,
-                                                     bool valid, bool extrema, const float (&a)[Env::A],
-                                                     const float (&nz)[Env::NZ > 0 ? Env::NZ : 1], float (&s)[Env::S],
-                                                     uint32_t& ep_st, uint32_t& ep_vi, bool& latched, typename Env::acc_t& ep_ret,
-                                                     float& rsum, RolloutAcc& acc, typename Env::acc_t& r_lo, typename Env::acc_t& r_hi,
-                                                     float* coop_buf, StepRecord<Env>* rec = nullptr)
-{
-    constexpr int S = Env::S;
-    using acc_t = typename Env::acc_t;
-    float ns[S];
-    const bool active = valid && !latched;
-    uint32_t st2, vi2, f, vm;
-    acc_t r;
-    bool need_reset = false;
-    step_core_unpacked<Env, CONS, CLIP, true>(p.cons, p.max_steps, s, a, nz, 0u, ep_st, ep_vi, st2, vi2, ns, r, f, vm);
-    if constexpr (REC) {
-        // step_kernel's outputs: the rollout computes r / f / vm for inactive lanes too, nig_step reports them as nothing happened
-        const bool done = (f & (NIG_F_TERMINATED | NIG_F_TRUNCATED)) != 0;
-#pragma unroll
-        for (int k = 0; k < S; ++k) rec->ns[k] = active ? ns[k] : s[k];
-        rec->r = active ? (float)r : 0.0f;
-        rec->f = !active ? (uint32_t)NIG_F_INACTIVE : (done && p.auto_reset) ? (f | (uint32_t)NIG_F_RESET) : f;
-        rec->vm = active ? vm : 0u;
-    }
-    if (active) {
-        const bool done = (f & (NIG_F_TERMINATED | NIG_F_TRUNCATED)) != 0;
-        rsum = add(rsum, (float)r);
-        ep_ret = ep_ret + r;
-        if constexpr (sizeof(acc_t) == 8) acc.rew_sum += r;      // fp32-reward envs: derived from rsum after the loop
-        acc.c_steps += 1; acc.c_viol += __popc(vm);
-        acc.c_crit += (f & NIG_F_CRITICAL) ? 1u : 0u;
-#pragma unroll
-        for (int k = 0; k < Env::NB; ++k) acc.c_con[k] += (vm >> k) & 1u;
-        if constexpr (cons_fast_extras(CONS) > 0) {
-#pragma unroll
-            for (int k = Env::NB; k < Env::NB + cons_fast_extras(CONS); ++k) acc.c_con[k] += (vm >> k) & 1u;
-        } else if constexpr (CONS != CONS_DEFAULT) {
-#pragma unroll
-            for (int k = Env::NB; k < NIG_MAX_CONSTRAINTS; ++k) acc.c_con[k] += (vm >> k) & 1u;
-        }
-        ep_st = st2; ep_vi = vi2;
-        if (done) {
-            const unsigned long long len = st2;
-            acc.c_ep += 1; acc.c_done += 1;
-            acc.c_term += (f & NIG_F_TERMINATED) ? 1u : 0u;
-            acc.c_trunc += (f & NIG_F_TRUNCATED) ? 1u : 0u;
-            acc.c_succ += (ep_ret > (acc_t)0) ? 1u : 0u;
-            acc.len_sum += len; acc.len_sq += len * len;
-            acc.ret_sum += (double)ep_ret; acc.ret_sq += (double)ep_ret * (double)ep_ret;
-            if (extrema) { r_lo = ep_ret < r_lo ? ep_ret : r_lo; r_hi = ep_ret > r_hi ? ep_ret : r_hi; }
-            if (p.auto_reset) {
-                if constexpr (Env::COOP_BLOCKS > 0 || Env::COOP_FK) need_reset = true;
-                else Env::reset(key, env, tick + 1u, epoch, s);
-                ep_st = 0u; ep_vi = 0u; ep_ret = (acc_t)0;
-            } else {
-#pragma unroll
-                for (int k = 0; k < S; ++k) s[k] = ns[k];
-                latched = true;
-            }
-        } else {
-#pragma unroll
-            for (int k = 0; k < S; ++k) s[k] = ns[k];
-        }
-    }
-    if constexpr (Env::COOP_BLOCKS > 0) coop_reset_blocks<Env>(key, env, tick + 1u, epoch, need_reset, s, coop_buf);
-    else if constexpr (Env::COOP_FK) coop_reset_fk<Env>(key, env, tick + 1u, epoch, need_reset, s, coop_buf);
 }
 
 // dynamic shared memory of a launch: the blob and the activation tiles, raised where needed so that no more CTAs fit on an SM

@@ -12,7 +12,7 @@
 
 namespace nig {
 
-// ---- the fused rollout with the MLP policy: rollout_kernel's generic loop (rollout_step_generic, nig_mlp.cuh) with the action from
+// ---- the fused rollout with the MLP policy: rollout_kernel's generic loop (rollout_step_generic, nig_kernels.cuh) with the action from
 // mlp_forward. 128 threads per CTA, one env per thread; CONS_DEFAULT and CONS_GENERIC (which also runs the CONS_PREFIX and
 // CONS_BOUNDS* sets, bit-identically); return extrema as a run-time switch (m.extrema).
 template <class Env, int CONS>
@@ -29,11 +29,7 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_mlp_kernel(const __grid_c
     __shared__ alignas(16) float coop_buf[CoopSmem<Env>::floats];
     extern __shared__ __align__(128) uint8_t mlp_smem[];
     BlockStats bs;
-    if (threadIdx.x < 4) sfl[threadIdx.x] = 0.0;
-    if (threadIdx.x < 2) sext[threadIdx.x] = 0ull;
-    if constexpr (Env::ROLLOUT_TAB_SMEM) normal_table_to_smem(s_tab);
-    const Rng key(p.key, Env::ROLLOUT_TAB_SMEM ? s_tab : g_normal_tab);
-    bs.init(sstat);
+    const Rng key = rollout_cta_init<Env>(p, bs, sstat, sfl, sext, s_tab, true);
     MlpCta mc;
     mlp_setup(mc, m, S, mlp_smem, bars, &tmem_slot);
     rollout_pdl_sync();
@@ -47,17 +43,13 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_mlp_kernel(const __grid_c
     const bool extrema = m.extrema != 0;
 
     float s[S];
-#pragma unroll
-    for (int k = 0; k < S; ++k) s[k] = p.state[k * p.pitch + ic];
-    const uint32_t w0 = p.ep_word[ic];
-    uint32_t ep_st = epw_step(w0), ep_vi = epw_viol(w0);
-    bool latched = (w0 >> 31) != 0u;
-    acc_t ep_ret = (acc_t)p.ep_return[ic];
+    uint32_t ep_st, ep_vi;
+    bool latched;
+    acc_t ep_ret;
+    rollout_load<Env>(p, ic, s, ep_st, ep_vi, latched, ep_ret);
     typename Env::NoiseGen ng;
     float rsum = 0.0f;
     RolloutAcc acc;
-#pragma unroll
-    for (int k = 0; k < NIG_MAX_CONSTRAINTS; ++k) acc.c_con[k] = 0;
     acc_t r_lo = (acc_t)INFINITY, r_hi = -(acc_t)INFINITY;
 
 #pragma unroll 1

@@ -3,7 +3,7 @@
 //  - rollout_record_kernel: teacher-forced actions (with or without teacher-forced noise) and the in-kernel policies UNIFORM,
 //    ZERO, PCTRL and BASELINE -- rollout_kernel's generic loop with the policy a run-time switch;
 //  - rollout_mlp_record_kernel: NIG_POLICY_MLP -- rollout_mlp_kernel's loop (same mlp_forward, tiling and tensor memory).
-// Both step through rollout_step_generic (nig_mlp.cuh) with its record outputs, so that dynamics, statistics and episode
+// Both step through rollout_step_generic (nig_kernels.cuh) with its record outputs, so that dynamics, statistics and episode
 // bookkeeping are nig_rollout's, and both end in rollout_epilogue. 128 threads per CTA, one env per thread; CONS_DEFAULT and
 // CONS_GENERIC (which runs every other constraint set bit-identically). AoS rows leave through the per-warp shared-memory
 // transpose (store_aos_warp) with streaming stores. See DESIGN.md §3.7 for the budgets.
@@ -59,11 +59,7 @@ __global__ void __launch_bounds__(kThreads) rollout_record_kernel(const __grid_c
     __shared__ float rec_tile[(kThreads / 32) * rec_tile_floats<Env>()];
     float* tile = rec_tile + (threadIdx.x >> 5) * rec_tile_floats<Env>();
     BlockStats bs;
-    if (threadIdx.x < 4) sfl[threadIdx.x] = 0.0;
-    if (threadIdx.x < 2) sext[threadIdx.x] = 0ull;
-    if constexpr (Env::ROLLOUT_TAB_SMEM) normal_table_to_smem(s_tab);
-    const Rng key(p.key, Env::ROLLOUT_TAB_SMEM ? s_tab : g_normal_tab);
-    bs.init(sstat);
+    const Rng key = rollout_cta_init<Env>(p, bs, sstat, sfl, sext, s_tab, true);
     rollout_pdl_sync();
 
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -76,17 +72,13 @@ __global__ void __launch_bounds__(kThreads) rollout_record_kernel(const __grid_c
     const bool pid = rp.policy == NIG_POLICY_BASELINE && p.pp.baseline.kind == NIG_BASELINE_PID && p.pid_state != nullptr;
 
     float s[S];
-#pragma unroll
-    for (int k = 0; k < S; ++k) s[k] = p.state[k * p.pitch + ic];
-    const uint32_t w0 = p.ep_word[ic];
-    uint32_t ep_st = epw_step(w0), ep_vi = epw_viol(w0);
-    bool latched = (w0 >> 31) != 0u;
-    acc_t ep_ret = (acc_t)p.ep_return[ic];
+    uint32_t ep_st, ep_vi;
+    bool latched;
+    acc_t ep_ret;
+    rollout_load<Env>(p, ic, s, ep_st, ep_vi, latched, ep_ret);
     typename Env::NoiseGen ng;
     float rsum = 0.0f;
     RolloutAcc acc;
-#pragma unroll
-    for (int k = 0; k < NIG_MAX_CONSTRAINTS; ++k) acc.c_con[k] = 0;
     acc_t r_lo = (acc_t)INFINITY, r_hi = -(acc_t)INFINITY;
     double pid_i[A], pid_e[A];             // POLICY_BASELINE: the PID agent's integral and previous error
 #pragma unroll
@@ -158,11 +150,7 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_mlp_record_kernel(const _
     __shared__ alignas(16) float coop_buf[CoopSmem<Env>::floats];
     extern __shared__ __align__(128) uint8_t mlp_smem[];
     BlockStats bs;
-    if (threadIdx.x < 4) sfl[threadIdx.x] = 0.0;
-    if (threadIdx.x < 2) sext[threadIdx.x] = 0ull;
-    if constexpr (Env::ROLLOUT_TAB_SMEM) normal_table_to_smem(s_tab);
-    const Rng key(p.key, Env::ROLLOUT_TAB_SMEM ? s_tab : g_normal_tab);
-    bs.init(sstat);
+    const Rng key = rollout_cta_init<Env>(p, bs, sstat, sfl, sext, s_tab, true);
     MlpCta mc;
     mlp_setup(mc, m, S, mlp_smem, bars, &tmem_slot);
     rollout_pdl_sync();
@@ -177,17 +165,13 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_mlp_record_kernel(const _
     const bool extrema = m.extrema != 0;
 
     float s[S];
-#pragma unroll
-    for (int k = 0; k < S; ++k) s[k] = p.state[k * p.pitch + ic];
-    const uint32_t w0 = p.ep_word[ic];
-    uint32_t ep_st = epw_step(w0), ep_vi = epw_viol(w0);
-    bool latched = (w0 >> 31) != 0u;
-    acc_t ep_ret = (acc_t)p.ep_return[ic];
+    uint32_t ep_st, ep_vi;
+    bool latched;
+    acc_t ep_ret;
+    rollout_load<Env>(p, ic, s, ep_st, ep_vi, latched, ep_ret);
     typename Env::NoiseGen ng;
     float rsum = 0.0f;
     RolloutAcc acc;
-#pragma unroll
-    for (int k = 0; k < NIG_MAX_CONSTRAINTS; ++k) acc.c_con[k] = 0;
     acc_t r_lo = (acc_t)INFINITY, r_hi = -(acc_t)INFINITY;
 
 #pragma unroll 1
